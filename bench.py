@@ -127,6 +127,41 @@ def cpu_reference_throughput(wl, n_triplets, procs, kind):
             "windows": n, "triplets": n_triplets}
 
 
+DUMP_WINDOWS = 1 << 16          # windows whose per-window results are written
+DUMP_READS = 1 << 16            # reads whose per-read counters are written
+DUMP_ROW_LETTERS = 4 << 20      # at most this many MSA row columns (3 per window column) are written
+
+
+def dump_outputs(out_dir, wl, d_rows, d_rowoff, d_stride, d_nring, d_s1, d_s2, d_cells, d_cnt, d_sums):
+    """What elector_poa_run_device + elector_merge_tally_device + elector_tally_sum_device left in their output buffers, as
+    float64 .npy files of at most ~50 MB in all: the global counters, and for samples of reads and of windows drawn with a
+    fixed seed from their counts alone (the same ones for the same arguments) the per-read counters, and per window the
+    ring length, DP scores, cell count and the three MSA rows, concatenated in the order rows_window_index lists them.
+    The rows stop at DUMP_ROW_LETTERS columns, counted from the input lengths, so that the cut does not depend on what
+    was computed."""
+    import torch
+    n, n_trip = len(wl["ref_off"]) - 1, len(wl["read_first"]) - 1
+    rng = np.random.default_rng(12345)
+    win = np.sort(rng.choice(n, min(n, DUMP_WINDOWS), replace=False))
+    reads = np.sort(rng.choice(n_trip, min(n_trip, DUMP_READS), replace=False))
+    nring = d_nring.cpu().numpy()
+    out = {"sums": d_sums.cpu().numpy(), "read_index": reads, "counters": d_cnt.cpu().numpy().reshape(n_trip, -1)[reads],
+           "window_index": win, "nring": nring[win], "score1": d_s1.cpu().numpy()[win], "score2": d_s2.cpu().numpy()[win],
+           "cells": d_cells.cpu().numpy()[win]}
+    # nring <= ref + cor + unc letters of the window: the row budget is cut on that bound
+    bound = sum(np.diff(wl[k])[win] for k in ("ref_off", "cor_off", "unc_off"))
+    rwin = win[:int(np.searchsorted(np.cumsum(3 * bound), DUMP_ROW_LETTERS, side="right"))]
+    ro, st, nr = d_rowoff.cpu().numpy()[rwin], d_stride.cpu().numpy()[rwin].astype(np.int64), nring[rwin].astype(np.int64)
+    starts = (ro[:, None] + st[:, None] * np.arange(3)).ravel()      # window-major, rows ref / cor / unc
+    lens = np.repeat(nr, 3)
+    idx = np.repeat(starts - np.concatenate(([0], np.cumsum(lens)[:-1])), lens) + np.arange(int(lens.sum()))
+    out["rows_window_index"] = rwin
+    out["rows"] = d_rows[torch.from_numpy(idx).to(d_rows.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -138,6 +173,11 @@ def main():
     ap.add_argument("--cpu-triplets", type=int, default=0, help="triplets of the CPU baseline sample (default: sized for ~10-20 s)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--e2e-main-only", action="store_true", help="time only the headline wire format and the byte path")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of the headline path computed as DIR/<name>.npy "
+                                                          "(float64; per-window results and MSA rows of a fixed sample of windows). The same "
+                                                          "arguments give the same inputs only from the same window source: compare dumps of "
+                                                          "runs whose JSON line has the same config.windows_from (the windows are cut by "
+                                                          "oracle/_ref/masterSplitter where it is built, else synthesised directly)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 0)
 
@@ -515,6 +555,8 @@ def main():
                                 "gcups": cb["gcups"]}
     if rank == 0:
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, wl, d_rows, d_rowoff, d_stride, d_nring, d_s1, d_s2, d_cells, d_cnt, d_sums)
     ctx.close()
     if world > 1:
         dist.destroy_process_group()

@@ -1,7 +1,12 @@
 import gzip
 import os
+import shutil
+import signal
 import subprocess
 import sys
+import tempfile
+import time
+import warnings
 
 import pytest
 
@@ -56,6 +61,47 @@ def golden_dir(tmp_path_factory):
     return d
 
 
+@pytest.fixture(scope="session", autouse=True)
+def service_ends_with_the_session():
+    """The drop-in executables hand their work to elector_server (elector_b200/csrc/service.h), which outlives them by
+    ELECTOR_SERVICE_IDLE seconds.  The session gives the server its own socket and a short idle time, and waits for it to
+    leave, so that no process of the tests outlives them."""
+    d = tempfile.mkdtemp(prefix="elsvc")          # short: a socket path has at most 107 bytes
+    sock = os.path.join(d, "sock")
+    mp = pytest.MonkeyPatch()
+    mp.setenv("ELECTOR_SERVICE_SOCKET", sock)
+    mp.setenv("ELECTOR_SERVICE_IDLE", "2")
+    yield
+    mp.undo()
+    deadline = time.time() + 60
+    while time.time() < deadline and service_pids(sock):
+        time.sleep(0.2)
+    left = service_pids(sock)
+    for pid in left:       # the socket is the session's own: these servers were started by its tests
+        try:
+            os.kill(pid, signal.SIGTERM)
+        except ProcessLookupError:
+            pass
+    if left:
+        warnings.warn("elector_server %s did not leave within 60 s of the last test; terminated" % left)
+    shutil.rmtree(d, ignore_errors=True)
+
+
+def service_pids(sock):
+    """pids of the elector_server processes listening on `sock` (their argv is [exe, sock])"""
+    pids = []
+    for p in os.listdir("/proc"):
+        if not p.isdigit():
+            continue
+        try:
+            argv = open("/proc/%s/cmdline" % p, "rb").read().split(b"\0")
+        except OSError:
+            continue
+        if len(argv) >= 2 and argv[0].endswith(b"elector_server") and argv[1] == sock.encode():
+            pids.append(int(p))
+    return pids
+
+
 @pytest.fixture(scope="session")
 def emul_bin():
     """CPU build of the per-window device code (tests/emul/poa_emul.cu)."""
@@ -63,6 +109,18 @@ def emul_bin():
     exe = os.path.join(ROOT, "tests", "emul", "poa_emul")
     csrc = os.path.join(ROOT, "elector_b200", "csrc")
     deps = [src] + [os.path.join(csrc, f) for f in os.listdir(csrc)]
+    if not os.path.exists(exe) or any(os.path.getmtime(exe) < os.path.getmtime(p) for p in deps):
+        subprocess.check_call(["nvcc", "-O2", "-std=c++17", "-arch=sm_100a", "-Wno-deprecated-gpu-targets", "-o", exe, src])
+    return exe
+
+
+@pytest.fixture(scope="session")
+def split_emul_bin():
+    """CPU build of the window-cutting device code with the reference splitter's driver around it (tests/emul/split_emul.cu)."""
+    src = os.path.join(ROOT, "tests", "emul", "split_emul.cu")
+    exe = os.path.join(ROOT, "tests", "emul", "split_emul")
+    csrc = os.path.join(ROOT, "elector_b200", "csrc")
+    deps = [src, os.path.join(csrc, "split_kernel.cuh"), os.path.join(csrc, "split_host.hpp")]
     if not os.path.exists(exe) or any(os.path.getmtime(exe) < os.path.getmtime(p) for p in deps):
         subprocess.check_call(["nvcc", "-O2", "-std=c++17", "-arch=sm_100a", "-Wno-deprecated-gpu-targets", "-o", exe, src])
     return exe
@@ -119,19 +177,18 @@ def load_example_golden():
 
 
 @pytest.fixture(scope="session")
-def example_chain(tmp_path_factory):
+def example_chain(tmp_path_factory, split_emul_bin):
     """The README example up to the `poa` inputs: reads unpacked from tests/golden/example_reads.tar.xz, sorted and
-    duplicated like readAndSortFiles.py, cut into shard files by the compiled reference splitter (oracle/_ref travels
-    to the GPU box).  -> dict(work, out, shards, gold)"""
+    duplicated like readAndSortFiles.py, cut into shard files by the serial CPU build of the cutting code
+    (tests/emul/split_emul), whose shard files are those of the reference splitter: every one has the md5 the reference's
+    has in the golden (test_example_full.py, test_split_emul.py).  -> dict(work, out, shards, gold)"""
     from oracle import example_prep as ep
-    if not os.path.exists(os.path.join(ep.REF, "masterSplitter")):
-        pytest.skip("oracle/_ref/masterSplitter not built (oracle/build_ref.sh needs /root/reference)")
     src = str(tmp_path_factory.mktemp("example_src"))
     work = str(tmp_path_factory.mktemp("example_work"))
     ep.unpack(src)
     ep.sort_and_duplicate(src, work)
     out = os.path.join(work, "out")
-    rc, shards = ep.reference_split(work, out)
+    rc, shards = ep.reference_split(work, out, exe=split_emul_bin)
     assert rc == 0
     return {"src": src, "work": work, "out": out, "shards": shards, "gold": load_example_golden()}
 

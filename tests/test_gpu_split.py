@@ -1,9 +1,12 @@
-"""GPU: the window cutting on the device (SURVEY.md 8f-1) against the UNMODIFIED masterSplitter:
-  - the `masterSplitter` drop-in (elector_b200/bin/masterSplitter, alignment.py:99's command line) on the README example:
-    md5 of every shard file == tests/golden/example_full.json.gz;
-  - the same executable against the compiled reference (oracle/_ref travels to the GPU box) on synthetic reads of configs 1-4,
-    several rounds through progress.txt;
-  - elector_reads_run (reads in, windows never leave the device) == reference splitter -> elector_pipeline_run on the same reads."""
+"""GPU: the window cutting on the device (SURVEY.md 8f-1):
+  - the `masterSplitter` drop-in (elector_b200/bin/masterSplitter, alignment.py:99's command line) on the README example against
+    the UNMODIFIED masterSplitter: md5 of every shard file == tests/golden/example_full.json.gz;
+  - the same executable on synthetic reads of configs 1-4, several rounds through progress.txt, against the compiled reference
+    (oracle/_ref/masterSplitter, only where oracle/build_ref.sh has built it) and against the serial CPU build of the project's
+    own cutting code (tests/emul/split_emul: the same source, run one job after the other, so that check holds the parallel
+    device run to the serial one, not to the reference);
+  - elector_reads_run (reads in, windows never leave the device) == splitter -> elector_pipeline_run on the same reads, with
+    the same two splitters."""
 import os
 import subprocess
 
@@ -42,17 +45,18 @@ def test_dropin_cuts_the_example_like_the_reference(tmp_path):
     assert int(open(out + "/wrongly_cor_reads.txt").read()) == g["wrongly_cor_reads"]
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SPLITTER), reason="oracle/_ref/masterSplitter not built")
-@pytest.mark.parametrize("cfg,reads,amount,thr", [(1, 400, 10000, "0.1"), (2, 600, 10000, "0.1"), (3, 24, 10000, "0.1"), (4, 1500, 10000, "0.1"),
-                                                  (2, 300, 110, "0.4"), (4, 400, 150, "0.9")])
-def test_dropin_equals_compiled_reference_on_synthetic_reads(tmp_path, cfg, reads, amount, thr):
+SYNTHETIC_CUTS = [(1, 400, 10000, "0.1"), (2, 600, 10000, "0.1"), (3, 24, 10000, "0.1"), (4, 1500, 10000, "0.1"),
+                  (2, 300, 110, "0.4"), (4, 400, 150, "0.9")]
+
+
+def dropin_cuts_like(exe, tmp_path, cfg, reads, amount, thr):
     import workloads
     pre = str(tmp_path / "r")
     subprocess.check_call([workloads.ensure_gen(), str(cfg), str(reads), "0", pre])
     files = [pre + ".ref.fa", pre + ".unc.fa", pre + ".cor.fa"]
-    a, b = str(tmp_path / "ref"), str(tmp_path / "gpu")
+    a, b = str(tmp_path / "cpu"), str(tmp_path / "gpu")
     for rnd in range(8):
-        ra = run_splitter(REF_SPLITTER, files, a, amount, thr)
+        ra = run_splitter(exe, files, a, amount, thr)
         rb = run_splitter(drop_in(), files, b, amount, thr)
         assert ra == rb, rnd
         compare_dirs(a, b)
@@ -63,9 +67,29 @@ def test_dropin_equals_compiled_reference_on_synthetic_reads(tmp_path, cfg, read
 
 
 @pytest.mark.skipif(not os.path.exists(REF_SPLITTER), reason="oracle/_ref/masterSplitter not built")
+@pytest.mark.parametrize("cfg,reads,amount,thr", SYNTHETIC_CUTS)
+def test_dropin_equals_compiled_reference_on_synthetic_reads(tmp_path, cfg, reads, amount, thr):
+    dropin_cuts_like(REF_SPLITTER, tmp_path, cfg, reads, amount, thr)
+
+
+@pytest.mark.parametrize("cfg,reads,amount,thr", SYNTHETIC_CUTS)
+def test_dropin_equals_serial_cpu_cutting_on_synthetic_reads(tmp_path, split_emul_bin, cfg, reads, amount, thr):
+    dropin_cuts_like(split_emul_bin, tmp_path, cfg, reads, amount, thr)
+
+
+@pytest.mark.skipif(not os.path.exists(REF_SPLITTER), reason="oracle/_ref/masterSplitter not built")
 @pytest.mark.parametrize("cfg,reads", [(1, 300), (2, 400)])
 def test_reads_run_equals_reference_splitter_then_pipeline(tmp_path, cfg, reads):
-    """the chained call: per-triplet counters, merged rows and window counts equal what the reference splitter's windows give
+    reads_run_equals_splitter_then_pipeline(REF_SPLITTER, tmp_path, cfg, reads)
+
+
+@pytest.mark.parametrize("cfg,reads", [(1, 300), (2, 400)])
+def test_reads_run_equals_serial_cpu_cutting_then_pipeline(tmp_path, split_emul_bin, cfg, reads):
+    reads_run_equals_splitter_then_pipeline(split_emul_bin, tmp_path, cfg, reads)
+
+
+def reads_run_equals_splitter_then_pipeline(exe, tmp_path, cfg, reads):
+    """the chained call: per-triplet counters, merged rows and window counts equal what the splitter's windows give
     through elector_pipeline_run (itself held to the reference poa / Donatello / computeStats by the other GPU tests)"""
     import elector_b200
     import workloads
@@ -75,8 +99,8 @@ def test_reads_run_equals_reference_splitter_then_pipeline(tmp_path, cfg, reads)
     _, unc, uo = workloads.parse_two_line_fasta(pre + ".unc.fa")
     _, cor, co = workloads.parse_two_line_fasta(pre + ".cor.fa")
     n = len(hr)
-    out = str(tmp_path / "ref")
-    assert run_splitter(REF_SPLITTER, [pre + ".ref.fa", pre + ".unc.fa", pre + ".cor.fa"], out, 10000, "0.1") == 0
+    out = str(tmp_path / "cut")
+    assert run_splitter(exe, [pre + ".ref.fa", pre + ".unc.fa", pre + ".cor.fa"], out, 10000, "0.1") == 0
     heads, parts = [], {q: ([], [np.zeros(1, np.int64)], 0) for q in (1, 2, 3)}
     for i in range(200):
         if os.path.getsize("%s/out3%d" % (out, i)) == 0:

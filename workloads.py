@@ -20,7 +20,8 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 SPLITTER = os.path.join(ROOT, "oracle", "_ref", "masterSplitter")
 GEN = os.path.join(ROOT, "tools", "gen_reads")
-CACHE = os.environ.get("ELECTOR_CACHE", "/tmp/elector_b200_cache")
+# per user: a directory another user created first is not writable
+CACHE = os.environ.get("ELECTOR_CACHE", os.path.join(tempfile.gettempdir(), "elector_b200_cache_%d" % os.getuid()))
 
 CONFIG_NAMES = {
     1: "synthetic 10k triplets, 10 kb reads, 10% raw / 1% corrected error",
