@@ -3,8 +3,9 @@
 The reference runs, per round of 10 001 triplets: one `masterSplitter` process (alignment.py:98-100), up to 200 `poa` processes through
 a multiprocessing.Pool (fpoa, :59-63, :117-119), 200 `Donatello` processes (:120-124) and two `rm` shells over ~800 temporary files.
 `getPOA` here has the reference's signature, return value and output file (`<outDir>/msa.fa` or `msa_<soft>.fa`, same bytes), and is one
-C-ABI call per batch of triplets on a context that stays alive between calls (elector_reads_run: the windows never leave the device);
-no process is started and no temporary file is written.  The per-read counters of the last call are kept for computeStats.py's
+C-ABI call per batch of triplets on a context that stays alive between calls (elector_reads_pipeline_run: the windows never leave the
+device; the library cuts the call into chunks that run on worker contexts of one or more devices: ELECTOR_DEVICES="0,1,..", else the
+context's device ELECTOR_DEVICE); no process is started and no temporary file is written.  The per-read counters of the last call are kept for computeStats.py's
 replacement (elector_b200/computeStats.py), which then needs no tally pass over msa.fa at all."""
 import os
 
@@ -13,7 +14,7 @@ import numpy as np
 from .poa import PoaContext
 
 _CTX = None
-BATCH_TRIPLETS = 20000     # triplets per device call (a call holds their letters, windows and MSA rows: ~1.5 GB at 10 kb reads)
+BATCH_TRIPLETS = 200000    # triplets per call: bounds the host buffers of the merged rows (3 x the letters of a batch); the device side is chunked by the library
 LAST = None                # what the last getPOA left for the report: dict(headers, counters, stretches, msa_path)
 
 
@@ -23,6 +24,12 @@ def context(device=None):
     if _CTX is None:
         _CTX = PoaContext(int(os.environ.get("ELECTOR_DEVICE", "0")) if device is None else device)
     return _CTX
+
+
+def devices():
+    """the devices of the reads-in call: ELECTOR_DEVICES="0,1,..", else None (the context's own device)"""
+    e = os.environ.get("ELECTOR_DEVICES", "").strip()
+    return [int(d) for d in e.split(",") if d.strip()] if e else None
 
 
 def read_two_line_fasta(path):
@@ -57,7 +64,7 @@ def pir_header(h):
 
 
 def getPOA(corrected, reference, uncorrected, threads, outDir, SIZE_CORRECTED_READ_THRESHOLD, soft=None):
-    """alignment.py:66-131 (oldMode False).  `threads` is accepted and ignored: the device runs every window of a batch at once."""
+    """alignment.py:66-131 (oldMode False).  `threads` is accepted and ignored: the devices run every window of a batch at once."""
     global LAST
     ctx = context()
     merge_out = outDir + ("/msa_" + soft + ".fa" if soft is not None else "/msa.fa")
@@ -82,8 +89,9 @@ def getPOA(corrected, reference, uncorrected, threads, outDir, SIZE_CORRECTED_RE
                 pos = np.repeat(off[idx] - o[:-1], lens) + np.arange(o[-1])
                 return let[pos], o
             (r, r_o), (u, u_o), (c, c_o) = gather(ref, ro), gather(unc, uo), gather(cor, co)
-            got = ctx.reads_run(r, r_o, u, u_o, c, c_o, [len(hr[t]) for t in idx], float(SIZE_CORRECTED_READ_THRESHOLD), merged=True)
-            st = ctx.last_stretches(len(idx))
+            got = ctx.reads_pipeline(r, r_o, u, u_o, c, c_o, [len(hr[t]) for t in idx], float(SIZE_CORRECTED_READ_THRESHOLD), merged=True,
+                                     devices=devices())
+            st = got["stretches"]
             small_reads += int((got["status"] == 1).sum())
             wrongly_cor_reads += int((got["status"] == 2).sum())
             chunks = []

@@ -83,6 +83,7 @@ struct elector_ctx {
   int64_t merged_cap = 0;  // bytes per merged-row buffer of the last merge
   // pipelined host entry point: child contexts (one per extra worker thread), per-worker sums and status of the call
   std::vector<elector_ctx *> workers;
+  std::vector<elector_ctx *> peers;   // worker contexts of elector_reads_pipeline_run on the other devices
   int64_t pipe_sums[ELECTOR_TALLY_K] = {};
   int64_t *h_sums = nullptr;   // pinned: global counters of a chunk + the tally overflow flag
   int pipe_rc = 0;
@@ -1005,6 +1006,9 @@ void elector_poa_free(elector_ctx *ctx) {
   elector_split_release(ctx);
   for (elector_ctx *w : ctx->workers) elector_poa_free(w);
   ctx->workers.clear();
+  for (elector_ctx *w : ctx->peers) { cudaSetDevice(w->device); elector_poa_free(w); }   // their buffers and streams belong to their device
+  if (!ctx->peers.empty()) cudaSetDevice(ctx->device);
+  ctx->peers.clear();
   if (ctx->h_sums) cudaFreeHost(ctx->h_sums);
   DevBuf *bufs[] = {&ctx->d_tab, &ctx->d_ref, &ctx->d_cor, &ctx->d_unc, &ctx->d_roff, &ctx->d_coff, &ctx->d_uoff,
                     &ctx->d_items, &ctx->d_scratch, &ctx->d_scratch_lin, &ctx->d_scratch2, &ctx->d_ctrl, &ctx->d_hist, &ctx->d_bintab, &ctx->d_key, &ctx->d_key2, &ctx->d_n1, &ctx->d_p1, &ctx->d_rows, &ctx->d_rowoff, &ctx->d_stride,

@@ -73,6 +73,8 @@ def load_library():
     lib.elector_split_run.restype = c.c_int
     lib.elector_reads_run.argtypes = [vp, c.c_int64] + [vp] * 7 + [c.c_double] + [vp] * 9 + [c.c_int64, vp, vp]
     lib.elector_reads_run.restype = c.c_int
+    lib.elector_reads_pipeline_run.argtypes = [vp, vp]
+    lib.elector_reads_pipeline_run.restype = c.c_int
     lib.elector_last_reads_ms.argtypes = [vp, c.POINTER(c.c_float), c.POINTER(c.c_float), c.POINTER(c.c_float)]
     lib.elector_last_reads_ms.restype = c.c_int
     lib.elector_last_stretches.argtypes = [vp, c.c_int64, vp]

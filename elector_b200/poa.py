@@ -41,6 +41,27 @@ class PipelineIoC(ctypes.Structure):  # struct elector_pipeline_io
                 ("ref_len16", ctypes.c_void_p), ("cor_len16", ctypes.c_void_p), ("unc_len16", ctypes.c_void_p)]
 
 
+class ReadsIoC(ctypes.Structure):     # struct elector_reads_io
+    _fields_ = [("n_triplets", ctypes.c_int64),
+                ("ref", ctypes.c_void_p), ("unc", ctypes.c_void_p), ("cor", ctypes.c_void_p),
+                ("ref_off", ctypes.c_void_p), ("unc_off", ctypes.c_void_p), ("cor_off", ctypes.c_void_p),
+                ("header_len", ctypes.c_void_p), ("threshold", ctypes.c_double),
+                ("devices", ctypes.c_void_p), ("n_devices", ctypes.c_int),
+                ("status", ctypes.c_void_p), ("k_used", ctypes.c_void_p),
+                ("read_first", ctypes.c_void_p), ("n_windows", ctypes.c_void_p),
+                ("counters_out", ctypes.c_void_p), ("sums_out", ctypes.c_void_p),
+                ("stretches_out", ctypes.c_void_p),
+                ("m_ref", ctypes.c_void_p), ("m_cor", ctypes.c_void_p), ("m_unc", ctypes.c_void_p),
+                ("m_off", ctypes.c_void_p), ("m_len", ctypes.c_void_p), ("m_cap", ctypes.c_int64)]
+
+
+def reads_merged_bound(ref_off, unc_off, cor_off):
+    """bytes per merged-row buffer that elector_reads_pipeline_run needs: letters of the call + 32 per triplet, rounded up to 16"""
+    n = len(ref_off) - 1
+    letters = sum(int(o[n] - o[0]) for o in (ref_off, unc_off, cor_off))
+    return (letters + 32 * n + 15) & ~15
+
+
 @dataclass
 class PackedLetters:
     """2 bits per letter + the exceptions (elector_pack_letters)"""
@@ -292,6 +313,41 @@ class PoaContext:
                                                 float(threshold), _p(status), _p(k_used), _p(read_first), ctypes.cast(ctypes.byref(nw), ctypes.c_void_p),
                                                 _p(counters), _p(sums), _p(m[0]), _p(m[1]), _p(m[2]), m_cap, _p(m_off), _p(m_len)))
         out = dict(status=status, k_used=k_used, read_first=read_first, n_windows=int(nw.value), counters=counters, sums=sums)
+        if merged:
+            out.update(m_ref=m[0], m_cor=m[1], m_unc=m[2], m_off=m_off, m_len=m_len)
+        return out
+
+    def reads_pipeline(self, ref, ref_off, unc, unc_off, cor, cor_off, header_len, threshold=0.1, merged=False, devices=None, m_cap=None):
+        """reads_run for any number of triplets (elector_reads_pipeline_run): the call is cut into chunks of whole triplets that run on
+        worker contexts of `devices` (None: this context's device; a device may be listed more than once).  -> the dict of reads_run
+        plus "stretches" (int32[n, 17], what last_stretches gives after reads_run).  m_cap: merged-row capacity (default: the bound)."""
+        n = len(ref_off) - 1
+        ref_off, unc_off, cor_off = (np.ascontiguousarray(o, dtype=np.int64) for o in (ref_off, unc_off, cor_off))
+        ref, unc, cor = (np.ascontiguousarray(s, dtype=np.uint8) for s in (ref, unc, cor))
+        header_len = np.ascontiguousarray(header_len, dtype=np.int32)
+        status, k_used = np.zeros(n, np.int32), np.zeros(n, np.int32)
+        read_first = np.zeros(n + 1, np.int64)
+        counters = np.zeros((n, len(TALLY_FIELDS)), dtype=np.int64)
+        sums = np.zeros(len(TALLY_FIELDS), dtype=np.int64)
+        stretches = np.zeros((n, 17), dtype=np.int32)
+        nw = np.zeros(1, np.int64)
+        io = ReadsIoC()
+        io.n_triplets = n
+        io.ref, io.unc, io.cor = ref.ctypes.data, unc.ctypes.data, cor.ctypes.data
+        io.ref_off, io.unc_off, io.cor_off = ref_off.ctypes.data, unc_off.ctypes.data, cor_off.ctypes.data
+        io.header_len, io.threshold = header_len.ctypes.data, float(threshold)
+        dev = np.ascontiguousarray(devices if devices is not None else [], dtype=np.intc)
+        io.devices, io.n_devices = (dev.ctypes.data if len(dev) else None), len(dev)
+        io.status, io.k_used, io.read_first, io.n_windows = status.ctypes.data, k_used.ctypes.data, read_first.ctypes.data, nw.ctypes.data
+        io.counters_out, io.sums_out, io.stretches_out = counters.ctypes.data, sums.ctypes.data, stretches.ctypes.data
+        if merged:
+            cap = reads_merged_bound(ref_off, unc_off, cor_off) if m_cap is None else int(m_cap)
+            m = [np.zeros(max(cap, 1), np.uint8) for _ in range(3)]
+            m_off, m_len = np.zeros(n, np.int64), np.zeros(n, np.int32)
+            io.m_ref, io.m_cor, io.m_unc = (b.ctypes.data for b in m)
+            io.m_off, io.m_len, io.m_cap = m_off.ctypes.data, m_len.ctypes.data, cap
+        self._check(self._lib.elector_reads_pipeline_run(self._ctx, ctypes.byref(io)))
+        out = dict(status=status, k_used=k_used, read_first=read_first, n_windows=int(nw[0]), counters=counters, sums=sums, stretches=stretches)
         if merged:
             out.update(m_ref=m[0], m_cor=m[1], m_unc=m[2], m_off=m_off, m_len=m_len)
         return out

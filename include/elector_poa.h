@@ -247,12 +247,48 @@ int elector_reads_run(elector_ctx *ctx, int64_t n_triplets, const char *ref, con
                       const int64_t *unc_off, const char *cor, const int64_t *cor_off, const int32_t *header_len, double threshold,
                       int32_t *status, int32_t *k_used, int64_t *read_first, int64_t *n_windows, int64_t *counters_out,
                       int64_t *sums_out, char *m_ref, char *m_cor, char *m_unc, int64_t m_cap, int64_t *m_off, int32_t *m_len);
-/* Device time of the last elector_reads_run: window cutting, alignment, merge + tally (CUDA events, ms). */
+/* Device time of the last elector_reads_run or elector_reads_pipeline_run (summed over its chunks): window cutting, alignment,
+ * merge + tally (CUDA events, ms). */
 int elector_last_reads_ms(const elector_ctx *ctx, float *ms_split, float *ms_poa, float *ms_merge_tally);
+
+/* ---- pipelined reads-in call ------------------------------------------------------------------------------------------
+ * Replaces: one or more rounds of elector/alignment.py:98-129 -- masterSplitter (Master_Splitter.cpp:352-472), Pool(fpoa)
+ * (main.c:265-284 per window), Donatello (Donatello.cpp:50-84) and the integer part of computeStats.py -- for any number of
+ * triplets in one call.  The call is cut into chunks of whole triplets (balanced by letters); each chunk runs the body of
+ * elector_reads_run start to finish on one worker context (own host thread and stream), so that one chunk's copies overlap
+ * another chunk's kernels, and the workers may sit on several devices.  Inputs as elector_reads_run, plus the devices:
+ * devices[0 .. n_devices - 1] (NULL / 0: the context's own device; a device may be listed more than once); every listed device
+ * gets ELECTOR_PIPELINE_WORKERS worker contexts (default 2), created on first use and kept until elector_poa_free.
+ * ELECTOR_PIPELINE_CHUNKS forces the number of chunks.  Every output may be NULL and is byte-identical to one elector_reads_run
+ * over the same triplets, however the call is chunked, except where m_off places the merged rows:
+ *   status[n], k_used[n], read_first[n + 1] (global window indices), *n_windows,
+ *   counters_out[n][ELECTOR_TALLY_K], sums_out[ELECTOR_TALLY_K],
+ *   stretches_out[n][ELECTOR_STRETCH_K]: what elector_last_stretches gives after elector_reads_run,
+ *   the merged rows of triplet t: m_len[t] bytes at m_off[t] of m_ref / m_cor / m_unc (all five or none).
+ * Placement rule: the rows of triplet t start at or after the bound of the triplets before it, B(t) = (letters of triplets
+ * 0 .. t-1 in the three kinds + 32 * t) rounded down to 16, so that every chunk writes into the caller's buffers at once.
+ * m_cap must be at least the bound of the call, letters of all triplets + 32 * n rounded up to 16; a smaller m_cap
+ * returns ELECTOR_ECAPACITY before any work.  A failure on any worker stops the others at their next chunk; the call returns
+ * that error and its text. */
+typedef struct elector_reads_io {
+  int64_t n_triplets;
+  const char *ref, *unc, *cor;                    /* letters as bytes, as in the FASTA files */
+  const int64_t *ref_off, *unc_off, *cor_off;     /* n_triplets + 1 offsets each */
+  const int32_t *header_len;                      /* length of each triplet's header line */
+  double threshold;                               /* SIZE_CORRECTED_READ_THRESHOLD */
+  const int *devices; int n_devices;
+  int32_t *status, *k_used;
+  int64_t *read_first, *n_windows;
+  int64_t *counters_out, *sums_out;
+  int32_t *stretches_out;
+  char *m_ref, *m_cor, *m_unc; int64_t *m_off; int32_t *m_len; int64_t m_cap;
+} elector_reads_io;
+
+int elector_reads_pipeline_run(elector_ctx *ctx, const elector_reads_io *io);
 
 /* ---- report (SURVEY.md 8f-2) -------------------------------------------------------------------------------------------
  * The border gap stretches of every read of the last tally on this context (elector_tally_run, elector_merge_tally_device,
- * elector_reads_run; not the chunked elector_pipeline_run*): what findGapStretches keeps (computeStats.py:179-189), as
+ * elector_reads_run; not the chunked elector_pipeline_run*; elector_reads_pipeline_run returns them in stretches_out): what findGapStretches keeps (computeStats.py:179-189), as
  * stretches_out[r*ELECTOR_STRETCH_K] = their number and (first, last) column pairs behind it.  With gapsLeft / gapsRight they
  * rebuild the column mask of getCorrectedPositions (:712-752). */
 #define ELECTOR_STRETCH_K 17
