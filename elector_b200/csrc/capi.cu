@@ -75,7 +75,7 @@ struct elector_ctx {
   cudaEvent_t ev_join[16] = {};
   elector::BinTable *h_bintab = nullptr;  // pinned: the two tables of the last call as the device left them (errors, scratch needs)
   cudaStream_t copy_in = nullptr, copy_out = nullptr;   // H2D / D2H of the pipelined host entry point
-  std::vector<cudaEvent_t> chunk_ev;                    // 2 per chunk: inputs resident, results ready
+  cudaEvent_t ev_call = nullptr;                        // ELECTOR_TRACE: start of a pipelined call on the device
   ScoreMatrix mat;
   ScoringSetup sc;
   DevBuf d_tab, d_ref, d_cor, d_unc, d_roff, d_coff, d_uoff, d_items, d_scratch, d_scratch_lin, d_scratch2, d_ctrl, d_hist, d_bintab, d_key, d_key2, d_n1, d_p1;
@@ -93,19 +93,13 @@ struct elector_ctx {
   DevBuf d_wdst, d_sums, d_tally_scan, d_tally_out, d_readfirst, d_mtot, d_moff, d_mlen, d_mref, d_mcor, d_munc;
   bool trace = false;
   int band_w = 6;          // ELECTOR_BAND_W: base half-width of the diagonal band of the packed linear kernels (+ rows/16 in phase 1, + rows/8 in phase 2; 0 = full DP)
-  bool no_dual = false;    // ELECTOR_NO_DUAL=1: general windows of phase 2 on the INT32 kernel with frontier sets
-  int resident_ph2d = 0;
-  int coop_mid = 3;        // ELECTOR_COOP_MID: bit 0 / bit 1 = the windows of 129 .. 256 rows run a warp per window in phase 1 / phase 2 (else thread-per-window, packed kernels)
-  bool no_ident = false;   // ELECTOR_NO_IDENT=1: windows whose cor is ref run DP1 like every other window
+  int resident_ph2d = 0;   // 0: the general windows of phase 2 run the INT32 kernel with frontier sets
   unsigned side_used = 0;        // side streams with launches that `st` has not been made to wait for yet
-  bool async_launch = false;     // ELECTOR_ASYNC_LAUNCH=1: no read-back of the plans; every segment is launched with a fixed grid (no host wait inside a call)
-  bool plans_on_host = false;
-  elector::BinTable *h_plan = nullptr;   // pinned: the plans of phase 1 / phase 2 of the current call
+  elector::BinTable *h_plan = nullptr;   // pinned: the plans of phase 1 / phase 2 of the current call (read_plans)
   // rows of a pipelined chunk in two regions: the windows of the linear segments of phase 2 (most windows, finished early)
   // write theirs behind their own cursor, so that they can leave for the host while the general windows still compute
   bool split_rows = false;          // set by process_chunk around run_device
   int64_t region_b_base = 0;        // out: where the linear region starts in the caller's row buffer
-  cudaEvent_t ev_regb[8] = {};      // after each launch that writes to the linear region
   cudaEvent_t ev_lin = nullptr;     // the linear region is complete; its cursor and start are in h_totals[6..7]
   cudaEvent_t ev_merged = nullptr;  // the merge of a chunk is done and its rows are packed for the wire (before the tally); the merged columns of the chunk are in h_totals[2]
   cudaEvent_t wait_in[2] = {nullptr, nullptr};   // run_device: phase 1 / phase 2 wait for these (letters still on their way), when set
@@ -180,10 +174,9 @@ cudaError_t launch_phase(int phase, int kind, cudaStream_t st, PoaArgs &a, int g
 // shared memory that keeps it: the SM's shared memory divided among the resident CTAs, minus the kernel's static part and
 // the 1 KB the system reserves per CTA.
 template <class K>
-void size_arena(K kernel, size_t smem_per_sm, int cap_warps, int &resident, int &arena_bytes) {
+void size_arena(K kernel, size_t smem_per_sm, int &resident, int &arena_bytes) {
   cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kernel, 32, 0);
-  if (cap_warps > 0 && cap_warps < resident) resident = cap_warps;
   arena_bytes = 0;
   if (resident < 1) return;
   cudaFuncAttributes fa;
@@ -200,18 +193,15 @@ void size_arena(K kernel, size_t smem_per_sm, int cap_warps, int &resident, int 
 
 template <bool GS>
 void resident_warps_per_sm(elector_ctx *ctx, size_t smem_per_sm) {
-  auto cap = [](const char *name) { const char *e = getenv(name); return e ? atoi(e) : 0; };
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->resident_coop, poa_dp2_coop_kernel<GS>, 32, 0);
   int coop1 = 0;
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&coop1, poa_dp1_coop_kernel<GS>, 32, 0);
   ctx->resident_coop = std::min(ctx->resident_coop, coop1);
-  // experiment knobs ELECTOR_WARPS_*: cap the resident warps per SM of a kernel (scratch footprint and arena size vs. latency hiding)
-  size_arena(poa_dp2_kernel<Phase2L, EL_MIN_WARPS_PH2L>, smem_per_sm, cap("ELECTOR_WARPS_PH2L"), ctx->resident_ph2l, ctx->arena_ph2l);
-  size_arena(poa_dp1_kernel<Phase1<GS>, EL_MIN_WARPS_PH1>, smem_per_sm, cap("ELECTOR_WARPS_PH1"), ctx->resident_ph1, ctx->arena_ph1);
-  size_arena(poa_dp2_kernel<Phase2<GS>, EL_MIN_WARPS_PH2>, smem_per_sm, cap("ELECTOR_WARPS_PH2"), ctx->resident_ph2, ctx->arena_ph2);
-  size_arena(poa_dp1_kernel<Phase1P, EL_MIN_WARPS_PH1P>, smem_per_sm, cap("ELECTOR_WARPS_PH1P"), ctx->resident_ph1p, ctx->arena_ph1p);
-  size_arena(poa_dp2_kernel<Phase2D, EL_MIN_WARPS_PH2D>, smem_per_sm, cap("ELECTOR_WARPS_PH2D"), ctx->resident_ph2d, ctx->arena_ph2d);
-  if (const char *e = getenv("ELECTOR_NO_ARENA")) if (e[0] == '1') ctx->arena_ph1 = ctx->arena_ph2 = ctx->arena_ph1p = ctx->arena_ph2l = ctx->arena_ph2d = 0;
+  size_arena(poa_dp2_kernel<Phase2L, EL_MIN_WARPS_PH2L>, smem_per_sm, ctx->resident_ph2l, ctx->arena_ph2l);
+  size_arena(poa_dp1_kernel<Phase1<GS>, EL_MIN_WARPS_PH1>, smem_per_sm, ctx->resident_ph1, ctx->arena_ph1);
+  size_arena(poa_dp2_kernel<Phase2<GS>, EL_MIN_WARPS_PH2>, smem_per_sm, ctx->resident_ph2, ctx->arena_ph2);
+  size_arena(poa_dp1_kernel<Phase1P, EL_MIN_WARPS_PH1P>, smem_per_sm, ctx->resident_ph1p, ctx->arena_ph1p);
+  size_arena(poa_dp2_kernel<Phase2D, EL_MIN_WARPS_PH2D>, smem_per_sm, ctx->resident_ph2d, ctx->arena_ph2d);
 }
 
 // ---- device-side planning of a sort view's segments --------------------------------------------------------------
@@ -304,12 +294,13 @@ struct SortView {
 // kernel of a segment (static: known before the sort runs, see SegStatic)
 int seg_kind(const elector_ctx *ctx, int phase, int s) {
   const bool small16 = ctx->sc.packed_ok && (int64_t)ctx->sc.maxabs * (kSmallMax + 4 * kN1q + 4) <= kPackedSpan;   // no score of a small window leaves 16 bits
-  const int coop_last = (ctx->coop_mid & (phase == 1 ? 1 : 2)) ? kBigTiers : kBigTiers - 1;   // last segment that runs a warp per window
-  if (phase == 1) return (s <= coop_last && ctx->coop_group > 0) ? kCoop : (s >= kBigTiers && small16) ? kPacked : kInt32;
-  const bool longest = s <= coop_last || (s == kFirstLinSeg2 && (ctx->coop_mid & 2));   // more than 128 rows: a warp per window
+  // windows of more than 128 rows run a warp per window: the big tiers and the first small segment (129 .. 256 rows) of phase 1,
+  // of the general and of the linear segments of phase 2
+  if (phase == 1) return (s <= kBigTiers && ctx->coop_group > 0) ? kCoop : (s >= kBigTiers && small16) ? kPacked : kInt32;
+  const bool longest = s <= kBigTiers || s == kFirstLinSeg2;
   if (longest && ctx->coop_group > 0) return kCoop;
   if (s < kBigTiers || !small16) return kInt32;
-  return s >= kFirstLinSeg2 ? kLinear : ctx->no_dual ? kInt32 : kDual;
+  return s >= kFirstLinSeg2 ? kLinear : ctx->resident_ph2d > 0 ? kDual : kInt32;
 }
 int seg_resident(const elector_ctx *ctx, int phase, int kind) {
   switch (kind) {
@@ -351,8 +342,7 @@ int sort_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, int32_t n, i
 // would serialise them.
 int launch_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, const SegStatic &ss, PoaArgs base, int first_side, bool region_b, int64_t n, int which = 2) {
   cudaEvent_t fork = ctx->ev_fork_v[(v.phase == 1 ? 0 : v.seg0 >= kFirstLinSeg2 ? 1 : 2) + (which == 1 ? 3 : 0)];
-  // exact mode (read_plans): only the segments that have work are launched, with the grids the device planned
-  const BinTable *host_tab = ctx->plans_on_host ? &ctx->h_plan[v.phase - 1] : nullptr;
+  const BinTable &plans = ctx->h_plan[v.phase - 1];   // read_plans
   CU(cudaEventRecord(fork, st));
   const int vi = v.phase == 1 ? 0 : v.seg0 >= kFirstLinSeg2 ? 1 : 2;
   if (ctx->trace) for (int w2 = 0; w2 < 2; ++w2) if (which == 2 || which == w2) CU(cudaEventRecord(ctx->ev_view[vi][w2][0], st));
@@ -362,11 +352,11 @@ int launch_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, const SegS
     for (int s = v.seg0; s < v.seg1; ++s) {
       const int kind = ss.kind[s];
       if ((kind == kCoop) != (pass == 0) || (which != 2 && which != pass)) continue;
-      if (host_tab && host_tab->plan[s].max_ctas == 0) continue;
-      const int grid = host_tab ? host_tab->plan[s].max_ctas : ss.grid[s];
-      // bulk: by its share of the windows when the plans are here, else the segments of the small windows (where the bulk of
-      // ELECTOR's windows is: at most 64 rows)
-      const bool bulk = kind != kCoop && (host_tab ? (int64_t)host_tab->plan[s].count * 8 > n : s >= v.seg1 - 2);
+      // only the segments that have work are launched, with the grids the device planned
+      const SegPlanDev &pl = plans.plan[s];
+      if (pl.max_ctas == 0) continue;
+      const int grid = pl.max_ctas;
+      const bool bulk = kind != kCoop && (int64_t)pl.count * 8 > n;
       const int side = first_side + (s - v.seg0);
       cudaStream_t ls = bulk ? st : ctx->side[side];
       if (!bulk) CU(cudaStreamWaitEvent(ls, fork, 0));
@@ -384,16 +374,13 @@ int launch_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, const SegS
     }
   return ELECTOR_OK;
 }
-// The plans of a phase, read back (one wait of the host per phase): without ELECTOR_ASYNC_LAUNCH=1 the host launches only the
-// segments that have work, with exact grids.  Measured on config 1: fixed-grid launches of all 27 segments (most of them
-// empty, thousands of CTAs that leave at once) cost 0.4 ms per phase, a read-back 0.03 ms.
+// The plans of a phase, read back (one wait of the host per phase): the host launches only the segments that have work, with
+// exact grids.  Measured on config 1: fixed-grid launches of all 27 segments (most of them empty, thousands of CTAs that leave
+// at once) cost 0.4 ms per phase, a read-back 0.03 ms.
 int read_plans(elector_ctx *ctx, int phase, BinTable *dtab, cudaStream_t a, cudaStream_t b) {
-  ctx->plans_on_host = false;
-  if (ctx->async_launch) return ELECTOR_OK;
   if (b) CU(cudaStreamSynchronize(b));
   CU(cudaMemcpyAsync(&ctx->h_plan[phase - 1], dtab, sizeof(BinTable), cudaMemcpyDeviceToHost, a));
   CU(cudaStreamSynchronize(a));
-  ctx->plans_on_host = true;
   return ELECTOR_OK;
 }
 // `st` waits for the side streams side[first .. first + count - 1] that have launched something since the last join
@@ -438,7 +425,7 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
     for (int k = 0; k < 4; ++k) tot[k] = ctx->h_totals[k];
   }
   CU(ctx->d_p1.reserve((size_t)(tot[0] - tot[2] + tot[1] - tot[3] + 8 * n + 8) * sizeof(uint16_t)));
-  // scratch pools: kept from call to call; a call that needs more says so in its tables and is run again (run_checked)
+  // scratch pools: kept from call to call; a call that needs more says so in its tables and its caller runs it again (check_tables)
   for (DevBuf *pool : {&ctx->d_scratch, &ctx->d_scratch_lin, &ctx->d_scratch2})
     if (pool->cap == 0) CU(pool->reserve(std::max<size_t>((size_t)64 << 20, std::min<size_t>((size_t)n * 1024, (size_t)2 << 30))));
   CU(cudaEventRecord(ctx->ev0, st));
@@ -463,7 +450,7 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   // windows whose corrected letters are the reference letters need no phase 1 (bin_kernel.cuh): the sort then reads the
   // letters, so it waits for them too.  Only when their phase 2 needs no node list: Phase2L for the small linear segments,
   // the warp-cooperative kernel (which rebuilds lin(ref)) for the long ones.
-  const bool ident_ok = ctx->sc.packed_ok && !ctx->no_ident && ctx->coop_group > 0 &&
+  const bool ident_ok = ctx->sc.packed_ok && ctx->coop_group > 0 &&
                         (int64_t)ctx->sc.maxabs * (kSmallMax + 4 * kN1q + 4) <= kPackedSpan;
   if (ident_ok && ctx->wait_in[0]) CU(cudaStreamWaitEvent(st, ctx->wait_in[0], 0));
   IdentArgs ida{(const uint8_t *)d_ref, (const uint8_t *)d_cor, ctx->d_n1.as<int32_t>(), ctx->d_key2.as<int32_t>(), hist2, dtab2->seg_max, d_s1, &dtab2->lin_bytes};
@@ -914,10 +901,6 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
   ctx->mat = mat;
   if (!ctx->sc.analyse(ctx->mat)) { ctx->err = ctx->sc.error; return bail(ELECTOR_EUNSUPPORTED); }
   ctx->trace = getenv("ELECTOR_TRACE") != nullptr;
-  if (const char *e = getenv("ELECTOR_NO_IDENT")) ctx->no_ident = e[0] == '1';
-  if (const char *e = getenv("ELECTOR_COOP_MID")) ctx->coop_mid = atoi(e) & 3;
-  if (const char *e = getenv("ELECTOR_ASYNC_LAUNCH")) ctx->async_launch = e[0] == '1';
-  if (const char *e = getenv("ELECTOR_NO_DUAL")) ctx->no_dual = e[0] == '1';
   if (const char *e = getenv("ELECTOR_BAND_W")) ctx->band_w = std::max(0, std::min(64, atoi(e)));
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
@@ -934,8 +917,7 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
   ctx->smem_optin = prop.sharedMemPerBlockOptin;
   int prio_lo = 0, prio_hi = 0;
   cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);   // numerically lower = higher priority
-  int prio = std::min(prio_lo, prio_hi + worker);
-  if (const char *pe = getenv("ELECTOR_NO_PRIORITIES")) if (pe[0] == '1') prio = prio_lo;
+  const int prio = std::min(prio_lo, prio_hi + worker);
   if ((e = cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio)) != cudaSuccess ||
       (e = cudaEventCreate(&ctx->ev0)) != cudaSuccess || (e = cudaEventCreate(&ctx->ev1)) != cudaSuccess ||
       (e = cudaEventCreate(&ctx->ev_mid)) != cudaSuccess ||
@@ -947,6 +929,7 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
       (e = cudaEventCreateWithFlags(&ctx->ev_in[0], cudaEventDisableTiming)) != cudaSuccess ||
       (e = cudaEventCreateWithFlags(&ctx->ev_in[1], cudaEventDisableTiming)) != cudaSuccess ||
       (e = cudaEventCreate(&ctx->uev0)) != cudaSuccess || (e = cudaEventCreate(&ctx->uev1)) != cudaSuccess ||
+      (e = cudaEventCreate(&ctx->ev_call)) != cudaSuccess ||
       (e = cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming)) != cudaSuccess ||
       (e = cudaStreamCreateWithPriority(&ctx->lin_stream, cudaStreamNonBlocking, prio)) != cudaSuccess ||
       (e = cudaEventCreateWithFlags(&ctx->ev_sorted, cudaEventDisableTiming)) != cudaSuccess ||
@@ -971,11 +954,6 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
       ctx->fail(ELECTOR_ECUDA, "context setup: %s", cudaGetErrorString(e));
       return bail(ELECTOR_ECUDA);
     }
-  for (int k = 0; k < 8; ++k)
-    if ((e = cudaEventCreateWithFlags(&ctx->ev_regb[k], cudaEventDisableTiming)) != cudaSuccess) {
-      ctx->fail(ELECTOR_ECUDA, "context setup: %s", cudaGetErrorString(e));
-      return bail(ELECTOR_ECUDA);
-    }
   for (int k = 0; k < kSideStreams; ++k)
     if ((e = cudaStreamCreateWithPriority(&ctx->side[k], cudaStreamNonBlocking, prio)) != cudaSuccess ||
         (e = cudaEventCreateWithFlags(&ctx->ev_join[k], cudaEventDisableTiming)) != cudaSuccess) {
@@ -986,8 +964,6 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
   else resident_warps_per_sm<false>(ctx, prop.sharedMemPerMultiprocessor);
   if (const char *e = getenv("ELECTOR_COOP_GROUP")) ctx->coop_group = std::max(0, std::min(32, atoi(e)));
   if (ctx->resident_coop < 1) ctx->coop_group = 0;
-  if (const char *e = getenv("ELECTOR_WARPS_COOP")) { const int c = atoi(e); if (c > 0 && c < ctx->resident_coop) ctx->resident_coop = c; }
-  if (ctx->resident_ph2d < 1) ctx->no_dual = true;
   if (ctx->trace)
     fprintf(stderr, "[elector trace] resident warps / arena bytes per warp: Phase1P %d / %d, Phase2L %d / %d, Phase2D %d / %d, Phase1 %d / %d, Phase2 %d / %d, coop %d\n",
             ctx->resident_ph1p, ctx->arena_ph1p, ctx->resident_ph2l, ctx->arena_ph2l, ctx->resident_ph2d, ctx->arena_ph2d, ctx->resident_ph1, ctx->arena_ph1,
@@ -1021,7 +997,6 @@ void elector_poa_free(elector_ctx *ctx) {
   for (cudaEvent_t ev : {ctx->ev_split0, ctx->ev_split1, ctx->ev_mt0, ctx->ev_mt1}) if (ev) cudaEventDestroy(ev);
   if (ctx->ev_rows) cudaEventDestroy(ctx->ev_rows);
   for (int k = 0; k < 2; ++k) if (ctx->ev_in[k]) cudaEventDestroy(ctx->ev_in[k]);
-  for (int k = 0; k < 8; ++k) if (ctx->ev_regb[k]) cudaEventDestroy(ctx->ev_regb[k]);
   if (ctx->ev_lin) cudaEventDestroy(ctx->ev_lin);
   if (ctx->ev_merged) cudaEventDestroy(ctx->ev_merged);
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
@@ -1041,7 +1016,7 @@ void elector_poa_free(elector_ctx *ctx) {
   }
   if (ctx->h_bintab) cudaFreeHost(ctx->h_bintab);
   if (ctx->h_plan) cudaFreeHost(ctx->h_plan);
-  for (cudaEvent_t e : ctx->chunk_ev) cudaEventDestroy(e);
+  if (ctx->ev_call) cudaEventDestroy(ctx->ev_call);
   if (ctx->copy_in) cudaStreamDestroy(ctx->copy_in);
   if (ctx->copy_out) cudaStreamDestroy(ctx->copy_out);
   if (ctx->h_totals) cudaFreeHost(ctx->h_totals);
@@ -1182,9 +1157,8 @@ int elector_pipeline_run2(elector_ctx *ctx, const elector_pipeline_io *iop) {
   // 10 000 reads of 10 kb.  ELECTOR_PIPELINE_CHUNKS forces a chunk count.
   // With packed letters the inputs are a quarter of the bytes and fewer, larger chunks win: two chunks of ~1 M windows measured
   // best for all output formats (counters only: 8.9 ms against 9.3 in three chunks and 11.9 in one).
-  int64_t chunk_windows = packed ? 1000000 : 700000;
+  const int64_t chunk_windows = packed ? 1000000 : 700000;
   int want_workers = 3;
-  if (const char *e = getenv("ELECTOR_PIPELINE_CHUNK_WINDOWS")) chunk_windows = std::max<int64_t>(1024, atoll(e));
   if (const char *e = getenv("ELECTOR_PIPELINE_WORKERS")) want_workers = std::max(1, std::min(8, atoi(e)));
   int64_t want_chunks = (n + chunk_windows - 1) / chunk_windows;
   if (const char *e = getenv("ELECTOR_PIPELINE_CHUNKS")) want_chunks = std::max(1, atoi(e));
@@ -1245,12 +1219,8 @@ int elector_pipeline_run2(elector_ctx *ctx, const elector_pipeline_io *iop) {
   std::atomic<long long> n_esc{0};
   cudaEvent_t h2d_prev = nullptr;
   for (size_t k = 0; k < jobs.size(); ++k) jobs[k].index = (int)k;
-  PipeArgs pa{iop, ro, co, uo, packed, ctx->ev_fork, &h2d_turn, &h2d_prev, &first_error, &n_esc};
-  if (trace) {
-    while (ctx->chunk_ev.empty()) { cudaEvent_t e; CU(cudaEventCreate(&e)); ctx->chunk_ev.push_back(e); }
-    pa.ev_call = ctx->chunk_ev[0];
-    CU(cudaEventRecord(pa.ev_call, ctx->stream));
-  }
+  PipeArgs pa{iop, ro, co, uo, packed, ctx->ev_call, &h2d_turn, &h2d_prev, &first_error, &n_esc};
+  if (trace) CU(cudaEventRecord(pa.ev_call, ctx->stream));
   std::atomic<size_t> next{0};
   const auto host_t0 = std::chrono::steady_clock::now();
   auto work = [&](elector_ctx *wk, int id) {

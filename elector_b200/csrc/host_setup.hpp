@@ -77,7 +77,6 @@ struct ScoringSetup {
       auto gcd = [](int a, int b) { a = std::abs(a); b = std::abs(b); while (b) { const int t = a % b; a = b; b = t; } return a; };
       const int q = gcd(gcd(mismatch, open), ext);
       packed_ok = uniform && match == 0 && mismatch < 0 && mismatch >= -16 && ext > 0 && open >= ext && open - ext <= q;
-      if (const char *e = getenv("ELECTOR_NO_PACKED")) if (e[0] == '1') packed_ok = false;
     }
     return true;
   }

@@ -36,8 +36,8 @@ if len(sys.argv) > 2 and sys.argv[2] == "child":
         ts = []
         for i in range(8):
             t0 = time.perf_counter(); ctx._check(lib.elector_pipeline_run2(ctx._ctx, ctypes.byref(io))); ts.append((time.perf_counter() - t0) * 1e3)
-        print("%-9s chunks=%s workers=%s prio=%s: %.2f ms (best of last 5: %.2f)" % (mode, os.environ.get("ELECTOR_PIPELINE_CHUNKS", "auto"), os.environ.get("ELECTOR_PIPELINE_WORKERS", "3"),
-              "off" if os.environ.get("ELECTOR_NO_PRIORITIES") == "1" else "on", sum(ts[3:]) / 5, min(ts[3:])), flush=True)
+        print("%-9s chunks=%s workers=%s: %.2f ms (best of last 5: %.2f)" % (mode, os.environ.get("ELECTOR_PIPELINE_CHUNKS", "auto"), os.environ.get("ELECTOR_PIPELINE_WORKERS", "3"),
+              sum(ts[3:]) / 5, min(ts[3:])), flush=True)
 else:
     reads = sys.argv[1] if len(sys.argv) > 1 else "10000"
     for env in ({}, {"ELECTOR_PIPELINE_CHUNKS": "1"}, {"ELECTOR_PIPELINE_CHUNKS": "2"}, {"ELECTOR_PIPELINE_CHUNKS": "4"}):
