@@ -81,12 +81,10 @@ struct elector_ctx {
   DevBuf d_tab, d_ref, d_cor, d_unc, d_roff, d_coff, d_uoff, d_items, d_scratch, d_scratch_lin, d_scratch2, d_ctrl, d_hist, d_bintab, d_key, d_key2, d_n1, d_p1;
   DevBuf d_rows, d_rowoff, d_stride, d_nring, d_s1, d_s2, d_cells;
   int64_t merged_cap = 0;  // bytes per merged-row buffer of the last merge
-  // pipelined host entry point: child contexts (one per extra worker thread), per-worker sums and status of the call
+  // worker contexts of the pipelined entry points (worker_slots): children on this device, one per extra worker thread
   std::vector<elector_ctx *> workers;
   std::vector<elector_ctx *> peers;   // worker contexts of elector_reads_pipeline_run on the other devices
-  int64_t pipe_sums[ELECTOR_TALLY_K] = {};
   int64_t *h_sums = nullptr;   // pinned: global counters of a chunk + the tally overflow flag
-  int pipe_rc = 0;
   DevBuf d_pk[3], d_exc_pos, d_exc_byte, d_rel, d_nib[3], d_esc_pos, d_esc_byte;   // compact wire format: packed letters, exceptions, 32-bit offsets in; 4-bit merged rows and their escapes out
   void *h_stage = nullptr; size_t h_stage_cap = 0;   // pinned staging of a chunk's 32-bit offsets
   DevBuf d_stretch; int64_t stretch_reads = 0;
@@ -139,6 +137,7 @@ int check_scan_overflow(elector_ctx *ctx, int64_t n_reads);
 const size_t kCtrlWords = 64;  // d_ctrl: [0..1] rows cursor (u64), [2] error flag, [3] tally overflow, [4..19] phase-1 and [20..35] phase-2 work counters, [36..37] rows cursor of the linear region, [38..39] where that region starts, [41] abort flag
 const int kAbortWord = 41;     // d_ctrl[41]: the alignment kernels of the call did not (all) run; merge and tally leave at once
 const int kSideStreams = 16;   // >= kMaxSegs: no two segments of a phase share a side stream
+const int kScratchRetries = 3; // runs of an alignment again after its scratch pools were grown (check_tables)
 
 #ifndef EL_MIN_WARPS_PH1P
 #define EL_MIN_WARPS_PH1P 28  // packed DP1: register cap 72 (64 spills since the diagonal band: 28 warps measured 0.2 ms per step faster than 32)
@@ -584,6 +583,29 @@ void add_kernel_ms(elector_ctx *ctx) {
   (void)cudaGetLastError();   // an event of a view that did not run this call has no time: not an error of the call
 }
 
+// One alignment on ctx's stream, waited for: run_device, the rows cursor read back, check_tables; a run whose scratch pools
+// were too small runs again with the grown pools.  d_rows_used (device memory, may be NULL) receives the rows cursor.
+int align_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_roff, const char *d_cor, const int64_t *d_coff,
+                 const char *d_unc, const int64_t *d_uoff, const int64_t *h_roff, const int64_t *h_coff, char *d_rows, int64_t rows_cap,
+                 int64_t *d_rowoff, int32_t *d_stride, int32_t *d_nring, int32_t *d_s1, int32_t *d_s2, int64_t *d_cells, int64_t *d_rows_used) {
+  for (int attempt = 0;; ++attempt) {
+    int rc = run_device(ctx, n, d_ref, d_roff, d_cor, d_coff, d_unc, d_uoff, h_roff, h_coff, d_rows, rows_cap, d_rowoff, d_stride, d_nring, d_s1, d_s2,
+                        d_cells, ctx->d_ctrl.as<unsigned long long>(), ctx->d_ctrl.as<int32_t>() + 2);
+    if (rc != ELECTOR_OK) return rc;
+    if (d_rows_used) CU(cudaMemcpyAsync(d_rows_used, ctx->d_ctrl.p, sizeof(int64_t), cudaMemcpyDeviceToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(&ctx->h_totals[4], ctx->d_ctrl.p, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));   // the one wait of the alignment
+    if (n == 0) return ELECTOR_OK;            // run_device queued nothing: no tables, no times
+    rc = check_tables(ctx);
+    if (rc == 1 && attempt < kScratchRetries) continue;
+    if (rc != ELECTOR_OK) return rc == 1 ? ctx->fail(ELECTOR_ECUDA, "scratch pools keep overflowing") : rc;
+    break;
+  }
+  add_kernel_ms(ctx);
+  if ((int32_t)(ctx->h_totals[5] & 0xffffffff)) return ctx->fail(ELECTOR_ECAPACITY, "row buffer capacity %lld too small", (long long)rows_cap);
+  return ELECTOR_OK;
+}
+
 
 struct ChunkJob { int64_t w0, w1, r0, r1, rows_base, rows_len, m_base; bool split; int index; };
 struct PipeArgs {
@@ -595,14 +617,13 @@ struct PipeArgs {
   // previous chunk's): chunk 0 computes while chunk 1 is still arriving
   std::atomic<int> *h2d_turn;
   cudaEvent_t *h2d_prev;
-  std::atomic<int> *failed;
   std::atomic<long long> *n_esc;    // escapes of the 4-bit merged rows appended so far (all chunks)
 };
 
 // One chunk of a pipelined call on one worker context: everything is queued on the worker's stream (the segment launches
-// fork to its side streams) and the function returns when the chunk's results are in the caller's host buffers.
-int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j) {
-  CU(cudaSetDevice(ctx->device));
+// fork to its side streams) and the function returns when the chunk's results are in the caller's host buffers.  Adds the
+// chunk's tally sums to sums; failed (run_pool) ends the wait for an input turn that an earlier chunk will not pass on.
+int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64_t *sums, const std::atomic<int> &failed) {
   const elector_pipeline_io &io = *pa.io;
   const int64_t w0 = j.w0, w1 = j.w1, nw = w1 - w0, r0 = j.r0, r1 = j.r1, nr = r1 - r0;
   const int64_t first[3] = {pa.ro[w0], pa.co[w0], pa.uo[w0]};
@@ -652,7 +673,7 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j) {
   }
   cudaStream_t st = ctx->stream;
   while (pa.h2d_turn->load(std::memory_order_acquire) != j.index) {
-    if (pa.failed->load() != ELECTOR_OK) return ctx->fail(ELECTOR_ECUDA, "another chunk of the call failed");
+    if (failed.load() != ELECTOR_OK) return ctx->fail(ELECTOR_ECUDA, "another chunk of the call failed");
     std::this_thread::yield();
   }
   struct PassTurn {   // whatever happens below, the next chunk gets its turn
@@ -793,7 +814,7 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j) {
     CU(cudaEventSynchronize(ctx->ev_rows));
     ctx->wait_in[0] = ctx->wait_in[1] = nullptr;   // the letters have arrived: a second attempt does not wait for them again
     rc = check_tables(ctx);
-    if (rc == 1 && attempt < 3) {   // a scratch pool was too small (first call, or longer windows than before): grown, run the chunk again
+    if (rc == 1 && attempt < kScratchRetries) {   // a scratch pool was too small (first call, or longer windows than before): grown, run the chunk again
       CU(cudaStreamSynchronize(st));
       CU(cudaStreamSynchronize(so));
       if (ctx->trace) fprintf(stderr, "[elector trace] chunk w%lld: scratch pools grown to %zu / %zu / %zu MiB, running it again\n", (long long)w0,
@@ -859,7 +880,7 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j) {
       cudaMemsetAsync(ctx->d_ctrl.as<int32_t>() + 3, 0, sizeof(int32_t), st);
       return ctx->fail(ELECTOR_EUNSUPPORTED, "a read has more than %d gap stretches at its borders", kMaxStretchKeys);
     }
-    for (int f = 0; f < ELECTOR_TALLY_K; ++f) ctx->pipe_sums[f] += ctx->h_sums[f];
+    for (int f = 0; f < ELECTOR_TALLY_K; ++f) sums[f] += ctx->h_sums[f];
   }
   return ELECTOR_OK;
 }
@@ -972,6 +993,89 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
   *out = ctx;
   return ELECTOR_OK;
 }
+
+// The worker contexts of a pipelined call: per_device contexts on every one of `devices` (a device may be listed more than
+// once), max_slots in all at most.  On ctx's device the first is ctx and the k-th after it ctx->workers[k - 1]; on other devices
+// they are ctx->peers.  Missing ones are created here and kept until elector_poa_free.
+int worker_slots(elector_ctx *ctx, const std::vector<int> &devices, int per_device, size_t max_slots, std::vector<elector_ctx *> &slots) {
+  slots.clear();
+  for (size_t i = 0; i < devices.size() && slots.size() < max_slots; ++i)
+    for (int w = 0; w < per_device && slots.size() < max_slots; ++w) {
+      int used = 0;   // contexts of this device already taken by earlier slots
+      for (elector_ctx *s : slots) used += s->device == devices[i];
+      elector_ctx *wk = nullptr;
+      if (devices[i] == ctx->device) {
+        while ((int)ctx->workers.size() < used) {
+          elector_ctx *child = nullptr;
+          const int rc = create_context(ctx->device, ctx->mat, &child, (int)ctx->workers.size() + 1);
+          if (rc != ELECTOR_OK) return ctx->fail(rc, "worker context: %s", g_init_error.c_str());
+          ctx->workers.push_back(child);
+        }
+        wk = used == 0 ? ctx : ctx->workers[(size_t)used - 1];
+      } else {
+        int seen = 0;
+        for (elector_ctx *p : ctx->peers)
+          if (p->device == devices[i] && seen++ == used) { wk = p; break; }
+        if (!wk) {
+          const int rc = create_context(devices[i], ctx->mat, &wk, used);
+          cudaSetDevice(ctx->device);
+          if (rc != ELECTOR_OK) return ctx->fail(rc, "worker context on device %d: %s", devices[i], g_init_error.c_str());
+          ctx->peers.push_back(wk);
+        }
+      }
+      slots.push_back(wk);
+    }
+  return ELECTOR_OK;
+}
+
+// Runs body(worker, slot, chunk, sums, failed) for the chunks 0 .. n_chunks - 1 of a pipelined call on the worker contexts
+// `slots`: slot 0 on the calling thread, every other slot on a thread of its own, each taking the next chunk until none is left
+// or a chunk has failed.  The body adds its chunk's tally sums to `sums` (the slot's own) and returns an error code; `failed`
+// lets a body that waits for another chunk see that the call has failed.  The first error wins: its code is returned and its
+// message is in ctx->err.  The device times and launch counts of the slots are summed into ctx; sums_out (may be NULL)
+// receives the tally sums of a call without error.  The calling thread is back on ctx's device afterwards.
+template <class Body>
+int run_pool(elector_ctx *ctx, const std::vector<elector_ctx *> &slots, size_t n_chunks, int64_t *sums_out, Body body) {
+  std::atomic<size_t> next{0};
+  std::atomic<int> failed{ELECTOR_OK};
+  int first = -1;   // slot of the first error: written by the one thread that sets `failed`, read after the join
+  std::vector<int64_t> sums(slots.size() * ELECTOR_TALLY_K, 0);
+  auto work = [&](int id) {
+    elector_ctx *wk = slots[(size_t)id];
+    wk->trace = ctx->trace;
+    wk->last_ms = wk->last_ms_phase1 = wk->last_ms_split = wk->last_ms_tally = 0.f;
+    wk->last_launches = 0;
+    int rc = cudaSetDevice(wk->device) == cudaSuccess ? ELECTOR_OK : wk->fail(ELECTOR_ECUDA, "cudaSetDevice(%d) failed", wk->device);
+    while (rc == ELECTOR_OK) {
+      const size_t k = next.fetch_add(1);
+      if (k >= n_chunks || failed.load() != ELECTOR_OK) break;
+      rc = body(wk, id, k, &sums[(size_t)id * ELECTOR_TALLY_K], failed);
+    }
+    int ok = ELECTOR_OK;
+    if (rc != ELECTOR_OK && failed.compare_exchange_strong(ok, rc)) first = id;
+  };
+  std::vector<std::thread> threads;
+  for (size_t i = 1; i < slots.size(); ++i) threads.emplace_back(work, (int)i);
+  work(0);
+  for (std::thread &t : threads) t.join();
+  cudaSetDevice(ctx->device);
+  float ms = 0.f, ms_phase1 = 0.f, ms_split = 0.f, ms_tally = 0.f;
+  int launches = 0;
+  for (const elector_ctx *wk : slots) {
+    ms += wk->last_ms; ms_phase1 += wk->last_ms_phase1; ms_split += wk->last_ms_split; ms_tally += wk->last_ms_tally; launches += wk->last_launches;
+  }
+  ctx->last_ms = ms; ctx->last_ms_phase1 = ms_phase1; ctx->last_ms_split = ms_split; ctx->last_ms_tally = ms_tally; ctx->last_launches = launches;
+  if (first >= 0) {
+    if (slots[(size_t)first] != ctx) ctx->err = slots[(size_t)first]->err;
+    return failed.load();
+  }
+  if (sums_out)
+    for (int f = 0; f < ELECTOR_TALLY_K; ++f) {
+      sums_out[f] = 0;
+      for (size_t i = 0; i < slots.size(); ++i) sums_out[f] += sums[i * ELECTOR_TALLY_K + (size_t)f];
+    }
+  return ELECTOR_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -1045,24 +1149,8 @@ int elector_poa_run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const
   ctx->trace = getenv("ELECTOR_TRACE") != nullptr;
   ctx->last_ms = ctx->last_ms_phase1 = 0.f;
   ctx->last_launches = 0;
-  for (int attempt = 0;; ++attempt) {
-    int rc = run_device(ctx, n, d_ref, d_roff, d_cor, d_coff, d_unc, d_uoff, h_roff, h_coff, d_rows, rows_cap,
-                        d_rowoff, d_stride, d_nring, d_s1, d_s2, d_cells, ctx->d_ctrl.as<unsigned long long>(),
-                        ctx->d_ctrl.as<int32_t>() + 2);
-    if (rc != ELECTOR_OK) return rc;
-    if (d_rows_used)
-      CU(cudaMemcpyAsync(d_rows_used, ctx->d_ctrl.p, sizeof(int64_t), cudaMemcpyDeviceToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(&ctx->h_totals[4], ctx->d_ctrl.p, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));   // the one wait of the call
-    if (n == 0) return ELECTOR_OK;
-    rc = check_tables(ctx);
-    if (rc == 1 && attempt < 3) continue;     // a scratch pool was too small and has been grown: run the call again
-    if (rc != ELECTOR_OK) return rc == 1 ? ctx->fail(ELECTOR_ECUDA, "scratch pools keep overflowing") : rc;
-    break;
-  }
-  add_kernel_ms(ctx);
-  if ((int32_t)(ctx->h_totals[5] & 0xffffffff)) return ctx->fail(ELECTOR_ECAPACITY, "rows_out capacity %lld too small", (long long)rows_cap);
-  return ELECTOR_OK;
+  return align_device(ctx, n, d_ref, d_roff, d_cor, d_coff, d_unc, d_uoff, h_roff, h_coff, d_rows, rows_cap, d_rowoff, d_stride, d_nring, d_s1, d_s2,
+                      d_cells, d_rows_used);
 }
 
 int elector_poa_run(elector_ctx *ctx, int64_t n, const char *ref, const int64_t *ro, const char *cor, const int64_t *co,
@@ -1207,56 +1295,28 @@ int elector_pipeline_run2(elector_ctx *ctx, const elector_pipeline_io *iop) {
     if (base > io.rows_cap) return ctx->fail(ELECTOR_ECAPACITY, "rows_out capacity %lld too small (%lld needed)", (long long)io.rows_cap, (long long)base);
   }
   // ---- workers ----
-  const int nworkers = (int)std::min<size_t>(jobs.size(), (size_t)want_workers);
-  while ((int)ctx->workers.size() < nworkers - 1) {
-    elector_ctx *child = nullptr;
-    const int rc = create_context(ctx->device, ctx->mat, &child, (int)ctx->workers.size() + 1);
-    if (rc != ELECTOR_OK) return ctx->fail(rc, "worker context: %s", g_init_error.c_str());
-    ctx->workers.push_back(child);
-  }
+  std::vector<elector_ctx *> slots;
+  int rc = worker_slots(ctx, {ctx->device}, want_workers, jobs.size(), slots);
+  if (rc != ELECTOR_OK) return rc;
   std::atomic<int> h2d_turn{0};
-  std::atomic<int> first_error{ELECTOR_OK};
   std::atomic<long long> n_esc{0};
   cudaEvent_t h2d_prev = nullptr;
   for (size_t k = 0; k < jobs.size(); ++k) jobs[k].index = (int)k;
-  PipeArgs pa{iop, ro, co, uo, packed, ctx->ev_call, &h2d_turn, &h2d_prev, &first_error, &n_esc};
+  PipeArgs pa{iop, ro, co, uo, packed, ctx->ev_call, &h2d_turn, &h2d_prev, &n_esc};
   if (trace) CU(cudaEventRecord(pa.ev_call, ctx->stream));
-  std::atomic<size_t> next{0};
   const auto host_t0 = std::chrono::steady_clock::now();
-  auto work = [&](elector_ctx *wk, int id) {
-    wk->trace = trace;
-    wk->last_ms = wk->last_ms_phase1 = 0.f;
-    wk->last_launches = 0;
-    memset(wk->pipe_sums, 0, sizeof wk->pipe_sums);
-    for (;;) {
-      const size_t k = next.fetch_add(1);
-      if (k >= jobs.size() || first_error.load() != ELECTOR_OK) break;
-      const double t_in = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count();
-      const int rc = process_chunk(wk, pa, jobs[k]);
-      if (trace)
-        fprintf(stderr, "[elector trace] chunk %zu (worker %d): %lld windows, host clock %.2f -> %.2f ms\n", k, id, (long long)(jobs[k].w1 - jobs[k].w0), t_in,
-                std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count());
-      if (rc != ELECTOR_OK) { int ok = ELECTOR_OK; first_error.compare_exchange_strong(ok, rc); wk->pipe_rc = rc; break; }
-    }
-  };
-  for (elector_ctx *w : ctx->workers) w->pipe_rc = ELECTOR_OK;
-  ctx->pipe_rc = ELECTOR_OK;
-  std::vector<std::thread> threads;
-  for (int i = 1; i < nworkers; ++i) threads.emplace_back(work, ctx->workers[i - 1], i);
-  work(ctx, 0);
-  for (std::thread &t : threads) t.join();
-  for (int i = 1; i < nworkers; ++i) {
-    elector_ctx *w = ctx->workers[i - 1];
-    ctx->last_ms += w->last_ms; ctx->last_ms_phase1 += w->last_ms_phase1; ctx->last_launches += w->last_launches;
-    for (int f = 0; f < ELECTOR_TALLY_K; ++f) ctx->pipe_sums[f] += w->pipe_sums[f];
-    if (w->pipe_rc != ELECTOR_OK && ctx->pipe_rc == ELECTOR_OK) { ctx->pipe_rc = w->pipe_rc; ctx->err = w->err; }
-  }
-  if (ctx->pipe_rc != ELECTOR_OK) return ctx->pipe_rc;
-  if (first_error.load() != ELECTOR_OK) return first_error.load();
-  if (io.sums_out) memcpy(io.sums_out, ctx->pipe_sums, sizeof ctx->pipe_sums);
+  rc = run_pool(ctx, slots, jobs.size(), io.sums_out, [&](elector_ctx *wk, int id, size_t k, int64_t *sums, const std::atomic<int> &failed) {
+    const double t_in = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count();
+    const int rc = process_chunk(wk, pa, jobs[k], sums, failed);
+    if (trace)
+      fprintf(stderr, "[elector trace] chunk %zu (worker %d): %lld windows, host clock %.2f -> %.2f ms\n", k, id, (long long)(jobs[k].w1 - jobs[k].w0), t_in,
+              std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count());
+    return rc;
+  });
+  if (rc != ELECTOR_OK) return rc;
   if (io.m_n_esc) *io.m_n_esc = n_esc.load();
-  if (trace) fprintf(stderr, "[elector trace] call returned at %.2f ms (host clock), %zu chunks on %d workers\n",
-                     std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count(), jobs.size(), nworkers);
+  if (trace) fprintf(stderr, "[elector trace] call returned at %.2f ms (host clock), %zu chunks on %zu workers\n",
+                     std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count(), jobs.size(), slots.size());
   return ELECTOR_OK;
 }
 

@@ -214,6 +214,42 @@ def test_device_that_does_not_exist(ctx, tmp_path_factory):
     assert_same(ctx.reads_pipeline(*r, 0.1, merged=True), want)
 
 
+def test_failed_chunk_in_the_worker_pool(ctx, tmp_path_factory, monkeypatch):
+    """a chunk that fails inside the worker pool of either pipelined call, while other workers run theirs, gives the call its own
+    error; a clean call on the same context afterwards gives what it gave before the failure"""
+    import elector_b200
+    import workloads
+    # elector_pipeline_run2: four chunks on three workers; the first window of the last read (last chunk) has no corrected letters
+    monkeypatch.setenv("ELECTOR_PIPELINE_CHUNKS", "4")
+    monkeypatch.setenv("ELECTOR_PIPELINE_WORKERS", "3")
+    wl = workloads.make_windows(2, 900)
+    clean = (wl["ref"], wl["ref_off"], wl["cor"], wl["cor_off"], wl["unc"], wl["unc_off"], wl["read_first"])
+    w = int(wl["read_first"][-2])
+    co = np.array(wl["cor_off"], dtype=np.int64)
+    cor = np.concatenate([wl["cor"][:co[w]], wl["cor"][co[w + 1]:]])
+    co[w + 1:] -= co[w + 1] - co[w]
+    want = ctx.pipeline_io(*clean)
+    with pytest.raises(elector_b200.ElectorError) as e:
+        ctx.pipeline_io(wl["ref"], wl["ref_off"], cor, co, wl["unc"], wl["unc_off"], wl["read_first"])
+    assert e.value.code == -1 and "empty sequence" in str(e.value)
+    got = ctx.pipeline_io(*clean)
+    for k in ("nring", "score1", "score2", "cells"):
+        assert np.array_equal(getattr(got["res"], k), getattr(want["res"], k)), k
+    assert np.array_equal(got["counters"], want["counters"]) and np.array_equal(got["sums"], want["sums"])
+    assert got["merged"] == want["merged"]
+    # elector_reads_pipeline_run: five chunks on two listed devices; the last triplet (last chunk) has an empty reference read
+    monkeypatch.setenv("ELECTOR_PIPELINE_CHUNKS", "5")
+    monkeypatch.delenv("ELECTOR_PIPELINE_WORKERS")
+    r = reads(tmp_path_factory, 1, 300)
+    ro = r[1].copy()
+    ro[-1] = ro[-2]
+    want = ctx.reads_pipeline(*r, 0.1, merged=True, devices=[0, 0])
+    with pytest.raises(elector_b200.ElectorError) as e:
+        ctx.reads_pipeline(r[0], ro, *r[2:], 0.1, merged=True, devices=[0, 0])
+    assert e.value.code == -1 and "empty reference read" in str(e.value)
+    assert_same(ctx.reads_pipeline(*r, 0.1, merged=True, devices=[0, 0]), want)
+
+
 def test_no_triplets(ctx):
     z8, z64 = np.zeros(0, np.uint8), np.zeros(1, np.int64)
     got = ctx.reads_pipeline(z8, z64, z8, z64, z8, z64, np.zeros(0, np.int32), 0.1, merged=True, devices=[0, 0])
