@@ -292,7 +292,7 @@ struct SortView {
 
 // kernel of a segment (static: known before the sort runs, see SegStatic)
 int seg_kind(const elector_ctx *ctx, int phase, int s) {
-  const bool small16 = ctx->sc.packed_ok && (int64_t)ctx->sc.maxabs * (kSmallMax + 4 * kN1q + 4) <= kPackedSpan;   // no score of a small window leaves 16 bits
+  const bool small16 = ctx->sc.small_packed();
   // windows of more than 128 rows run a warp per window: the big tiers and the first small segment (129 .. 256 rows) of phase 1,
   // of the general and of the linear segments of phase 2
   if (phase == 1) return (s <= kBigTiers && ctx->coop_group > 0) ? kCoop : (s >= kBigTiers && small16) ? kPacked : kInt32;
@@ -449,8 +449,7 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   // windows whose corrected letters are the reference letters need no phase 1 (bin_kernel.cuh): the sort then reads the
   // letters, so it waits for them too.  Only when their phase 2 needs no node list: Phase2L for the small linear segments,
   // the warp-cooperative kernel (which rebuilds lin(ref)) for the long ones.
-  const bool ident_ok = ctx->sc.packed_ok && ctx->coop_group > 0 &&
-                        (int64_t)ctx->sc.maxabs * (kSmallMax + 4 * kN1q + 4) <= kPackedSpan;
+  const bool ident_ok = ctx->sc.small_packed() && ctx->coop_group > 0;
   if (ident_ok && ctx->wait_in[0]) CU(cudaStreamWaitEvent(st, ctx->wait_in[0], 0));
   IdentArgs ida{(const uint8_t *)d_ref, (const uint8_t *)d_cor, ctx->d_n1.as<int32_t>(), ctx->d_key2.as<int32_t>(), hist2, dtab2->seg_max, d_s1, &dtab2->lin_bytes};
   bin1_count_kernel<<<bgrid, 256, 0, st>>>((int32_t)n, d_roff, d_coff, d_uoff, ctx->d_key.as<int32_t>(), hist1, dtab1, ident_ok, ida);
@@ -1274,13 +1273,15 @@ int elector_pipeline_run2(elector_ctx *ctx, const elector_pipeline_io *iop) {
   // caller's buffer allows it (or takes no rows at all), else the exact one (one pass over the offsets).
   const bool loose = !io.rows_out || io.rows_cap >= elector_poa_rows_bound(n, ro, co, uo);
   if (loose) {
-    // region k = [lo16(bound of the windows before it), lo16(bound of the windows up to its end)): the regions tile the O(1)
+    // region k = [lo4(bound of the windows before it), lo4(bound of the windows up to its end)): the regions tile the O(1)
     // bound of the call whatever the chunking.  A window's share of the bound is 3 * (letters + 3) bytes and it needs at most
     // 3 * ((columns + 3) & ~3) with columns <= letters - 1 (every DP aligns something or, at worst, ('AAAAA','C','G')-like
-    // inputs give letters - 1 columns): at least 3 spare bytes per window.  Two regions per chunk lose up to 30 bytes to the
-    // two 16-byte roundings, so a chunk is only split when it has 64 windows or more (192 spare bytes); the kernels check
+    // inputs give letters - 1 columns): at least 3 spare bytes per window, so the rounding of a region to the 4-byte row
+    // words (at most 3 bytes) fits even a chunk of one window.  (Rounding to 16 bytes did not: a call of one window with as
+    // many columns as letters - 1 overflowed its region.)  Two regions per chunk lose up to 30 bytes more to the 16-byte
+    // boundary between them, so a chunk is only split when it has 64 windows or more (192 spare bytes); the kernels check
     // rows_cap anyway, so the failure mode of a wrong margin is ELECTOR_ECAPACITY, never a stray write.
-    auto before = [&](int64_t w) { return (3 * (ro[w] + co[w] + uo[w] + 3 * w)) & ~(int64_t)15; };
+    auto before = [&](int64_t w) { return (3 * (ro[w] + co[w] + uo[w] + 3 * w)) & ~(int64_t)3; };
     for (ChunkJob &j : jobs) { j.rows_base = before(j.w0); j.rows_len = before(j.w1) - j.rows_base; j.split = j.w1 - j.w0 >= 64; }
   } else {
     int64_t base = 0;

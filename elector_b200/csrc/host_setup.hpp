@@ -10,6 +10,7 @@
 
 #include "host_io.hpp"
 #include "poa_kernel.cuh"
+#include "poa_packed.cuh"
 
 namespace elector {
 
@@ -80,6 +81,11 @@ struct ScoringSetup {
     }
     return true;
   }
+
+  // The small segments (every sequence <= kSmallMax, len(P1) < 4 kN1q) run the packed kernels: no score of a small window
+  // leaves 16 bits.  The launcher's kernel choice (seg_kind), the cor-is-ref shortcut of the size sort and the CPU emulation
+  // all ask this one question.
+  bool small_packed() const { return packed_ok && (int64_t)maxabs * (kSmallMax + 4 * kN1q + 4) <= kPackedSpan; }
 };
 
 }  // namespace elector

@@ -6,6 +6,7 @@
 //
 // usage: poa_emul MATRIX|- REF.fa COR.fa UNC.fa OUT.pir [OUT.scores|-] [packed|dual-general|coop]
 // packed: windows the library would run through the 16-bit packed kernels (poa_packed.cuh) do so here too
+// stderr, first line: the matrix class ScoringSetup::analyse found
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -65,12 +66,12 @@ static int run(const ScoringSetup &sc, FastaFile &R, FastaFile &C, FastaFile &U,
       int bj = -1;
       coop_dp_emulated<GS>(p1, bset.data(), lr, lc, s1, bj);
       n1 = coop1_after<GS>(p1, L1, lr, lc, bj, nodes_p, spcode);
-    } else if (packed && !general_only && sc.packed_ok && lr == lc && lr <= kSmallMax && lu <= kSmallMax && memcmp(ref, cor, (size_t)lr) == 0) {
+    } else if (packed && !general_only && sc.small_packed() && lr == lc && lr <= kSmallMax && lu <= kSmallMax && memcmp(ref, cor, (size_t)lr) == 0) {
       // cor is ref: the size sort of the library (bin1_count_kernel) skips phase 1 -- P1 = lin(ref), every node carries both letters
       n1 = lr; s1 = 0; spcode = 0;
       ident = true;
       ++n_ident1;
-    } else if (packed && sc.packed_ok && (long)sc.maxabs * (cap_r + cap_c + 4) <= kPackedSpan) {
+    } else if (packed && sc.small_packed() && std::max(lr, lc) <= kSmallMax) {   // a small segment of the library (bin1_of)
       Layout1P L1;
       make_layout1p(L1, cap_r, cap_c);
       std::vector<uint32_t> scratch1((size_t)L1.total * 32, 0xdeadbeefu);
@@ -113,7 +114,7 @@ static int run(const ScoringSetup &sc, FastaFile &R, FastaFile &C, FastaFile &U,
     const uint32_t row_words = (uint32_t)(n1 + lu) / 4 + 2;
     std::vector<uint32_t> rows((size_t)3 * row_words, 0xdeadbeefu);
     RowSink sink{rows.data(), rows.data() + row_words, rows.data() + 2 * row_words};
-    const bool fits16 = packed && sc.packed_ok && (long)sc.maxabs * (cap_n + cap_u + 4) <= kPackedSpan;
+    const bool fits16 = packed && sc.small_packed() && seg >= kBigTiers;   // a small segment of the library (bin2_of)
     if (coop) {   // the warp-cooperative DP2 of poa_coop.cuh (32 lanes emulated one after the other), serial steps of Phase2
       Layout2 L2;
       make_layout2(L2, cap_n, cap_u);
@@ -207,6 +208,8 @@ int main(int argc, char **argv) {
   else if (m.load(argv[1]) <= 0) { fprintf(stderr, "cannot read matrix\n"); return 1; }
   ScoringSetup sc;
   if (!sc.analyse(m)) { fprintf(stderr, "unsupported matrix: %s\n", sc.error.c_str()); return 3; }
+  // the class the library's kernel choice starts from (capi.cu seg_kind)
+  fprintf(stderr, "matrix class: packed_ok %d generic_sub %d maxabs %d small_packed %d\n", (int)sc.packed_ok, (int)sc.generic_sub, sc.maxabs, (int)sc.small_packed());
   FastaFile R, C, U;
   if (read_fasta_file(argv[3], C) < 0 || read_fasta_file(argv[4], U) < 0 || read_fasta_file(argv[2], R) < 0) return 1;
   FILE *pir = fopen(argv[5], "w");

@@ -6,7 +6,8 @@ import subprocess
 
 import pytest
 
-from conftest import GOLDEN_SETS, parse_dump
+from conftest import GOLDEN_SETS, parse_dump, read_fasta_simple
+from oracle import synth
 
 
 @pytest.mark.parametrize("mode", ["int32", "packed", "dual-general", "coop"])
@@ -45,20 +46,73 @@ def test_emulated_band_dp_is_exact(golden_dir, emul_bin, name, band_w, tmp_path,
     assert [(g["s1"], g["s2"], g["n1"]) for g in gold] == [e[:3] for e in got]
 
 
+MATRIX_IDS = [m[0] for m in synth.MATRICES]
+
+
+@pytest.fixture(scope="module")
+def sweep(golden_dir, tmp_path_factory):
+    """inputs of the matrix sweep: the golden set `hard`, bubble windows for the dual-frontier kernel and the small windows of
+    the edge set (every sequence <= kSmallMax: the packed kernels' size classes), as FASTA files; the oracle's PIR per
+    matrix, computed once"""
+    d = str(tmp_path_factory.mktemp("sweep"))
+    S = synth.kernel_constants()["kSmallMax"]
+    hard = list(zip(*[[s for _, s in read_fasta_simple("%s/hard.%s.fa" % (golden_dir, key))] for key in ("ref", "cor", "unc")]))
+    wins = [("h%d" % i,) + w for i, w in enumerate(hard)] + synth.bubble_windows(2000)
+    wins += [w for w in synth.edge_windows() if max(map(len, w[1:])) <= S]
+    synth.write_windows([("w%d" % i,) + w[1:] for i, w in enumerate(wins)], d + "/in")
+    return {"dir": d, "oracle": {}}
+
+
+def sweep_matrix(sweep, mid):
+    from oracle import oracle
+    mp = "%s/%s.mat" % (sweep["dir"], mid)
+    if mid not in sweep["oracle"]:
+        open(mp, "w").write(synth.matrix_text(mid))
+        opir = "%s/%s.oracle.pir" % (sweep["dir"], mid)
+        assert oracle.poa_files(mp, *["%s/in.%s.fa" % (sweep["dir"], k) for k in ("ref", "cor", "unc")], opir) == 0
+        sweep["oracle"][mid] = open(opir, "rb").read()
+    return mp, sweep["oracle"][mid]
+
+
 def test_emulated_kernel_generic_matrix(golden_dir, emul_bin, tmp_path):
     """non-uniform substitution scores + other gap penalties: table path vs the oracle"""
-    from elector_b200.matrix import ALPHABET
     from oracle import oracle
     d = golden_dir
     mp = str(tmp_path / "m.mat")
-    lines = ["GAP-TRUNCATION-LENGTH=4", "GAP-DECAY-LENGTH=0", "GAP-PENALTIES=7 3 3", "  " + " ".join(ALPHABET)]
-    for i, a in enumerate(ALPHABET):
-        lines.append(a + " " + " ".join(str(4 if i == j else -((i * 7 + j * 3) % 5) - 1) for j in range(len(ALPHABET))))
-    open(mp, "w").write("\n".join(lines) + "\n")
+    open(mp, "w").write(synth.matrix_text("table"))
     pir, opir = str(tmp_path / "e.pir"), str(tmp_path / "o.pir")
     assert subprocess.call([emul_bin, mp, d + "/hard.ref.fa", d + "/hard.cor.fa", d + "/hard.unc.fa", pir]) == 0
     assert oracle.poa_files(mp, d + "/hard.ref.fa", d + "/hard.cor.fa", d + "/hard.unc.fa", opir) == 0
     assert open(pir, "rb").read() == open(opir, "rb").read()
+
+
+@pytest.mark.parametrize("mode", ["int32", "packed", "dual-general", "coop"])
+@pytest.mark.parametrize("mid", MATRIX_IDS)
+def test_emulated_kernel_matrix_sweep(sweep, emul_bin, mid, mode, tmp_path):
+    """every matrix of oracle/synth.MATRICES (the packed class at its edges, INT32 compare-select, the substitution table)
+    through every kernel family, on hard, bubble and small edge windows, vs the oracle"""
+    mp, want = sweep_matrix(sweep, mid)
+    pir = str(tmp_path / "e.pir")
+    ins = ["%s/in.%s.fa" % (sweep["dir"], k) for k in ("ref", "cor", "unc")]
+    assert subprocess.call([emul_bin, mp] + ins + [pir] + (["-", mode] if mode != "int32" else []), stderr=subprocess.DEVNULL) == 0
+    assert open(pir, "rb").read() == want
+
+
+@pytest.mark.parametrize("mid", MATRIX_IDS)
+def test_matrix_lands_in_its_class(golden_dir, emul_bin, mid, tmp_path):
+    """ScoringSetup::analyse puts each matrix of the sweep into the class oracle/synth.MATRICES names for it (packed_ok,
+    generic_sub, maxabs, small windows packed): no matrix can drift into another kernel family unnoticed"""
+    mp = str(tmp_path / "m.mat")
+    open(mp, "w").write(synth.matrix_text(mid))
+    d = golden_dir
+    p = subprocess.run([emul_bin, mp, d + "/edge.ref.fa", d + "/edge.cor.fa", d + "/edge.unc.fa", str(tmp_path / "e.pir")],
+                       capture_output=True, text=True)
+    assert p.returncode == 0
+    line = [l for l in p.stderr.splitlines() if l.startswith("matrix class:")]
+    assert len(line) == 1
+    t = line[0].split()
+    got = tuple(int(t[t.index(key) + 1]) for key in ("packed_ok", "generic_sub", "maxabs", "small_packed"))
+    assert got == next(m[4] for m in synth.MATRICES if m[0] == mid)
 
 
 def test_emulated_kernel_rejects_unsupported_matrix(golden_dir, emul_bin, tmp_path):
@@ -104,28 +158,8 @@ def test_emulated_dual_kernel_on_bubble_windows(golden_dir, emul_bin, mode, tmp_
     that open and close at every position of a band, in the low and in the high half, back to back, at the first and at the last
     node; late starts and early ends of either sequence) against a noisier uncorrected one, lengths around the band sizes"""
     from oracle import oracle, synth
-    rng = synth.SplitMix64(20261018)
-    wins = []
-    for i in range(6000):
-        L = [7, 8, 9, 15, 16, 17, 23, 24, 25, 31, 32, 33, 40, 48, 50, 55, 64, 65, 80, 100, 127][rng.below(21)]
-        ref = "".join("ACGT"[rng.below(4)] for _ in range(L))
-        cor = synth.mutate(rng, ref, [0.01, 0.02, 0.05, 0.1, 0.2][rng.below(5)], "ACGT")
-        t = rng.below(8)
-        if t == 0:
-            cor = cor[1 + rng.below(3):]                      # cor starts late: INITIAL node with the virtual link first
-        elif t == 1:
-            cor = cor[:max(1, len(cor) - 1 - rng.below(3))]   # cor ends early: several FINAL nodes
-        elif t == 2:
-            cor = "ACGT"[rng.below(4)] * (1 + rng.below(3)) + cor   # cor starts with an insertion
-        unc = synth.mutate(rng, ref, [0.05, 0.1, 0.2][rng.below(3)], "ACGT")
-        wins.append((ref, cor or "A", unc or "C"))
-    paths = []
-    for k, key in enumerate(("ref", "cor", "unc")):
-        p = str(tmp_path / (key + ".fa"))
-        with open(p, "w") as f:
-            for i, w in enumerate(wins):
-                f.write(">w%d\n%s\n" % (i, w[k]))
-        paths.append(p)
+    synth.write_windows(synth.bubble_windows(6000, seed=20261018), str(tmp_path / "in"))
+    paths = [str(tmp_path / ("in.%s.fa" % key)) for key in ("ref", "cor", "unc")]
     pir, opir = str(tmp_path / "e.pir"), str(tmp_path / "o.pir")
     mp = golden_dir + "/blosum80.mat"
     assert subprocess.call([emul_bin, mp, paths[0], paths[1], paths[2], pir, "-", mode], stderr=subprocess.DEVNULL) == 0

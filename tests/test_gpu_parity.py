@@ -152,19 +152,46 @@ def test_band_dp_is_exact_whatever_the_width(band_w, monkeypatch):
 def test_generic_matrix_vs_oracle(golden_dir, tmp_path):
     """non-uniform substitution scores and other gap penalties (table path of the kernel)"""
     import elector_b200
-    from elector_b200.matrix import ALPHABET
-    from oracle import oracle
+    from oracle import oracle, synth
     d = golden_dir
     mp = str(tmp_path / "m.mat")
-    lines = ["GAP-TRUNCATION-LENGTH=4", "GAP-DECAY-LENGTH=0", "GAP-PENALTIES=7 3 3", "  " + " ".join(ALPHABET)]
-    for i, a in enumerate(ALPHABET):
-        lines.append(a + " " + " ".join(str(4 if i == j else -((i * 7 + j * 3) % 5) - 1) for j in range(len(ALPHABET))))
-    open(mp, "w").write("\n".join(lines) + "\n")
+    open(mp, "w").write(synth.matrix_text("table"))
     out, oout = str(tmp_path / "g.pir"), str(tmp_path / "o.pir")
     with elector_b200.PoaContext(0, mp) as c2:
         c2.files(d + "/hard.ref.fa", d + "/hard.cor.fa", d + "/hard.unc.fa", out)
     assert oracle.poa_files(mp, d + "/hard.ref.fa", d + "/hard.cor.fa", d + "/hard.unc.fa", oout) == 0
     assert open(out, "rb").read() == open(oout, "rb").read()
+
+
+def matrix_sweep_params():
+    from oracle import synth
+    # the matrices whose small windows run packed, at the default band and at the narrowest
+    return [pytest.param(m[0], b, id=m[0] + ("-band" + b if b else "")) for m in synth.MATRICES for b in ([None, "1"] if m[4][3] else [None])]
+
+
+@pytest.mark.parametrize("mid,band_w", matrix_sweep_params())
+def test_matrix_sweep_vs_oracle(tmp_path, mid, band_w, monkeypatch):
+    """every matrix of oracle/synth.MATRICES: the packed class at its edges, INT32 compare-select (a positive match, one step
+    outside the packed class, packed_ok beyond the small-window limit), the substitution table; on hard, bubble and the
+    small edge windows, every output vs the oracle"""
+    import elector_b200
+    from elector_b200 import windows_to_csr
+    from oracle import oracle, synth
+    mp = str(tmp_path / "m.mat")
+    open(mp, "w").write(synth.matrix_text(mid))
+    if band_w is not None:
+        monkeypatch.setenv("ELECTOR_BAND_W", band_w)
+    S = synth.kernel_constants()["kSmallMax"]
+    ma = next(m for m in synth.MATRICES if m[0] == mid)[4][2]
+    wins = synth.hard_windows(3000) + synth.bubble_windows() + [w for w in synth.edge_windows(maxabs=ma) if max(map(len, w[1:])) <= S]
+    r, ro = windows_to_csr([w[1] for w in wins]); c, co = windows_to_csr([w[2] for w in wins]); u, uo = windows_to_csr([w[3] for w in wins])
+    with elector_b200.PoaContext(0, mp) as c2:
+        res = c2.run_csr(r, ro, c, co, u, uo)
+    o = oracle.batch(r, ro, c, co, u, uo, m=oracle.matrix(mp), nthreads=os.cpu_count() or 1)
+    assert np.array_equal(res.nring, o["nring"]) and np.array_equal(res.cells, o["cells"])
+    assert np.array_equal(res.score1, o["score1"]) and np.array_equal(res.score2, o["score2"])
+    for w in range(len(wins)):
+        assert res.window_rows(w) == oracle.window_rows(o, w), wins[w][0]
 
 
 def test_errors(ctx, golden_dir, tmp_path):
