@@ -14,6 +14,10 @@
 #include <stdint.h>
 
 #include "poa_kernel.cuh"
+#ifdef __CUDACC__
+#include <cub/block/block_radix_sort.cuh>
+#include <cub/block/block_scan.cuh>
+#endif
 
 namespace elector {
 
@@ -132,6 +136,36 @@ __global__ void set_u64_kernel(unsigned long long *p, unsigned long long v) { *p
 // negative: the packed class): P1 is lin(ref) with every node carrying both letters, best score 0.  With `id` non-null
 // the sort recognises them, leaves them out of the phase-1 work list (key -2) and does what phase 1 would have left for
 // phase 2: len(P1), the phase-2 sort bin and histogram, the segment maxima and the row bytes of the linear region.
+#ifdef __CUDACC__
+// The letters from p on as consecutive 16-byte words, whatever p's alignment: aligned 16-byte loads, realigned by a
+// word select and a funnel shift (the shift is fixed for the whole string).  A load never touches a 16-byte block that
+// holds no letter of [p, end); bytes past end are left to the caller to ignore.
+struct Letters16 {
+  const uint4 *q;
+  uint4 cur;
+  uint32_t sel, sh;
+  const uint8_t *end;
+  __device__ __forceinline__ void init(const uint8_t *p, const uint8_t *e) {
+    q = reinterpret_cast<const uint4 *>(reinterpret_cast<uintptr_t>(p) & ~(uintptr_t)15);
+    sel = (uint32_t)(reinterpret_cast<uintptr_t>(p) >> 2) & 3u;
+    sh = 8u * ((uint32_t)reinterpret_cast<uintptr_t>(p) & 3u);
+    end = e;
+    cur = __ldg(q);
+  }
+  __device__ __forceinline__ uint4 next() {
+    ++q;
+    const uint4 nx = reinterpret_cast<const uint8_t *>(q) < end ? __ldg(q) : make_uint4(0, 0, 0, 0);
+    // words sel .. sel + 4 of cur : nx
+    const bool s2 = sel & 2u, s1 = sel & 1u;
+    const uint32_t t0 = s2 ? cur.z : cur.x, t1 = s2 ? cur.w : cur.y, t2 = s2 ? nx.x : cur.z, t3 = s2 ? nx.y : cur.w, t4 = s2 ? nx.z : nx.x,
+                   t5 = s2 ? nx.w : nx.y;
+    const uint32_t u0 = s1 ? t1 : t0, u1 = s1 ? t2 : t1, u2 = s1 ? t3 : t2, u3 = s1 ? t4 : t3, u4 = s1 ? t5 : t4;
+    cur = nx;
+    return make_uint4(__funnelshift_r(u0, u1, sh), __funnelshift_r(u1, u2, sh), __funnelshift_r(u2, u3, sh), __funnelshift_r(u3, u4, sh));
+  }
+};
+#endif
+
 struct IdentArgs {
   const uint8_t *ref, *cor;
   int32_t *n1, *key2, *hist2, *seg2_max, *score1;
@@ -150,13 +184,20 @@ __global__ void __launch_bounds__(256) bin1_count_kernel(int32_t n, const int64_
       if (use_ident && lr == lc && lr <= kSmallMax && lu <= kSmallMax) {
         const uint8_t *a = id.ref + ro[w], *b = id.cor + co[w];
         const int len = (int)lr;
+        Letters16 sa, sb;
+        sa.init(a, a + len);
+        sb.init(b, b + len);
         uint32_t d = 0;
-        int i = 0;
-        for (; i + 8 <= len && !d; i += 8) {   // eight independent byte pairs per step (the letters are not aligned)
+        for (int i = 0; i < len && !d; i += 16) {   // 16 letters of each per step, from aligned 16-byte loads
+          const uint4 x = sa.next(), y = sb.next();
+          const uint32_t e[4] = {x.x ^ y.x, x.y ^ y.y, x.z ^ y.z, x.w ^ y.w};
+          const int m = len - i;   // letters left; bytes of a word past them are not compared
 #pragma unroll
-          for (int k = 0; k < 8; ++k) d |= (uint32_t)(a[i + k] ^ b[i + k]);
+          for (int k = 0; k < 4; ++k) {
+            const int v = m - 4 * k;
+            d |= v >= 4 ? e[k] : v > 0 ? e[k] & ((1u << (8 * v)) - 1u) : 0u;
+          }
         }
-        for (; i < len && !d; ++i) d |= (uint32_t)(a[i] ^ b[i]);
         ident = d == 0;
       }
       if (ident) {
@@ -237,20 +278,53 @@ __global__ void __launch_bounds__(1024) bin_scan_totals_kernel(int32_t nchunks, 
   }
 }
 
-// keys in bin0 .. bin1-1 only; cursor = the table's scanned histogram, chunk_base relative to bin0
-__global__ void __launch_bounds__(256) bin_scatter_kernel(int32_t n, const int32_t *key, int32_t *cursor, const int32_t *chunk_base,
-                                                           int32_t *items, int32_t bin0, int32_t bin1) {
-  for (int32_t w = blockIdx.x * blockDim.x + threadIdx.x; w < n; w += gridDim.x * blockDim.x) {
-    const int bin = key[w];
-    if (bin < bin0 || bin >= bin1) continue;  // invalid window (reported by bin1_count_kernel), a window that needs no phase 1, or another sort's
-    // neighbouring windows often share a bin: one atomic per distinct bin of the warp's active lanes
-    const unsigned peers = __match_any_sync(__activemask(), bin);
-    const int leader = __ffs(peers) - 1, lane = threadIdx.x & 31;
-    int base = 0;
-    if (lane == leader) base = atomicAdd(&cursor[bin], __popc(peers));
-    base = __shfl_sync(peers, base, leader);
-    items[chunk_base[(bin - bin0) / kScanChunk] + base + __popc(peers & ((1u << lane) - 1u))] = w;
+// keys in bin0 .. bin1-1 only; cursor = the table's scanned histogram, chunk_base relative to bin0.
+// Each CTA takes a contiguous tile of windows and sorts it by bin in shared memory (stable radix sort on the bits of
+// bin - bin0, end_bit = bits of bin1 - bin0): a run of equal bins then reserves its range with one global atomic.  A
+// window-by-window atomic would serialise in the L2 on the few hundred bins that hold most windows.  Inside a bin the
+// windows of a tile keep their id order.
+constexpr int kScatterThreads = 256, kScatterItems = 8, kScatterTile = kScatterThreads * kScatterItems;
+#ifdef __CUDACC__
+__global__ void __launch_bounds__(kScatterThreads) bin_scatter_kernel(int32_t n, const int32_t *key, int32_t *cursor, const int32_t *chunk_base,
+                                                                       int32_t *items, int32_t bin0, int32_t bin1, int end_bit) {
+  using Sort = cub::BlockRadixSort<uint32_t, kScatterThreads, kScatterItems, int32_t>;
+  using Scan = cub::BlockScan<int32_t, kScatterThreads>;
+  __shared__ union { typename Sort::TempStorage sort; typename Scan::TempStorage scan; uint32_t key[kScatterTile]; } sm;
+  __shared__ int32_t run_base[kScatterTile];
+  const uint32_t none = (uint32_t)(bin1 - bin0);   // invalid window, one that needs no phase 1, another sort's, past the end
+  const int p0 = threadIdx.x * kScatterItems;     // blocked: thread t holds tile positions p0 .. p0 + kScatterItems - 1
+  uint32_t k[kScatterItems];
+  int32_t w[kScatterItems];
+#pragma unroll
+  for (int i = 0; i < kScatterItems; ++i) {
+    const int64_t x = (int64_t)blockIdx.x * kScatterTile + p0 + i;
+    const int bin = x < n ? key[x] : -1;
+    k[i] = (bin >= bin0 && bin < bin1) ? (uint32_t)(bin - bin0) : none;
+    w[i] = (int32_t)x;
   }
+  Sort(sm.sort).Sort(k, w, 0, end_bit);   // stable: the tile in (bin, window id) order
+  __syncthreads();
+#pragma unroll
+  for (int i = 0; i < kScatterItems; ++i) sm.key[p0 + i] = k[i];
+  __syncthreads();
+  int32_t start[kScatterItems];   // first position of the item's run of equal bins
+  bool last[kScatterItems];       // the item ends its run
+#pragma unroll
+  for (int i = 0; i < kScatterItems; ++i) {
+    const int p = p0 + i;
+    start[i] = (p == 0 || sm.key[p - 1] != k[i]) ? p : 0;
+    last[i] = p == kScatterTile - 1 || sm.key[p + 1] != k[i];
+  }
+  __syncthreads();
+  Scan(sm.scan).InclusiveScan(start, start, cub::Max());
+#pragma unroll
+  for (int i = 0; i < kScatterItems; ++i)
+    if (k[i] != none && last[i]) run_base[start[i]] = atomicAdd(&cursor[bin0 + k[i]], p0 + i - start[i] + 1);
+  __syncthreads();
+#pragma unroll
+  for (int i = 0; i < kScatterItems; ++i)
+    if (k[i] != none) items[chunk_base[k[i] / kScanChunk] + run_base[start[i]] + (p0 + i - start[i])] = w[i];
 }
+#endif
 
 }  // namespace elector

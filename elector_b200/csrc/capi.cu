@@ -68,8 +68,8 @@ struct elector_ctx {
   cudaStream_t stream = nullptr;
   cudaStream_t side[16] = {};   // one per segment that does not run on the main stream
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_mid = nullptr, uev0 = nullptr, uev1 = nullptr, ev_fork = nullptr, ev_rows = nullptr;
-  cudaStream_t lin_stream = nullptr;   // the linear segments of phase 2 run next to phase 1
-  cudaEvent_t ev_fork_v[6] = {}, ev_sorted = nullptr, ev_lin_done = nullptr, ev_lin_sorted = nullptr;
+  cudaStream_t lin_stream = nullptr;   // the sort of the linear segments of phase 2 (next to that of phase 1), then the sort of the general ones
+  cudaEvent_t ev_fork_v[6] = {}, ev_sorted = nullptr, ev_lin_done = nullptr, ev_lin_sorted = nullptr, ev_bulk1 = nullptr;
   cudaEvent_t ev_view[3][2][2] = {};   // ELECTOR_TRACE=2: start / end of the launches of a view (phase 1, linear, general) x (cooperative, others)
   float last_ms_phase1 = 0.f;  // sort 1 + phase-1 kernels of the last run (last_ms covers everything)
   cudaEvent_t ev_join[16] = {};
@@ -312,11 +312,13 @@ int seg_resident(const elector_ctx *ctx, int phase, int kind) {
 }
 
 // scan + scatter + plan of one view, all on `st`
-int sort_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, int32_t n, int bgrid, SegStatic &ss, long long rows_cap, bool split_rows) {
+int sort_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, int32_t n, SegStatic &ss, long long rows_cap, bool split_rows) {
   const int nb = v.bin1 - v.bin0, nch = (nb + kScanChunk - 1) / kScanChunk;
   bin_scan_chunks_kernel<<<nch, kScanChunk, 0, st>>>(nb, v.hist + v.bin0, v.chunks);
   bin_scan_totals_kernel<<<1, 1024, 0, st>>>(nch, v.chunks, v.hist, v.dtab, v.seg0, v.seg1, v.bin0, v.bin1);
-  bin_scatter_kernel<<<bgrid, 256, 0, st>>>(n, v.key, v.hist, v.chunks, v.items, v.bin0, v.bin1);
+  const int end_bit = 32 - __builtin_clz((unsigned)nb);   // bits of bin - bin0, and of the "not in this view" key nb
+  bin_scatter_kernel<<<(int)(((int64_t)n + kScatterTile - 1) / kScatterTile), kScatterThreads, 0, st>>>(n, v.key, v.hist, v.chunks, v.items,
+                                                                                                        v.bin0, v.bin1, end_bit);
   memset(&ss, 0, sizeof ss);
   ss.seg0 = v.seg0; ss.seg1 = v.seg1; ss.phase = v.phase; ss.coop_group = std::max(1, ctx->coop_group); ss.counter0 = v.counter0;
   ss.pool_words = v.pool->cap / 4;
@@ -332,19 +334,21 @@ int sort_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, int32_t n, i
   return ELECTOR_OK;
 }
 
-// every segment of a view on its own side stream (side[first_side ...]), forked from and joined back into `st`
-// which: 0 = the warp-cooperative segments, 1 = the others, 2 = all (cooperative first).
+// every segment of a view on its own side stream (side[first_side ...]), forked from `fork_from` (default `st`) and joined
+// back into `st` by join_view.  which: 0 = the warp-cooperative segments, 1 = the others, 2 = all (cooperative first).
 // A segment with a large share of the call's windows (bulk) goes to `st` itself, behind the bulk segments launched before it;
-// the others get a side stream each, starting behind what `st` holds at this moment.  (Measured on config 1: two bulk kernels
+// the others get a side stream each, starting behind what `fork_from` holds at this moment.  (Measured on config 1: two bulk kernels
 // side by side are slower than one after the other -- each alone fills the SMs, together they evict each other's scratch
 // from the L2.)  join_view makes `st` wait for the side streams -- after ALL launches of a phase: a join between two passes
 // would serialise them.
-int launch_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, const SegStatic &ss, PoaArgs base, int first_side, bool region_b, int64_t n, int which = 2) {
+int launch_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, const SegStatic &ss, PoaArgs base, int first_side, bool region_b, int64_t n,
+                int which = 2, cudaStream_t fork_from = nullptr) {
+  if (!fork_from) fork_from = st;
   cudaEvent_t fork = ctx->ev_fork_v[(v.phase == 1 ? 0 : v.seg0 >= kFirstLinSeg2 ? 1 : 2) + (which == 1 ? 3 : 0)];
   const BinTable &plans = ctx->h_plan[v.phase - 1];   // read_plans
-  CU(cudaEventRecord(fork, st));
+  CU(cudaEventRecord(fork, fork_from));
   const int vi = v.phase == 1 ? 0 : v.seg0 >= kFirstLinSeg2 ? 1 : 2;
-  if (ctx->trace) for (int w2 = 0; w2 < 2; ++w2) if (which == 2 || which == w2) CU(cudaEventRecord(ctx->ev_view[vi][w2][0], st));
+  if (ctx->trace) for (int w2 = 0; w2 < 2; ++w2) if (which == 2 || which == w2) CU(cudaEventRecord(ctx->ev_view[vi][w2][0], fork_from));
   int nregb = 0;
   // the warp-cooperative segments first (they hold the longest windows and set the latency floor of a call)
   for (int pass = 0; pass < 2; ++pass)
@@ -373,12 +377,11 @@ int launch_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, const SegS
     }
   return ELECTOR_OK;
 }
-// The plans of a phase, read back (one wait of the host per phase): the host launches only the segments that have work, with
-// exact grids.  Measured on config 1: fixed-grid launches of all 27 segments (most of them empty, thousands of CTAs that leave
-// at once) cost 0.4 ms per phase, a read-back 0.03 ms.
-int read_plans(elector_ctx *ctx, int phase, BinTable *dtab, cudaStream_t a, cudaStream_t b) {
-  if (b) CU(cudaStreamSynchronize(b));
-  CU(cudaMemcpyAsync(&ctx->h_plan[phase - 1], dtab, sizeof(BinTable), cudaMemcpyDeviceToHost, a));
+// The plans of `ntab` tables from phase `phase` on, read back on `a` (one wait of the host, for `a` alone): the host launches
+// only the segments that have work, with exact grids.  Measured on config 1: fixed-grid launches of all 27 segments (most of
+// them empty, thousands of CTAs that leave at once) cost 0.4 ms per phase, a read-back 0.03 ms.
+int read_plans(elector_ctx *ctx, int phase, int ntab, BinTable *dtab, cudaStream_t a) {
+  CU(cudaMemcpyAsync(&ctx->h_plan[phase - 1], dtab, ntab * sizeof(BinTable), cudaMemcpyDeviceToHost, a));
   CU(cudaStreamSynchronize(a));
   return ELECTOR_OK;
 }
@@ -390,11 +393,13 @@ int join_view(elector_ctx *ctx, cudaStream_t st, int first, int count, int view)
   return ELECTOR_OK;
 }
 
-// Core: all pointers are device pointers; nothing here waits for the device.  Launch structure of one call:
-//   main stream  : set-up -> size sort (recognises the windows whose cor is ref) -> sort + plan of phase 1 and of the linear
-//                  segments of phase 2 -> phase-1 segments -> sort + plan of the general segments -> general segments
-//   linear stream: the linear segments of phase 2, as soon as their sort is done (they overlap phase 1)
-// Every segment runs on a side stream of its own.  h_roff / h_coff (host copies of the offsets) spare a read-back of four
+// Core: all pointers are device pointers; the host waits for the device twice, for the plans (read_plans).  Launch structure
+// of one call:
+//   main stream  : set-up -> size sort (recognises the windows whose cor is ref) -> sort + plan of phase 1 -> [read-back of
+//                  the plans of phase 1 and of the linear segments] -> phase-1 bulk -> linear bulk -> general bulk
+//   linear stream: sort + plan of the linear segments of phase 2 (next to that of phase 1); once phase 1 is done, sort + plan
+//                  of the general segments -> [read-back of their plans]
+// A segment that is not bulk runs on a side stream of its own.  h_roff / h_coff (host copies of the offsets) spare a read-back of four
 // totals; errors (bad window, scratch pool too small) are left in the tables, which travel to h_bintab at the end.
 int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_roff, const char *d_cor,
                const int64_t *d_coff, const char *d_unc, const int64_t *d_uoff, const int64_t *h_roff, const int64_t *h_coff,
@@ -465,8 +470,8 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   cudaStream_t sl = ctx->lin_stream;
   CU(cudaEventRecord(ctx->ev_sorted, st));
   CU(cudaStreamWaitEvent(sl, ctx->ev_sorted, 0));
-  int rc = sort_view(ctx, st, v1, (int32_t)n, bgrid, ss1, rows_cap, false);
-  if (rc == ELECTOR_OK) rc = sort_view(ctx, sl, vL, (int32_t)n, bgrid, ssL, rows_cap, ctx->split_rows);
+  int rc = sort_view(ctx, st, v1, (int32_t)n, ss1, rows_cap, false);
+  if (rc == ELECTOR_OK) rc = sort_view(ctx, sl, vL, (int32_t)n, ssL, rows_cap, ctx->split_rows);
   if (rc != ELECTOR_OK) return rc;
   CU(cudaEventRecord(ctx->ev_lin_sorted, sl));
 
@@ -485,40 +490,44 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   a.band_w = ctx->band_w;
   a.band_span = band_span_limit(ctx->sc.maxabs);
 
-  // ---- phase 1 ----
-  rc = read_plans(ctx, 1, dtab1, st, nullptr);
+  // ---- phase 1, then the linear segments of phase 2 behind it ----
+  // one read-back brings the plans of phase 1 and of the linear view (table 2; the general view's plans follow after sort 2)
+  CU(cudaStreamWaitEvent(st, ctx->ev_lin_sorted, 0));
+  rc = read_plans(ctx, 1, 2, dtab1, st);
   if (rc != ELECTOR_OK) return rc;
   if (ctx->wait_in[0]) CU(cudaStreamWaitEvent(st, ctx->wait_in[0], 0));
   rc = launch_view(ctx, st, v1, ss1, a, 0, false, n);
-  if (rc == ELECTOR_OK) rc = join_view(ctx, st, 0, 12, 0);
   if (rc != ELECTOR_OK) return rc;
-  CU(cudaEventRecord(ctx->ev_mid, st));
-  // ---- phase 2: the linear segments (sorted by the size sort; with two row regions theirs leaves for the host as soon as they
-  // are done) on the linear stream, the general segments (phase 1 filled their keys, histogram and maxima) on the main stream.
-  // Launch order: the warp-cooperative segments of both (the longest windows: the latency floor of the call), then the linear
-  // segments, then the general ones.
-  // (Starting the linear segments next to phase 1 was measured slower on config 1, 6.96 against 6.72 ms per step: the kernels of
-  // the two phases evict each other's scratch from the L2.)
+  CU(cudaEventRecord(ctx->ev_bulk1, st));
   PoaArgs al = a, ag = a;
   if (ctx->split_rows) {
     al.rows_cursor = ctx->d_ctrl.as<unsigned long long>() + 18;   // two row regions: the linear segments behind their own cursor, up to the end of the buffer
     ag.rows_cap_dev = reinterpret_cast<const long long *>(ctx->d_ctrl.as<unsigned long long>() + 19);   // the general region ends where the linear one starts
   }
-  rc = sort_view(ctx, st, v2, (int32_t)n, bgrid, ss2, rows_cap, false);
-  if (rc == ELECTOR_OK) rc = read_plans(ctx, 2, dtab2, st, sl);
-  if (rc != ELECTOR_OK) return rc;
+  // The linear segments need nothing from phase 1 (their windows skip it): their bulk runs on `st` right behind phase 1's,
+  // their cooperative segments on side streams forked there, so that they do not wait for phase 1's cooperative ones.
+  // (Starting them next to phase 1 instead was measured slower on config 1, 6.96 against 6.72 ms per step: the kernels of the
+  // two phases evict each other's scratch from the L2.)
   if (ctx->wait_in[1]) CU(cudaStreamWaitEvent(st, ctx->wait_in[1], 0));
-  CU(cudaStreamWaitEvent(st, ctx->ev_lin_sorted, 0));
-  rc = launch_view(ctx, st, vL, ssL, al, 12, ctx->split_rows, n, 0);
-  if (rc == ELECTOR_OK) rc = launch_view(ctx, st, v2, ss2, ag, 0, false, n, 0);
-  if (rc == ELECTOR_OK) rc = launch_view(ctx, st, vL, ssL, al, 12, ctx->split_rows, n, 1);
+  rc = launch_view(ctx, st, vL, ssL, al, 12, ctx->split_rows, n);
   if (rc != ELECTOR_OK) return rc;
   if (ctx->split_rows) {   // the copy stream learns where the linear region starts and ends as soon as its last segment is done
     CU(cudaMemcpyAsync(&ctx->h_totals[6], ctx->d_ctrl.as<unsigned long long>() + 18, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->copy_out));
     CU(cudaEventRecord(ctx->ev_lin, ctx->copy_out));
   }
   CU(cudaEventRecord(ctx->ev_lin_done, st));
-  rc = launch_view(ctx, st, v2, ss2, ag, 0, false, n, 1);
+  // ---- sort 2 on the linear stream once phase 1 is done (its bulk on `st`, its other segments on side[0 .. 11]) ----
+  CU(cudaStreamWaitEvent(sl, ctx->ev_bulk1, 0));
+  rc = join_view(ctx, sl, 0, 12, 0);
+  if (rc != ELECTOR_OK) return rc;
+  CU(cudaEventRecord(ctx->ev_mid, sl));
+  rc = sort_view(ctx, sl, v2, (int32_t)n, ss2, rows_cap, false);
+  if (rc == ELECTOR_OK) rc = read_plans(ctx, 2, 1, dtab2, sl);   // the host waits for sort 2 alone; the linear segments run meanwhile
+  if (rc != ELECTOR_OK) return rc;
+  if (ctx->wait_in[1]) CU(cudaStreamWaitEvent(sl, ctx->wait_in[1], 0));
+  // ---- the general segments of phase 2: bulk on `st` behind the linear bulk, the others forked from the linear stream
+  // (phase 1 and sort 2 are done there), on side[0 .. 11]: they never queue behind a linear segment ----
+  rc = launch_view(ctx, st, v2, ss2, ag, 0, false, n, 2, sl);
   if (rc == ELECTOR_OK) rc = join_view(ctx, st, 0, 16, 2);
   if (rc != ELECTOR_OK) return rc;
   CU(cudaMemcpyAsync(ctx->h_bintab, dtab1, 2 * sizeof(BinTable), cudaMemcpyDeviceToHost, st));   // errors and needs of the call
@@ -955,6 +964,7 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
       (e = cudaEventCreateWithFlags(&ctx->ev_sorted, cudaEventDisableTiming)) != cudaSuccess ||
       (e = cudaEventCreate(&ctx->ev_lin_done)) != cudaSuccess ||
       (e = cudaEventCreateWithFlags(&ctx->ev_lin_sorted, cudaEventDisableTiming)) != cudaSuccess ||
+      (e = cudaEventCreateWithFlags(&ctx->ev_bulk1, cudaEventDisableTiming)) != cudaSuccess ||
       (e = cudaStreamCreateWithFlags(&ctx->copy_in, cudaStreamNonBlocking)) != cudaSuccess ||
       (e = cudaStreamCreateWithFlags(&ctx->copy_out, cudaStreamNonBlocking)) != cudaSuccess ||
       (e = cudaMallocHost((void **)&ctx->h_bintab, 2 * sizeof(BinTable))) != cudaSuccess ||
@@ -1111,6 +1121,7 @@ void elector_poa_free(elector_ctx *ctx) {
   if (ctx->ev_lin_done) cudaEventDestroy(ctx->ev_lin_done);
   for (int k = 0; k < 6; ++k) if (ctx->ev_fork_v[k]) cudaEventDestroy(ctx->ev_fork_v[k]);
   if (ctx->ev_lin_sorted) cudaEventDestroy(ctx->ev_lin_sorted);
+  if (ctx->ev_bulk1) cudaEventDestroy(ctx->ev_bulk1);
   for (int k = 0; k < 12; ++k) if (ctx->ev_view[k / 4][(k / 2) & 1][k & 1]) cudaEventDestroy(ctx->ev_view[k / 4][(k / 2) & 1][k & 1]);
   if (ctx->lin_stream) cudaStreamDestroy(ctx->lin_stream);
   for (int k = 0; k < kSideStreams; ++k) {
