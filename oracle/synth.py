@@ -395,3 +395,261 @@ def letter_variants(win, n, seed):
             u = u[:p] + "ACGT"[rng.below(4)] + u[p + 1:]
         out.append(("%s v%d" % (name, i), ref.translate(tr), cor.translate(tr), u))
     return out
+
+
+# ---- merged reads at the edges of the tally kernel ----------------------------------------------------------------------
+def tally_constants():
+    """the constants of the tally kernel (tally_kernel.cuh), so that the edges of tally_edge_reads follow the code"""
+    src = open(os.path.join(_CSRC, "tally_kernel.cuh")).read()
+    out = {name: int(val) for name, val in re.findall(r"constexpr int (k\w+) = (\d+);", src)}
+    out.update((name, int(val)) for name, val in re.findall(r"\b(T_THRESH2?) = (\d+)", src))
+    return out
+
+
+def msa_background(rng, L, raw_rate=0.10, keep=0.1, max_run=3, max_crun=3):
+    """three aligned rows (R, C, U) of L columns with the error profile of config 1: every reference base has an error in the
+    uncorrected row with probability raw_rate (insertion, deletion or substitution), which the corrected row keeps with
+    probability `keep`.  No row has a dot run longer than max_run (max_crun for the corrected row) and the first and last three
+    columns are plain bases, so the background alone never reaches a border gap, a gap stretch or a cr threshold."""
+    R, C, U = [], [], []
+    while len(R) < L:
+        b = "ACGT"[rng.below(4)]
+        if rng.unit() < raw_rate:
+            k, kept, x = rng.below(3), rng.unit() < keep, "ACGT"[rng.below(4)]
+            if k == 0:
+                cols = [(".", x if kept else ".", x), (b, b, b)]
+            elif k == 1:
+                cols = [(b, "." if kept else b, ".")]
+            else:
+                cols = [(b, x if kept else b, x)]
+        else:
+            cols = [(b, b, b)]
+        for r, c, u in cols:
+            R.append(r); C.append(c); U.append(u)
+    R, C, U = R[:L], C[:L], U[:L]
+    run = [0, 0, 0]
+    for i in range(L):
+        run = [run[s] + 1 if row[i] == "." else 0 for s, row in enumerate((R, C, U))]
+        if i < 3 or i >= L - 3 or max(run[0], run[2]) > max_run or run[1] > max_crun:
+            R[i] = C[i] = U[i] = "ACGT"[rng.below(4)]
+            run = [0, 0, 0]
+    return R, C, U
+
+
+def gap_counters(C, R):
+    """(cg, cr) of findGapStretches (computeStats.py:104-189) after every column: the corrected-gap run and the reference-gap
+    counter that advances only while the previous corrected column is a gap"""
+    cg = cr = 0
+    prev, out = None, []
+    for c, r in zip(C, R):
+        if prev == ".":
+            if c == ".":
+                cg = cg + 1 if cg > 0 else 2
+            if r == ".":
+                cr = cr + 1 if cr > 0 else 2
+        if prev is None:
+            cg, cr = cg + (c == "."), cr + (r == ".")
+        if c != ".":
+            cg = 0
+        if r != ".":
+            cr = 0
+        out.append((cg, cr))
+        prev = c
+    return out
+
+
+def _runs(row):
+    out, i = set(), 0
+    while i < len(row):
+        if row[i] == ".":
+            j = i
+            while j + 1 < len(row) and row[j + 1] == ".":
+                j += 1
+            out.add("%d-%d" % (i, j))
+            i = j + 1
+        else:
+            i += 1
+    return out
+
+
+def tally_measures(R, C, U):
+    """what a tally edge tag may state about a merged read (values as strings): L, assessed, gl / gr (and per row glr, glu,
+    grr, gru), ext (extended), nk and keys (the sorted gap stretches, 'a-b,...' or 'none'), crun / rrun (maximal dot runs of
+    the corrected / reference row: a tag lists some of them), crmax (largest cr on a column where cg >= T_THRESH), dots2 /
+    dots3 (columns where exactly two / all three rows are dots), iupac (R or U holds a letter outside ACGTacgt), lower (R or C
+    holds g or c)"""
+    from oracle import tally_oracle as to
+    T = tally_constants()["T_THRESH"]
+    m = dict(L=len(R), assessed=int(len(R) > 10), glr=to.nb_left_gaps(R), glu=to.nb_left_gaps(U), grr=to.nb_right_gaps(R),
+             gru=to.nb_right_gaps(U), ext=to.tally_read(R, C, U)["extended"])
+    m["gl"], m["gr"] = min(m["glr"], m["glu"]), min(m["grr"], m["gru"])
+    keys = sorted(to.gap_stretch_keys(C, R))
+    m["nk"], m["keys"] = len(keys), ",".join("%d-%d" % k for k in keys) or "none"
+    m["crmax"] = max([cr for cg, cr in gap_counters(C, R) if cg >= T], default=0)
+    ndots = [(r == ".") + (c == ".") + (u == ".") for r, c, u in zip(R, C, U)]
+    m["dots2"], m["dots3"] = ndots.count(2), ndots.count(3)
+    m["iupac"] = int(any(ch not in "ACGTacgt." for ch in R + U))
+    m["lower"] = int(any(ch in "gc" for ch in R + C))
+    m = {k: str(v) for k, v in m.items()}
+    m["crun"], m["rrun"] = _runs(C), _runs(R)
+    return m
+
+
+def tally_tag_mismatches(tag, R, C, U):
+    """the (key, stated, measured) triples of a tally edge tag that the read does not have"""
+    m = tally_measures(R, C, U)
+    bad = []
+    for kv in tag.split()[1:]:          # the first word names the shape
+        k, v = kv.split("=")
+        if k in ("crun", "rrun"):
+            bad += [(k, r, "absent") for r in v.split(",") if r not in m[k]]
+        elif m[k] != v:
+            bad.append((k, v, m[k]))
+    return bad
+
+
+def _tally_shapes():
+    """(tag, L, segments, max_crun) of every tally edge read; a segment (pos, n, R, C, U) sets n columns from pos, each row
+    given as one character for all n columns or as n characters: 'b' is the column's base (the same in every row that has 'b'),
+    anything else is taken as it is.  Two plain columns on either side of each segment keep it apart from the background."""
+    k = tally_constants()
+    T, T2, S = k["T_THRESH"], k["T_THRESH2"], k["kSmemCols"]
+    STEP = 32 * 32                     # next_pair_warp: 32 lanes, one 32-column word each
+    out = []
+
+    def add(tag, L, segs, max_crun=3):
+        out.append((tag, L, segs, max_crun))
+
+    def dots(s, n):                    # n characters, dots at the offsets in s
+        return "".join("." if i in s else "b" for i in range(n))
+
+    # lengths: not assessed / assessed, 16-column groups, 32-column words, 1 024-column steps, the shared-memory bitmasks
+    for L in (10, 11, 15, 16, 17, 31, 32, 33, 1023, 1024, 1025, 2049, S - 1, S, S + 1, 65537, 150001):
+        sparse = 1 if L > S else 3     # long reads: no counting run of the corrected row but the ones placed here
+        add("len L=%d nk=0" % L, L, [], sparse)
+        if L <= 10:
+            continue
+        if L < 64:
+            add("lenb L=%d gl=%d gr=%d" % (L, T, T + 1), L, [(0, T, ".", "b", "."), (L - T, T, ".", "b", ".")])
+            if L > 30:
+                add("lenk L=%d keys=0-%d crun=2-%d" % (L, L - 1, L - 3), L, [(2, L - 4, "b", ".", "b")])
+            continue
+        segs = [(0, T, ".", "b", "."), (8, 33, "b", ".", "b"), (L - 40, 31, "b", ".", "b"), (L - 6, 6, ".", "b", ".")]
+        crun = ["8-40", "%d-%d" % (L - 40, L - 10)]
+        for j in range(1, min(L // STEP, 4) + 1):
+            if 100 < j * STEP < L - 100:
+                segs.append((j * STEP - 1, 2, "b", ".", "b")); crun.append("%d-%d" % (j * STEP - 1, j * STEP))
+        if L > S + 100:
+            segs.append((S - 1, 2, "b", ".", "b")); crun.append("%d-%d" % (S - 1, S))
+        add("lenb L=%d gl=%d gr=7 keys=0-40,%d-%d crun=%s" % (L, T, L - 40, L - 1, ",".join(crun)), L, segs, sparse)
+
+    # border gaps (nbLeftGaps / nbRightGaps and the extension): L = 400
+    L = 400
+    for n in (T - 1, T, T2 - 1, T2, T2 + 1):
+        g = n if n >= T else 0
+        add("bordl:n%d gl=%d ext=%d" % (n, g, g if g >= T2 else -1), L, [(0, n, ".", "b", ".")])
+        add("bordr:n%d gr=%d ext=%d" % (n, g + (g > 0), g + 1 if g + 1 >= T2 else -1), L, [(L - n, n, ".", "b", ".")])
+    for sep in (T, T + 1):             # two runs of T dots, sep bases apart: the second counts only while nt <= T
+        g = 2 * T + sep if sep == T else T
+        add("bordsepl:sep%d gl=%d" % (sep, g), L, [(0, T, ".", "b", "."), (T + sep, T, ".", "b", ".")])
+        add("bordsepr:sep%d gr=%d" % (sep, g + 1), L, [(L - T, T, ".", "b", "."), (L - 2 * T - sep, T, ".", "b", ".")])
+    add("bordw gl=40 gr=36 ext=76", L, [(0, 40, ".", "b", "."), (L - 35, 35, ".", "b", ".")])        # runs across a word
+    add("bordmin glr=20 glu=7 gl=7 grr=7 gru=26 gr=7", L, [(0, 20, ".", "b", dots(range(7), 20)), (L - 25, 25, dots(range(19, 25), 25), "b", ".")])
+    add("bordmin glr=6 glu=25 gl=6 grr=23 gru=10 gr=10 ext=-1", L, [(0, 25, dots(range(6), 25), "b", "."), (L - 22, 22, ".", "b", dots(range(13, 22), 22))])
+    # extension with corrected dots inside; on the right the count starts one column after L - gr (computeStats.py:490)
+    add("borde gl=25 gr=25 ext=45 dots3=5", L, [(0, 25, ".", dots({3, 4, 10}, 25), "."), (L - 25, 25, "b" + "." * 24, dots({0, 1, 24}, 25), "b" + "." * 24)])
+
+    # runs of the corrected row (find_gap_stretches / next_pair_warp): a stretch's first column shows in a key (a, L-1) when it
+    # ends within T2 columns of the right border, its last column in a key (0, b) when it starts within T2 of the left one
+    for a in (31, 32, 95, 96, STEP - 1, STEP, 2 * STEP - 1, 2 * STEP):
+        L = a + 40
+        add("crunr:a%d keys=%d-%d crun=%d-%d" % (a, a, L - 1, a, a + 30), L, [(a, 31, "b", ".", "b")], 1)
+    for b in (31, 32, 63, 64, STEP - 1, STEP, 2 * STEP - 1, 2 * STEP):
+        add("crunl:b%d keys=0-%d crun=8-%d" % (b, b, b), b + 200, [(8, b - 7, "b", ".", "b")], 1)
+    # the scan resumes after a 2-dot run at column 37, so the warp's steps start at word 1: a pair across the last word of one
+    add("crunstep keys=%d-%d crun=37-38,%d-%d" % (STEP + 31, STEP + 54, STEP + 31, STEP + 35), STEP + 55,
+        [(37, 2, "b", ".", "b"), (STEP + 31, 5, "b", ".", "b"), (STEP + 39, 12, "b", ".", "b")], 1)
+    # runs of 1 (column 0 and elsewhere), 2, 4, 5, 6 dots; a pair whose second dot opens a word; a run of n dots ends 4 bases
+    # before a stretch that reaches the right border: n >= T makes it a stretch of its own that the pending merge joins
+    for n in (1, 2, T - 1, T, T + 1):
+        L = 300
+        segs = [(0, 1, "b", ".", "b"), (50, 1, "b", ".", "b"), (63, 2, "b", ".", "b"), (100, 2, "b", ".", "b"), (110, 4, "b", ".", "b"),
+                (L - 45, n, "b", ".", "b"), (L - 45 + n + 3, 45 - n - 3 - 8, "b", ".", "b")]
+        ka = L - 45 if n >= T else L - 45 + n + 3
+        add("crunk:n%d keys=%d-%d crun=0-0,50-50,63-64,100-101,110-113,%d-%d" % (n, ka, L - 1, L - 45, L - 45 + n - 1), L, segs, 1)
+
+    # reference-gap runs (cr): inside a stretch of the corrected row, before it (sr < st, with and without corrected dots in
+    # between), from column 0, and words of a stretch without reference dots next to words with them
+    for n in (T2 - 2, T2 - 1, T2, T2 + 1, T2 + 2):
+        add("cr:n%d crmax=%d keys=0-%d" % (n, n, 8 + min(n, T2 - 1) - 1), 200, [(8, n, ".", ".", "b")], 1)
+    add("crsr:k0 keys=0-28 crmax=31", 200, [(3, 48, ".", dots(range(7, 38), 48), "b")], 1)            # R dots from 3, C run 10..40
+    add("crsr:k1 keys=0-27 crmax=32", 200, [(3, 48, ".", dots({2} | set(range(7, 38)), 48), "b")], 1)
+    add("crsr:k1dot keys=0-27 crmax=32 rrun=3-50", 200, [(2, 49, "b" + "." * 48, dots({0} | set(range(8, 39)), 49), "b")], 1)   # the dot before sr
+    add("crs0:k0 keys=0-28 rrun=0-50 crmax=31", 200, [(0, 51, ".", dots(range(10, 41), 51), "b")], 1)
+    add("crs0:k1 keys=0-27 rrun=0-50 crmax=32", 200, [(0, 51, ".", dots({0} | set(range(10, 41)), 51), "b")], 1)
+    # 15 single corrected dots inside the reference gap before the stretch: cr starts at 16 and no column qualifies until the
+    # reference gap ends
+    pre = set(range(2, 32, 2))
+    add("crpre keys=167-204 crun=150-190 rrun=100-170", 205,
+        [(100, 91, "." * 71 + "b" * 20, dots(pre | set(range(50, 91)), 91), "b")], 1)
+    add("crrb keys=0-167 crun=8-220 rrun=8-40,150-221", 300, [(8, 214, dots(set(range(33)) | set(range(142, 214)), 214), dots(range(213), 214), "b")], 1)
+    add("crrb keys=0-117 crun=8-300 rrun=100-301", 400, [(8, 294, dots(range(92, 294), 294), dots(range(293), 294), "b")], 1)
+
+    # stretches within T2 of a border, pending stretches T and T + 1 apart, overlapping keys, the most keys a read can have
+    for a in (T2, T2 + 1):
+        add("slotl:a%d keys=%s" % (a, "0-%d" % (a + 30) if a <= T2 else "none"), 300, [(a, 31, "b", ".", "b")], 1)
+    for d in (T2, T2 + 1):
+        L = 300
+        add("slotr:d%d keys=%s" % (d, "%d-%d" % (L - 60, L - 1) if d <= T2 else "none"), L, [(L - 60, 61 - d, "b", ".", "b")], 1)
+    for g in (T, T + 1):
+        L = 300
+        ka = L - 60 if g <= T else L - 45 + g
+        add("slotp:g%d keys=%d-%d" % (g, ka, L - 1), L, [(L - 60, 16, "b", ".", "b"), (L - 45 + g, 45 - g - 9, "b", ".", "b")], 1)
+    for L, r in ((200, (130, 150, 170)), (433, (370, 390, 410))):
+        # key 0 from a stretch at the left border; a stretch in the middle whose pending merge with the stretch that reaches the
+        # right border keeps its start; that stretch's own key once a last stretch inside the border merges with it
+        segs = [(3, 28, "b", ".", "b"), (L - 100, 21, "b", ".", "b"), (L - 76, 67, dots({x - (L - 76) for x in r}, 67), ".", "b"),
+                (L - 7, 5, "b", ".", "b")]
+        add("keys3 nk=3 keys=0-30,%d-%d,%d-%d" % (L - 100, L - 1, L - 76, L - 1), L, segs, 1)
+
+    # classification: case, N and IUPAC letters, columns with two or three dots
+    add("cls iupac=1 lower=1 dots3=1", 600,
+        [(100, 16, "gGcCaAtTNRYKMSWn", "gGcCaAtTgcGCacgt", "GgCcNnRYKMSWBDHV"), (200, 1, ".", ".", "."), (210, 1, ".", ".", "b"),
+         (220, 1, ".", "b", "."), (230, 1, "b", ".", "."), (300, 8, "NnRYacgt", "cCgGacgt", "gcGCNnKM")])
+    # mask ends (gapsLeft, L - gapsRight, both ends of a key) at every offset inside a 16-column group
+    for i in range(16):
+        L, gl, gr = 700 + i, T + i, T + 1 + (2 * i) % 16   # a right run of n dots is gr = n + 1
+        b = 40 + i
+        segs = [(0, b + 1, "." * gl + "b" * (b + 1 - gl), "b" * 6 + "." * (b - 5), "." * gl + "b" * (b + 1 - gl)),
+                (L - 45, 45, "b" * (46 - gr) + "." * (gr - 1), "." * 43 + "bb", "b" * (46 - gr) + "." * (gr - 1))]
+        add("mask:i%d gl=%d gr=%d keys=0-%d,%d-%d" % (i, gl, gr, b, L - 45, L - 1), L, segs, 1)
+    return out
+
+
+def tally_edge_reads(seed=11, copies=3):
+    """Merged reads (tag, R, C, U) at the edges of the tally kernel (tally_kernel.cuh): three rows of equal length without
+    'n' in C, as the merge leaves them.  Each shape of _tally_shapes comes in `copies` copies on different config-1
+    backgrounds (msa_background); its tag is 'group k=v ...' with measures tally_measures must find.
+
+    The most gap stretches (keys) a read can have is 3, below kMaxStretchKeys: a key other than 0 ends at L - 1, so it comes
+    from a pending entry merged into (or being) the first entry that ends at L - 1, i.e. the first stretch ending within T2
+    of the right border; every later stretch starts inside the border and is too short for a key.  Key 0 is the third
+    (group keys3 has all three), so the overflow branch of the kernel is dead code."""
+    out = []
+    for c in range(copies):
+        rng = SplitMix64(seed * 1000003 + c)
+        for tag, L, segs, max_crun in _tally_shapes():
+            R, C, U = msa_background(rng, L, max_crun=max_crun)
+            for pos, n, *_ in segs:                  # plain columns around every segment first, then the segments
+                for i in list(range(pos - 2, pos)) + list(range(pos + n, pos + n + 2)):
+                    if 0 <= i < L:
+                        R[i] = C[i] = U[i] = "ACGT"[rng.below(4)]
+            for pos, n, *rows in segs:
+                rows = [r * n if len(r) == 1 else r for r in rows]
+                assert all(len(r) == n for r in rows) and pos + n <= L, (tag, pos, n)
+                for i in range(n):
+                    b = "ACGT"[rng.below(4)]
+                    for row, ch in zip((R, C, U), (r[i] for r in rows)):
+                        row[pos + i] = b if ch == "b" else ch
+            out.append((tag, "".join(R), "".join(C), "".join(U)))
+    return out

@@ -1,5 +1,6 @@
 """GPU: merge (Donatello) + tally (computeStats) kernels through the C-ABI against the
-reference-generated goldens and the oracle."""
+reference-generated goldens and the oracle.  The reads at the kernels' own edges (long reads, word and step edges of
+the scanners, gap stretches, row offsets) are in tests/test_gpu_tally_edges.py."""
 import gzip
 import json
 import os
