@@ -11,6 +11,7 @@
 // Everything stays on the device; the host reads back one small table per phase.
 #pragma once
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
 
 #include "poa_kernel.cuh"
@@ -113,18 +114,42 @@ inline void fill_segments2(BinTable &t) {
   t.seg[kNumSegs2].first_bin = kNumBins2;
 }
 
-// set-up of one call on the device: control words (rows cursor = words 0..1), both segment tables
+// The control block of a call, shared by the host and the kernels.  The kernels take the addresses of its fields; the DP
+// kernels take the block itself as 32-bit words and index their work counters from its start (SegPlanDev::counter).
+// The head is what the host reads back after the alignment (and its tally_overflow after the tally).
+struct CallCtrlHead {
+  unsigned long long rows_cursor;   // next free byte of the rows (of the general region when the rows go to two regions)
+  int32_t row_error;                // the rows of a window did not fit
+  int32_t tally_overflow;           // a read has more border gap stretches than the tally's scanner holds
+};
+struct CallCtrl {
+  CallCtrlHead head;
+  int32_t work1[16];                // work counters of phase 1's segments
+  int32_t work2[16];                // work counters of phase 2's segments
+  unsigned long long lin_cursor;    // next free byte of the linear region (two row regions)
+  unsigned long long lin_start;     // where the linear region starts, and the general one ends
+  int32_t unused;
+  int32_t abort;                    // the alignment kernels of the call did not (all) run: merge, tally and wire pack leave at once
+  unsigned long long n_esc;         // escapes written by the wire pack of the merged rows
+  int32_t pad[20];
+};
+static_assert(offsetof(CallCtrl, head.rows_cursor) == 0 && offsetof(CallCtrl, head.row_error) == 2 * 4 && offsetof(CallCtrl, head.tally_overflow) == 3 * 4, "CallCtrl layout");
+static_assert(offsetof(CallCtrl, work1) == 4 * 4 && offsetof(CallCtrl, work2) == 20 * 4 && offsetof(CallCtrl, lin_cursor) == 36 * 4, "CallCtrl layout");
+static_assert(offsetof(CallCtrl, lin_start) == 38 * 4 && offsetof(CallCtrl, abort) == 41 * 4 && offsetof(CallCtrl, n_esc) == 42 * 4, "CallCtrl layout");
+static_assert(sizeof(CallCtrl) == 64 * 4 && kNumSegs1 <= 16 && kNumSegs2 <= 16, "CallCtrl layout");
+
+// set-up of one call on the device: control block, both segment tables
 struct SegFirstBins { int32_t first1[kMaxSegs + 1], first2[kMaxSegs + 1], nseg1, nbins1, nseg2, nbins2; };
-__global__ void init_call_kernel(int32_t *ctrl, int nctrl, unsigned long long cursor_init, BinTable *tabs, SegFirstBins fb) {
-  int32_t *t = reinterpret_cast<int32_t *>(tabs);
+__global__ void init_call_kernel(CallCtrl *ctrl, unsigned long long cursor_init, BinTable *tabs, SegFirstBins fb) {
+  int32_t *t = reinterpret_cast<int32_t *>(tabs), *c = reinterpret_cast<int32_t *>(ctrl);
   for (int i = threadIdx.x; i < (int)(2 * sizeof(BinTable) / 4); i += blockDim.x) t[i] = 0;
-  for (int i = threadIdx.x; i < nctrl; i += blockDim.x) ctrl[i] = 0;
+  for (int i = threadIdx.x; i < (int)(sizeof(CallCtrl) / 4); i += blockDim.x) c[i] = 0;
   __syncthreads();
   if ((int)threadIdx.x <= kMaxSegs) { tabs[0].seg[threadIdx.x].first_bin = fb.first1[threadIdx.x]; tabs[1].seg[threadIdx.x].first_bin = fb.first2[threadIdx.x]; }
   if (threadIdx.x == 0) {
     tabs[0].nseg = fb.nseg1; tabs[0].nbins = fb.nbins1; tabs[1].nseg = fb.nseg2; tabs[1].nbins = fb.nbins2;
     tabs[0].err_window = 0x7fffffff;
-    *reinterpret_cast<unsigned long long *>(ctrl) = cursor_init;
+    ctrl->head.rows_cursor = cursor_init;
   }
 }
 

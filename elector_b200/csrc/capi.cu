@@ -55,6 +55,17 @@ struct DevBuf {
   template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
 
+// pinned: what a context reads back from the device, one field per value (and copies of exactly its size)
+struct ReadBack {
+  int64_t off_totals[4];     // run_device without host offsets: last ref and cor offsets, then first ref and cor offsets
+  int64_t split_totals[4];   // split_device: windows, letters of ref / unc / cor
+  int32_t split_overflow;    // split_device: a triplet has more windows than its share of the record buffer
+  CallCtrlHead head;
+  struct { unsigned long long cursor, start; } lin;   // CallCtrl's lin_cursor and lin_start
+  int64_t merged_cols; unsigned long long n_esc;   // wire pack: merged columns and escapes
+  int64_t sums[ELECTOR_TALLY_K];
+};
+
 }  // namespace
 
 struct elector_ctx {
@@ -64,7 +75,7 @@ struct elector_ctx {
   int resident_ph1 = 0, resident_ph2 = 0, resident_ph1p = 0, resident_ph2l = 0, resident_coop = 0;  // POA kernel CTAs (one warp each) resident per SM
   int arena_ph1 = 0, arena_ph2 = 0, arena_ph1p = 0, arena_ph2l = 0, arena_ph2d = 0;   // bytes of the per-warp shared-memory arena of each kernel (fast part of the layouts)
   int coop_group = kCoopGroupDefault;  // windows per warp of the warp-cooperative kernel; 0 = the longest windows stay thread-per-window (ELECTOR_COOP_GROUP)
-  int64_t *h_totals = nullptr;             // pinned: letters of ref / cor of the current call
+  ReadBack *h_back = nullptr;              // pinned
   cudaStream_t stream = nullptr;
   cudaStream_t side[16] = {};   // one per segment that does not run on the main stream
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_mid = nullptr, uev0 = nullptr, uev1 = nullptr, ev_fork = nullptr, ev_rows = nullptr;
@@ -78,13 +89,13 @@ struct elector_ctx {
   cudaEvent_t ev_call = nullptr;                        // ELECTOR_TRACE: start of a pipelined call on the device
   ScoreMatrix mat;
   ScoringSetup sc;
-  DevBuf d_tab, d_ref, d_cor, d_unc, d_roff, d_coff, d_uoff, d_items, d_scratch, d_scratch_lin, d_scratch2, d_ctrl, d_hist, d_bintab, d_key, d_key2, d_n1, d_p1;
+  CallCtrl *d_ctrl = nullptr;
+  DevBuf d_tab, d_ref, d_cor, d_unc, d_roff, d_coff, d_uoff, d_items, d_scratch, d_scratch_lin, d_scratch2, d_hist, d_bintab, d_key, d_key2, d_n1, d_p1;
   DevBuf d_rows, d_rowoff, d_stride, d_nring, d_s1, d_s2, d_cells;
   int64_t merged_cap = 0;  // bytes per merged-row buffer of the last merge
   // worker contexts of the pipelined entry points (worker_slots): children on this device, one per extra worker thread
   std::vector<elector_ctx *> workers;
   std::vector<elector_ctx *> peers;   // worker contexts of elector_reads_pipeline_run on the other devices
-  int64_t *h_sums = nullptr;   // pinned: global counters of a chunk + the tally overflow flag
   DevBuf d_pk[3], d_exc_pos, d_exc_byte, d_rel, d_nib[3], d_esc_pos, d_esc_byte;   // compact wire format: packed letters, exceptions, 32-bit offsets in; 4-bit merged rows and their escapes out
   void *h_stage = nullptr; size_t h_stage_cap = 0;   // pinned staging of a chunk's 32-bit offsets
   DevBuf d_stretch; int64_t stretch_reads = 0;
@@ -97,9 +108,8 @@ struct elector_ctx {
   // rows of a pipelined chunk in two regions: the windows of the linear segments of phase 2 (most windows, finished early)
   // write theirs behind their own cursor, so that they can leave for the host while the general windows still compute
   bool split_rows = false;          // set by process_chunk around run_device
-  int64_t region_b_base = 0;        // out: where the linear region starts in the caller's row buffer
-  cudaEvent_t ev_lin = nullptr;     // the linear region is complete; its cursor and start are in h_totals[6..7]
-  cudaEvent_t ev_merged = nullptr;  // the merge of a chunk is done and its rows are packed for the wire (before the tally); the merged columns of the chunk are in h_totals[2]
+  cudaEvent_t ev_lin = nullptr;     // the linear region is complete; its cursor and start are in h_back->lin
+  cudaEvent_t ev_merged = nullptr;  // the merge of a chunk is done and its rows are packed for the wire (before the tally); h_back->merged_cols and n_esc hold their size
   cudaEvent_t wait_in[2] = {nullptr, nullptr};   // run_device: phase 1 / phase 2 wait for these (letters still on their way), when set
   cudaEvent_t ev_in[2] = {nullptr, nullptr};
   void *split_state = nullptr;   // device buffers of the window cutting (split_capi.inl)
@@ -126,16 +136,10 @@ struct elector_ctx {
     if (e_ != cudaSuccess) return ctx->fail(ELECTOR_ECUDA, "%s: %s", #call, cudaGetErrorString(e_)); \
   } while (0)
 
+#include "tally_capi.inl"   // ahead of process_chunk, which queues its merge-and-tally stage
+
 namespace {
 
-int merge_device(elector_ctx *ctx, int64_t n_reads, const int64_t *h_read_first, int64_t n_windows, const uint8_t *d_rows,
-                 int64_t rows_bytes, const int64_t *d_row_off, const int32_t *d_row_stride, const int32_t *d_nring);
-int tally_device(elector_ctx *ctx, int64_t n_reads, const uint8_t *dR, const uint8_t *dC, const uint8_t *dU,
-                 const int64_t *d_off, const int32_t *d_len, int64_t *d_counters, int64_t total_bytes);
-int check_scan_overflow(elector_ctx *ctx, int64_t n_reads);
-
-const size_t kCtrlWords = 64;  // d_ctrl: [0..1] rows cursor (u64), [2] error flag, [3] tally overflow, [4..19] phase-1 and [20..35] phase-2 work counters, [36..37] rows cursor of the linear region, [38..39] where that region starts, [41] abort flag
-const int kAbortWord = 41;     // d_ctrl[41]: the alignment kernels of the call did not (all) run; merge and tally leave at once
 const int kSideStreams = 16;   // >= kMaxSegs: no two segments of a phase share a side stream
 const int kScratchRetries = 3; // runs of an alignment again after its scratch pools were grown (check_tables)
 
@@ -231,9 +235,8 @@ __device__ uint32_t layout_words(int phase, int kind, int m0, int m1) {
 }
 
 // one warp: a segment per lane, then lane 0 adds up the scratch.  split_rows: the view is the linear one of a call whose rows
-// go to two regions -- the linear segments write [cap_a, rows_cap), the general ones [cursor, cap_a); ctrl64[18] = cursor of
-// the linear region, [19] = cap_a
-__global__ void plan_segments_kernel(BinTable *tab, SegStatic ss, unsigned long long *ctrl64, long long rows_cap, int split_rows) {
+// go to two regions -- the linear segments write [cap_a, rows_cap), the general ones [cursor, cap_a)
+__global__ void plan_segments_kernel(BinTable *tab, SegStatic ss, CallCtrl *ctrl, long long rows_cap, int split_rows) {
   __shared__ unsigned long long s_words[32];
   __shared__ int s_big;
   const int lane = threadIdx.x, s = ss.seg0 + lane;
@@ -272,11 +275,11 @@ __global__ void plan_segments_kernel(BinTable *tab, SegStatic ss, unsigned long 
       if (tab->err_code == 0) tab->err_code = s_big ? 4 : 3;
       if (total > tab->need_words) tab->need_words = total;
     }
-    if (overflow || invalid) reinterpret_cast<int32_t *>(ctrl64)[kAbortWord] = 1;   // merge and tally have nothing defined to work on
+    if (overflow || invalid) ctrl->abort = 1;   // merge and tally have nothing defined to work on
     if (split_rows) {
       const unsigned long long cap_a = (unsigned long long)((rows_cap - (long long)tab->lin_bytes) & ~15ll);
-      ctrl64[18] = cap_a;
-      ctrl64[19] = cap_a;
+      ctrl->lin_cursor = cap_a;
+      ctrl->lin_start = cap_a;
     }
   }
 }
@@ -287,7 +290,6 @@ struct SortView {
   int32_t *chunks;    // chunk totals of this view
   const int32_t *key; int32_t *items;
   DevBuf *pool;
-  int counter0;
 };
 
 // kernel of a segment (static: known before the sort runs, see SegStatic)
@@ -320,7 +322,8 @@ int sort_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, int32_t n, S
   bin_scatter_kernel<<<(int)(((int64_t)n + kScatterTile - 1) / kScatterTile), kScatterThreads, 0, st>>>(n, v.key, v.hist, v.chunks, v.items,
                                                                                                         v.bin0, v.bin1, end_bit);
   memset(&ss, 0, sizeof ss);
-  ss.seg0 = v.seg0; ss.seg1 = v.seg1; ss.phase = v.phase; ss.coop_group = std::max(1, ctx->coop_group); ss.counter0 = v.counter0;
+  ss.seg0 = v.seg0; ss.seg1 = v.seg1; ss.phase = v.phase; ss.coop_group = std::max(1, ctx->coop_group);
+  ss.counter0 = (int32_t)((v.phase == 1 ? offsetof(CallCtrl, work1) : offsetof(CallCtrl, work2)) / sizeof(int32_t));
   ss.pool_words = v.pool->cap / 4;
   ss.budget_words = ((unsigned long long)24 << 30) / 4;
   for (int s = v.seg0; s < v.seg1; ++s) {
@@ -328,7 +331,7 @@ int sort_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, int32_t n, S
     ss.kind[s] = (int8_t)kind;
     ss.grid[s] = std::max(1, seg_resident(ctx, v.phase, kind)) * ctx->sm_count;
   }
-  plan_segments_kernel<<<1, 32, 0, st>>>(v.dtab, ss, ctx->d_ctrl.as<unsigned long long>(), rows_cap, split_rows ? 1 : 0);
+  plan_segments_kernel<<<1, 32, 0, st>>>(v.dtab, ss, ctx->d_ctrl, rows_cap, split_rows ? 1 : 0);
   CU(cudaGetLastError());
   ctx->last_launches += 4;
   return ELECTOR_OK;
@@ -364,7 +367,7 @@ int launch_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, const SegS
       cudaStream_t ls = bulk ? st : ctx->side[side];
       if (!bulk) CU(cudaStreamWaitEvent(ls, fork, 0));
       PoaArgs a = base;
-      a.tab = v.dtab; a.seg = s; a.items_base = v.items; a.scratch_base = v.pool->as<uint32_t>(); a.ctrl = ctx->d_ctrl.as<int32_t>();
+      a.tab = v.dtab; a.seg = s; a.items_base = v.items; a.scratch_base = v.pool->as<uint32_t>(); a.ctrl = reinterpret_cast<int32_t *>(ctx->d_ctrl);
       const bool linear_seg = v.phase == 2 && s >= kFirstLinSeg2;
       const cudaError_t e = ctx->sc.generic_sub ? launch_phase<true>(v.phase, kind, ls, a, grid, ctx->d_tab.as<SymbolTables>(), ss.coop_group, linear_seg, ctx)
                                                 : launch_phase<false>(v.phase, kind, ls, a, grid, ctx->d_tab.as<SymbolTables>(), ss.coop_group, linear_seg, ctx);
@@ -400,11 +403,11 @@ int join_view(elector_ctx *ctx, cudaStream_t st, int first, int count, int view)
 //   linear stream: sort + plan of the linear segments of phase 2 (next to that of phase 1); once phase 1 is done, sort + plan
 //                  of the general segments -> [read-back of their plans]
 // A segment that is not bulk runs on a side stream of its own.  h_roff / h_coff (host copies of the offsets) spare a read-back of four
-// totals; errors (bad window, scratch pool too small) are left in the tables, which travel to h_bintab at the end.
+// totals; errors (bad window, scratch pool too small) are left in the tables, which travel to h_bintab at the end (the rows cursor to h_back).
 int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_roff, const char *d_cor,
                const int64_t *d_coff, const char *d_unc, const int64_t *d_uoff, const int64_t *h_roff, const int64_t *h_coff,
                char *d_rows, int64_t rows_cap, int64_t *d_rowoff, int32_t *d_stride, int32_t *d_nring, int32_t *d_s1, int32_t *d_s2,
-               int64_t *d_cells, unsigned long long *d_cursor, int32_t *d_errflag, int64_t cursor_init = 0) {
+               int64_t *d_cells, int64_t cursor_init = 0) {
   if (n == 0) return ELECTOR_OK;
   if (n > 0x7fffffff - 64) return ctx->fail(ELECTOR_EINVAL, "too many windows in one call");
   cudaStream_t st = ctx->stream;
@@ -421,12 +424,12 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   int64_t tot[4];
   if (h_roff && h_coff) { tot[0] = h_roff[n]; tot[1] = h_coff[n]; tot[2] = h_roff[0]; tot[3] = h_coff[0]; }
   else {   // slow path: a read-back
-    CU(cudaMemcpyAsync(&ctx->h_totals[0], d_roff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&ctx->h_totals[1], d_coff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&ctx->h_totals[2], d_roff, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&ctx->h_totals[3], d_coff, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[0], d_roff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[1], d_coff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[2], d_roff, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[3], d_coff, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    for (int k = 0; k < 4; ++k) tot[k] = ctx->h_totals[k];
+    for (int k = 0; k < 4; ++k) tot[k] = ctx->h_back->off_totals[k];
   }
   CU(ctx->d_p1.reserve((size_t)(tot[0] - tot[2] + tot[1] - tot[3] + 8 * n + 8) * sizeof(uint16_t)));
   // scratch pools: kept from call to call; a call that needs more says so in its tables and its caller runs it again (check_tables)
@@ -445,7 +448,7 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
     SegFirstBins fb;
     for (int k = 0; k <= kMaxSegs; ++k) { fb.first1[k] = htab1->seg[k].first_bin; fb.first2[k] = htab2->seg[k].first_bin; }
     fb.nseg1 = htab1->nseg; fb.nbins1 = htab1->nbins; fb.nseg2 = htab2->nseg; fb.nbins2 = htab2->nbins;
-    init_call_kernel<<<1, 128, 0, st>>>(ctx->d_ctrl.as<int32_t>(), (int)kCtrlWords, (unsigned long long)cursor_init, dtab1, fb);
+    init_call_kernel<<<1, 128, 0, st>>>(ctx->d_ctrl, (unsigned long long)cursor_init, dtab1, fb);
     CU(cudaGetLastError());
     ++ctx->last_launches;
   }
@@ -461,9 +464,9 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   CU(cudaGetLastError());
   ++ctx->last_launches;
   const int lin_bin0 = kBigTiers + kSmallBins2;
-  const SortView v1{dtab1, 1, 0, kNumSegs1, 0, kNumBins1, hist1, chunks1, ctx->d_key.as<int32_t>(), items1, &ctx->d_scratch, 4};
-  const SortView vL{dtab2, 2, kFirstLinSeg2, kNumSegs2, lin_bin0, kNumBins2, hist2, chunksL, ctx->d_key2.as<int32_t>(), itemsL, &ctx->d_scratch_lin, 20};
-  const SortView v2{dtab2, 2, 0, kFirstLinSeg2, 0, lin_bin0, hist2, chunks2, ctx->d_key2.as<int32_t>(), items2, &ctx->d_scratch2, 20};
+  const SortView v1{dtab1, 1, 0, kNumSegs1, 0, kNumBins1, hist1, chunks1, ctx->d_key.as<int32_t>(), items1, &ctx->d_scratch};
+  const SortView vL{dtab2, 2, kFirstLinSeg2, kNumSegs2, lin_bin0, kNumBins2, hist2, chunksL, ctx->d_key2.as<int32_t>(), itemsL, &ctx->d_scratch_lin};
+  const SortView v2{dtab2, 2, 0, kFirstLinSeg2, 0, lin_bin0, hist2, chunks2, ctx->d_key2.as<int32_t>(), items2, &ctx->d_scratch2};
   SegStatic ss1, ssL, ss2;
   // the sort of phase 1 on the main stream; that of the linear segments of phase 2 (their keys and histogram are complete
   // after the size sort) on the linear stream, next to phase 1
@@ -484,9 +487,9 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   a.ro0 = tot[2]; a.co0 = tot[3];
   a.p1_nodes = ctx->d_p1.as<uint16_t>(); a.n1 = ctx->d_n1.as<int32_t>(); a.key2 = ctx->d_key2.as<int32_t>();
   a.hist2 = hist2; a.seg2_max = dtab2->seg_max;
-  a.rows_out = (uint8_t *)d_rows; a.rows_cursor = d_cursor; a.rows_cap = rows_cap;
+  a.rows_out = (uint8_t *)d_rows; a.rows_cursor = &ctx->d_ctrl->head.rows_cursor; a.rows_cap = rows_cap;
   a.row_off = d_rowoff; a.row_stride = d_stride; a.nring = d_nring; a.score1 = d_s1; a.score2 = d_s2; a.cells = d_cells;
-  a.error_flag = d_errflag;
+  a.error_flag = &ctx->d_ctrl->head.row_error;
   a.band_w = ctx->band_w;
   a.band_span = band_span_limit(ctx->sc.maxabs);
 
@@ -501,8 +504,8 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   CU(cudaEventRecord(ctx->ev_bulk1, st));
   PoaArgs al = a, ag = a;
   if (ctx->split_rows) {
-    al.rows_cursor = ctx->d_ctrl.as<unsigned long long>() + 18;   // two row regions: the linear segments behind their own cursor, up to the end of the buffer
-    ag.rows_cap_dev = reinterpret_cast<const long long *>(ctx->d_ctrl.as<unsigned long long>() + 19);   // the general region ends where the linear one starts
+    al.rows_cursor = &ctx->d_ctrl->lin_cursor;   // two row regions: the linear segments behind their own cursor, up to the end of the buffer
+    ag.rows_cap_dev = reinterpret_cast<const long long *>(&ctx->d_ctrl->lin_start);   // the general region ends where the linear one starts
   }
   // The linear segments need nothing from phase 1 (their windows skip it): their bulk runs on `st` right behind phase 1's,
   // their cooperative segments on side streams forked there, so that they do not wait for phase 1's cooperative ones.
@@ -512,7 +515,7 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   rc = launch_view(ctx, st, vL, ssL, al, 12, ctx->split_rows, n);
   if (rc != ELECTOR_OK) return rc;
   if (ctx->split_rows) {   // the copy stream learns where the linear region starts and ends as soon as its last segment is done
-    CU(cudaMemcpyAsync(&ctx->h_totals[6], ctx->d_ctrl.as<unsigned long long>() + 18, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->copy_out));
+    CU(cudaMemcpyAsync(&ctx->h_back->lin, &ctx->d_ctrl->lin_cursor, sizeof ctx->h_back->lin, cudaMemcpyDeviceToHost, ctx->copy_out));
     CU(cudaEventRecord(ctx->ev_lin, ctx->copy_out));
   }
   CU(cudaEventRecord(ctx->ev_lin_done, st));
@@ -532,6 +535,7 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   if (rc != ELECTOR_OK) return rc;
   CU(cudaMemcpyAsync(ctx->h_bintab, dtab1, 2 * sizeof(BinTable), cudaMemcpyDeviceToHost, st));   // errors and needs of the call
   CU(cudaEventRecord(ctx->ev1, st));
+  CU(cudaMemcpyAsync(&ctx->h_back->head, &ctx->d_ctrl->head, sizeof(CallCtrlHead), cudaMemcpyDeviceToHost, st));
   return ELECTOR_OK;
 }
 
@@ -539,7 +543,7 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
 // and has been grown: run the call again
 int check_tables(elector_ctx *ctx) {
   const BinTable *t1 = ctx->h_bintab, *t2 = ctx->h_bintab + 1;
-  if (t1->err_code || t2->err_code) cudaMemsetAsync(ctx->d_ctrl.as<int32_t>() + kAbortWord, 0, sizeof(int32_t), ctx->stream);   // for stand-alone merge / tally calls
+  if (t1->err_code || t2->err_code) cudaMemsetAsync(&ctx->d_ctrl->abort, 0, sizeof(int32_t), ctx->stream);   // for stand-alone merge / tally calls
   if (t1->err_code == 1) return ctx->fail(ELECTOR_EINVAL, "window %d has an empty sequence (undefined in the reference)", t1->err_window);
   if (t1->err_code == 2) return ctx->fail(ELECTOR_ETOOLARGE, "window %d: a sequence longer than %d letters, or reference + corrected longer than %d (16-bit node indices)", t1->err_window, kMaxWindowLen, kMaxNodes);
   if (t1->err_code == 4 || t2->err_code == 4) return ctx->fail(ELECTOR_ETOOLARGE, "a segment of the call needs %llu MiB of scratch (windows too long)", (unsigned long long)((std::max(t1->need_words, t2->need_words) * 4) >> 20));
@@ -597,11 +601,9 @@ int align_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *
                  const char *d_unc, const int64_t *d_uoff, const int64_t *h_roff, const int64_t *h_coff, char *d_rows, int64_t rows_cap,
                  int64_t *d_rowoff, int32_t *d_stride, int32_t *d_nring, int32_t *d_s1, int32_t *d_s2, int64_t *d_cells, int64_t *d_rows_used) {
   for (int attempt = 0;; ++attempt) {
-    int rc = run_device(ctx, n, d_ref, d_roff, d_cor, d_coff, d_unc, d_uoff, h_roff, h_coff, d_rows, rows_cap, d_rowoff, d_stride, d_nring, d_s1, d_s2,
-                        d_cells, ctx->d_ctrl.as<unsigned long long>(), ctx->d_ctrl.as<int32_t>() + 2);
+    int rc = run_device(ctx, n, d_ref, d_roff, d_cor, d_coff, d_unc, d_uoff, h_roff, h_coff, d_rows, rows_cap, d_rowoff, d_stride, d_nring, d_s1, d_s2, d_cells);
     if (rc != ELECTOR_OK) return rc;
-    if (d_rows_used) CU(cudaMemcpyAsync(d_rows_used, ctx->d_ctrl.p, sizeof(int64_t), cudaMemcpyDeviceToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(&ctx->h_totals[4], ctx->d_ctrl.p, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    if (d_rows_used) CU(cudaMemcpyAsync(d_rows_used, &ctx->d_ctrl->head.rows_cursor, sizeof(int64_t), cudaMemcpyDeviceToDevice, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));   // the one wait of the alignment
     if (n == 0) return ELECTOR_OK;            // run_device queued nothing: no tables, no times
     rc = check_tables(ctx);
@@ -610,10 +612,17 @@ int align_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *
     break;
   }
   add_kernel_ms(ctx);
-  if ((int32_t)(ctx->h_totals[5] & 0xffffffff)) return ctx->fail(ELECTOR_ECAPACITY, "row buffer capacity %lld too small", (long long)rows_cap);
+  if (ctx->h_back->head.row_error) return ctx->fail(ELECTOR_ECAPACITY, "row buffer capacity %lld too small", (long long)rows_cap);
   return ELECTOR_OK;
 }
 
+// device buffers of an alignment's outputs for nw windows into rows_bytes of rows, and of the tally of its n_reads reads
+int reserve_outputs(elector_ctx *ctx, int64_t nw, int64_t rows_bytes, int64_t n_reads) {
+  CU(ctx->d_rows.reserve(rows_bytes)); CU(ctx->d_rowoff.reserve(nw * 8)); CU(ctx->d_stride.reserve(nw * 4));
+  CU(ctx->d_nring.reserve(nw * 4)); CU(ctx->d_s1.reserve(nw * 4)); CU(ctx->d_s2.reserve(nw * 4)); CU(ctx->d_cells.reserve(nw * 8));
+  if (n_reads > 0) CU(ctx->d_tally_out.reserve(n_reads * ELECTOR_TALLY_K * 8));
+  return ELECTOR_OK;
+}
 
 struct ChunkJob { int64_t w0, w1, r0, r1, rows_base, rows_len, m_base; bool split; int index; };
 struct PipeArgs {
@@ -643,9 +652,8 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64
   const char *h_let[3] = {io.ref, io.cor, io.unc};
   const elector_packed *h_pk[3] = {io.pref, io.pcor, io.punc};
   for (int k = 0; k < 3; ++k) { CU(d_let[k]->reserve(len[k] + 8)); CU(d_off[k]->reserve((nw + 1) * 8)); }
-  CU(ctx->d_rows.reserve(j.rows_len)); CU(ctx->d_rowoff.reserve(nw * 8)); CU(ctx->d_stride.reserve(nw * 4));
-  CU(ctx->d_nring.reserve(nw * 4)); CU(ctx->d_s1.reserve(nw * 4)); CU(ctx->d_s2.reserve(nw * 4)); CU(ctx->d_cells.reserve(nw * 8));
-  if (nr > 0) { CU(ctx->d_tally_out.reserve(nr * ELECTOR_TALLY_K * 8)); CU(ctx->d_sums.reserve(ELECTOR_TALLY_K * 8)); }
+  int rc = reserve_outputs(ctx, nw, j.rows_len, nr);
+  if (rc != ELECTOR_OK) return rc;
   // compact wire format: the 32-bit offsets of the chunk (relative to its first letter) are made here, on the worker's
   // thread, while the chunks before it are on their way; the exceptions of the chunk are found by binary search
   int64_t exc0[3] = {0, 0, 0}, exc1[3] = {0, 0, 0};
@@ -757,54 +765,21 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64
   const bool want_merged = io.m_ref != nullptr;
   for (int attempt = 0;; ++attempt) {
     ctx->split_rows = j.split && want_rows;
-    int rc = run_device(ctx, nw, ctx->d_ref.as<char>() - br0, ctx->d_roff.as<int64_t>(), ctx->d_cor.as<char>() - bc0, ctx->d_coff.as<int64_t>(),
-                        ctx->d_unc.as<char>() - bu0, ctx->d_uoff.as<int64_t>(), pa.ro + w0, pa.co + w0, d_rows_v, j.rows_base + j.rows_len,
-                        ctx->d_rowoff.as<int64_t>(), ctx->d_stride.as<int32_t>(), ctx->d_nring.as<int32_t>(), ctx->d_s1.as<int32_t>(),
-                        ctx->d_s2.as<int32_t>(), ctx->d_cells.as<int64_t>(), ctx->d_ctrl.as<unsigned long long>(), ctx->d_ctrl.as<int32_t>() + 2, j.rows_base);
+    rc = run_device(ctx, nw, ctx->d_ref.as<char>() - br0, ctx->d_roff.as<int64_t>(), ctx->d_cor.as<char>() - bc0, ctx->d_coff.as<int64_t>(),
+                    ctx->d_unc.as<char>() - bu0, ctx->d_uoff.as<int64_t>(), pa.ro + w0, pa.co + w0, d_rows_v, j.rows_base + j.rows_len,
+                    ctx->d_rowoff.as<int64_t>(), ctx->d_stride.as<int32_t>(), ctx->d_nring.as<int32_t>(), ctx->d_s1.as<int32_t>(),
+                    ctx->d_s2.as<int32_t>(), ctx->d_cells.as<int64_t>(), j.rows_base);
     const bool split = ctx->split_rows;
     ctx->split_rows = false;
     if (rc != ELECTOR_OK) { ctx->wait_in[0] = ctx->wait_in[1] = nullptr; cudaStreamSynchronize(ctx->copy_in); cudaStreamSynchronize(st); return rc; }
-    CU(cudaMemcpyAsync(&ctx->h_totals[4], ctx->d_ctrl.p, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
     CU(cudaEventRecord(ctx->ev_rows, st));
     if (nr > 0) {
       std::vector<int64_t> rf(io.read_first + r0, io.read_first + r1 + 1);
       for (int64_t &v : rf) v -= w0;
-      CU(cudaMemsetAsync(ctx->d_sums.p, 0, ELECTOR_TALLY_K * 8, st));
-      rc = merge_device(ctx, nr, rf.data(), nw, reinterpret_cast<const uint8_t *>(d_rows_v), 3 * (br + bc + bu), ctx->d_rowoff.as<int64_t>(),
-                        ctx->d_stride.as<int32_t>(), ctx->d_nring.as<int32_t>());
+      const WirePack pack{io.m_nibbles, j.m_base, io.m_esc_cap};
+      rc = queue_merge_tally(ctx, nr, rf.data(), nw, reinterpret_cast<const uint8_t *>(d_rows_v), 3 * (br + bc + bu), ctx->d_rowoff.as<int64_t>(), ctx->d_stride.as<int32_t>(),
+                             ctx->d_nring.as<int32_t>(), ctx->d_tally_out.as<int64_t>(), true, want_merged ? &pack : nullptr, nullptr, ctx->ev1);   // ev1: the chunk's device time covers merge + tally too
       if (rc != ELECTOR_OK) { ctx->wait_in[0] = ctx->wait_in[1] = nullptr; cudaStreamSynchronize(st); return rc; }
-      // the merged rows are packed and on their way before the tally runs: the copy stream takes them while the tally kernels run
-      if (want_merged && io.m_nibbles == 2) {   // one byte per column for the three rows together; characters outside the code go to the escape list
-        CU(ctx->d_nib[0].reserve((size_t)ctx->merged_cap + 16));
-        CU(ctx->d_esc_pos.reserve((size_t)(io.m_esc_cap + 3) * 8)); CU(ctx->d_esc_byte.reserve((size_t)io.m_esc_cap + 8));
-        CU(cudaMemsetAsync(ctx->d_ctrl.as<unsigned long long>() + 21, 0, 8, st));
-        column_pack_kernel<<<(unsigned)nr, 128, 0, st>>>(nr, ctx->d_mref.as<uint8_t>(), ctx->d_mcor.as<uint8_t>(), ctx->d_munc.as<uint8_t>(),
-            ctx->d_moff.as<int64_t>(), ctx->d_mlen.as<int32_t>(), ctx->d_nib[0].as<uint8_t>(), j.m_base,
-            ctx->d_ctrl.as<unsigned long long>() + 21, ctx->d_esc_pos.as<int64_t>(), ctx->d_esc_byte.as<uint8_t>(), io.m_esc_cap, ctx->d_ctrl.as<int32_t>() + kAbortWord);
-        CU(cudaGetLastError());
-        ++ctx->last_launches;
-      } else if (want_merged && io.m_nibbles) {   // two columns per byte before they leave; the few characters outside the code go to the escape list
-        for (int k = 0; k < 3; ++k) CU(ctx->d_nib[k].reserve((size_t)ctx->merged_cap / 2 + 16));
-        CU(ctx->d_esc_pos.reserve((size_t)(io.m_esc_cap + 1) * 8)); CU(ctx->d_esc_byte.reserve((size_t)io.m_esc_cap + 8));
-        CU(cudaMemsetAsync(ctx->d_ctrl.as<unsigned long long>() + 21, 0, 8, st));
-        nibble_pack_kernel<<<(unsigned)((3 * nr + 3) / 4), 128, 0, st>>>(nr, ctx->d_mref.as<uint8_t>(), ctx->d_mcor.as<uint8_t>(), ctx->d_munc.as<uint8_t>(),
-            ctx->d_moff.as<int64_t>(), ctx->d_mlen.as<int32_t>(), ctx->d_nib[0].as<uint8_t>(), ctx->d_nib[1].as<uint8_t>(), ctx->d_nib[2].as<uint8_t>(), j.m_base,
-            ctx->d_ctrl.as<unsigned long long>() + 21, ctx->d_esc_pos.as<int64_t>(), ctx->d_esc_byte.as<uint8_t>(), io.m_esc_cap, ctx->d_ctrl.as<int32_t>() + kAbortWord);
-        CU(cudaGetLastError());
-        ++ctx->last_launches;
-      }
-      CU(cudaMemcpyAsync(&ctx->h_totals[2], ctx->d_moff.as<int64_t>() + nr, sizeof(int64_t), cudaMemcpyDeviceToHost, st));      // merged columns of the chunk
-      CU(cudaMemcpyAsync(&ctx->h_totals[3], ctx->d_ctrl.as<unsigned long long>() + 21, sizeof(int64_t), cudaMemcpyDeviceToHost, st));   // escapes
-      CU(cudaEventRecord(ctx->ev_merged, st));
-      rc = tally_device(ctx, nr, ctx->d_mref.as<uint8_t>(), ctx->d_mcor.as<uint8_t>(), ctx->d_munc.as<uint8_t>(), ctx->d_moff.as<int64_t>(),
-                        ctx->d_mlen.as<int32_t>(), ctx->d_tally_out.as<int64_t>(), ctx->merged_cap);
-      if (rc != ELECTOR_OK) { ctx->wait_in[0] = ctx->wait_in[1] = nullptr; cudaStreamSynchronize(st); return rc; }
-      tally_sum_kernel<<<std::min<int>(64, (int)((nr + 7) / 8)), 256, 0, st>>>(nr, ctx->d_tally_out.as<int64_t>(), ctx->d_sums.as<unsigned long long>());
-      CU(cudaGetLastError());
-      ++ctx->last_launches;
-      CU(cudaEventRecord(ctx->ev1, st));   // the chunk's device time covers merge + tally too
-      CU(cudaMemcpyAsync(ctx->h_sums, ctx->d_sums.p, ELECTOR_TALLY_K * 8, cudaMemcpyDeviceToHost, st));
-      CU(cudaMemcpyAsync(ctx->h_sums + ELECTOR_TALLY_K, ctx->d_ctrl.as<int32_t>() + 3, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
       if (io.counters_out) CU(cudaMemcpyAsync(io.counters_out + r0 * ELECTOR_TALLY_K, ctx->d_tally_out.p, nr * ELECTOR_TALLY_K * 8, cudaMemcpyDeviceToHost, st));
       if (io.m_off) CU(cudaMemcpyAsync(io.m_off + r0, ctx->d_moff.p, nr * 8, cudaMemcpyDeviceToHost, st));
       if (io.m_len) CU(cudaMemcpyAsync(io.m_len + r0, ctx->d_mlen.p, nr * 4, cudaMemcpyDeviceToHost, st));
@@ -815,7 +790,7 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64
     int64_t base_b = end_b, used_b = end_b;
     if (split) {
       CU(cudaEventSynchronize(ctx->ev_lin));
-      used_b = ctx->h_totals[6]; base_b = ctx->h_totals[7];
+      used_b = (int64_t)ctx->h_back->lin.cursor; base_b = (int64_t)ctx->h_back->lin.start;
       if (base_b >= j.rows_base && used_b > base_b && used_b <= end_b)
         CU(cudaMemcpyAsync(io.rows_out + base_b, d_rows_v + base_b, used_b - base_b, cudaMemcpyDeviceToHost, so));
     }
@@ -830,8 +805,8 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64
       continue;
     }
     if (rc != ELECTOR_OK) { cudaStreamSynchronize(st); cudaStreamSynchronize(so); return rc == 1 ? ctx->fail(ELECTOR_ECUDA, "scratch pools keep overflowing") : rc; }
-    const int64_t used = ctx->h_totals[4];
-    if ((int32_t)(ctx->h_totals[5] & 0xffffffff) || used > base_b || used_b > end_b) {
+    const int64_t used = (int64_t)ctx->h_back->head.rows_cursor;
+    if (ctx->h_back->head.row_error || used > base_b || used_b > end_b) {
       cudaStreamSynchronize(st);
       cudaStreamSynchronize(so);
       return ctx->fail(ELECTOR_ECAPACITY, "rows of a chunk exceed their bound (%lld + %lld > %lld)", (long long)(used - j.rows_base), (long long)(used_b - base_b),
@@ -848,7 +823,7 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64
     if (io.cells) CU(cudaMemcpyAsync(io.cells + w0, ctx->d_cells.p, nw * 8, cudaMemcpyDeviceToHost, so));
     if (nr > 0 && want_merged) {   // the merged rows: their size is known once the merge has run
       CU(cudaEventSynchronize(ctx->ev_merged));
-      const int64_t cols = ctx->h_totals[2];
+      const int64_t cols = ctx->h_back->merged_cols;
       if (j.m_base + cols > io.m_cap) { cudaStreamSynchronize(st); cudaStreamSynchronize(so); return ctx->fail(ELECTOR_ECAPACITY, "merged rows need more than m_cap = %lld columns", (long long)io.m_cap); }
       char *dst[3] = {io.m_ref, io.m_cor, io.m_unc};
       DevBuf *srcb[3] = {&ctx->d_mref, &ctx->d_mcor, &ctx->d_munc};
@@ -858,7 +833,7 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64
         else CU(cudaMemcpyAsync(dst[k] + j.m_base, srcb[k]->p, (size_t)cols, cudaMemcpyDeviceToHost, so));
       }
       if (io.m_nibbles) {
-        const int64_t ne = ctx->h_totals[3];
+        const int64_t ne = (int64_t)ctx->h_back->n_esc;
         if (ne > 0) {
           const long long at = pa.n_esc->fetch_add(ne);
           if (at + ne > io.m_esc_cap || ne > io.m_esc_cap) { cudaStreamSynchronize(st); cudaStreamSynchronize(so); return ctx->fail(ELECTOR_ECAPACITY, "more than m_esc_cap = %lld characters outside the 4-bit code", (long long)io.m_esc_cap); }
@@ -884,11 +859,9 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64
   }
   add_kernel_ms(ctx);
   if (nr > 0) {
-    if ((int32_t)ctx->h_sums[ELECTOR_TALLY_K]) {
-      cudaMemsetAsync(ctx->d_ctrl.as<int32_t>() + 3, 0, sizeof(int32_t), st);
-      return ctx->fail(ELECTOR_EUNSUPPORTED, "a read has more than %d gap stretches at its borders", kMaxStretchKeys);
-    }
-    for (int f = 0; f < ELECTOR_TALLY_K; ++f) sums[f] += ctx->h_sums[f];
+    rc = tally_status(ctx);
+    if (rc != ELECTOR_OK) return rc;
+    for (int f = 0; f < ELECTOR_TALLY_K; ++f) sums[f] += ctx->h_back->sums[f];
   }
   return ELECTOR_OK;
 }
@@ -969,11 +942,10 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
       (e = cudaStreamCreateWithFlags(&ctx->copy_out, cudaStreamNonBlocking)) != cudaSuccess ||
       (e = cudaMallocHost((void **)&ctx->h_bintab, 2 * sizeof(BinTable))) != cudaSuccess ||
       (e = cudaMallocHost((void **)&ctx->h_plan, 2 * sizeof(BinTable))) != cudaSuccess ||
-      (e = cudaMallocHost((void **)&ctx->h_totals, 8 * sizeof(int64_t))) != cudaSuccess ||
-      (e = cudaMallocHost((void **)&ctx->h_sums, (ELECTOR_TALLY_K + 1) * sizeof(int64_t))) != cudaSuccess ||
+      (e = cudaMallocHost((void **)&ctx->h_back, sizeof(ReadBack))) != cudaSuccess ||
       (e = ctx->d_tab.reserve(sizeof(SymbolTables))) != cudaSuccess ||
-      (e = ctx->d_ctrl.reserve(kCtrlWords * sizeof(int32_t))) != cudaSuccess ||
-      (e = cudaMemset(ctx->d_ctrl.p, 0, kCtrlWords * sizeof(int32_t))) != cudaSuccess ||
+      (e = cudaMalloc((void **)&ctx->d_ctrl, sizeof(CallCtrl))) != cudaSuccess ||
+      (e = cudaMemset(ctx->d_ctrl, 0, sizeof(CallCtrl))) != cudaSuccess ||
       (e = cudaMemcpy(ctx->d_tab.p, &ctx->sc.tab, sizeof(SymbolTables), cudaMemcpyHostToDevice)) != cudaSuccess) {
     ctx->fail(ELECTOR_ECUDA, "context setup: %s", cudaGetErrorString(e));
     return bail(ELECTOR_ECUDA);
@@ -1098,9 +1070,9 @@ void elector_poa_free(elector_ctx *ctx) {
   for (elector_ctx *w : ctx->peers) { cudaSetDevice(w->device); elector_poa_free(w); }   // their buffers and streams belong to their device
   if (!ctx->peers.empty()) cudaSetDevice(ctx->device);
   ctx->peers.clear();
-  if (ctx->h_sums) cudaFreeHost(ctx->h_sums);
+  if (ctx->d_ctrl) cudaFree(ctx->d_ctrl);
   DevBuf *bufs[] = {&ctx->d_tab, &ctx->d_ref, &ctx->d_cor, &ctx->d_unc, &ctx->d_roff, &ctx->d_coff, &ctx->d_uoff,
-                    &ctx->d_items, &ctx->d_scratch, &ctx->d_scratch_lin, &ctx->d_scratch2, &ctx->d_ctrl, &ctx->d_hist, &ctx->d_bintab, &ctx->d_key, &ctx->d_key2, &ctx->d_n1, &ctx->d_p1, &ctx->d_rows, &ctx->d_rowoff, &ctx->d_stride,
+                    &ctx->d_items, &ctx->d_scratch, &ctx->d_scratch_lin, &ctx->d_scratch2, &ctx->d_hist, &ctx->d_bintab, &ctx->d_key, &ctx->d_key2, &ctx->d_n1, &ctx->d_p1, &ctx->d_rows, &ctx->d_rowoff, &ctx->d_stride,
                     &ctx->d_nring, &ctx->d_s1, &ctx->d_s2, &ctx->d_cells, &ctx->d_wdst, &ctx->d_sums, &ctx->d_stretch, &ctx->d_tally_scan, &ctx->d_tally_out,
                     &ctx->d_readfirst, &ctx->d_mtot, &ctx->d_moff, &ctx->d_mlen, &ctx->d_mref, &ctx->d_mcor, &ctx->d_munc};
   for (DevBuf *b : bufs) b->release();
@@ -1133,7 +1105,7 @@ void elector_poa_free(elector_ctx *ctx) {
   if (ctx->ev_call) cudaEventDestroy(ctx->ev_call);
   if (ctx->copy_in) cudaStreamDestroy(ctx->copy_in);
   if (ctx->copy_out) cudaStreamDestroy(ctx->copy_out);
-  if (ctx->h_totals) cudaFreeHost(ctx->h_totals);
+  if (ctx->h_back) cudaFreeHost(ctx->h_back);
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
 }
@@ -1450,6 +1422,5 @@ int elector_last_kernel_ms(const elector_ctx *ctx, float *ms, int *launches) {
 
 }  // extern "C"
 
-#include "tally_capi.inl"
 #include "split_capi.inl"
 #include "report_capi.inl"
