@@ -37,6 +37,10 @@ thread_local std::string g_init_error;
 struct DevBuf {
   void *p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf &) = delete;
+  DevBuf &operator=(const DevBuf &) = delete;
+  ~DevBuf() { release(); }
   cudaError_t reserve(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
     if (p) cudaFree(p);
@@ -55,6 +59,54 @@ struct DevBuf {
   template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
 
+// T's in pinned host memory (Device: in device memory); reserve allocates exactly `bytes` when it has to grow
+template <class T, bool Device = false> struct Mem {
+  T *p = nullptr;
+  size_t cap = 0;
+  Mem() = default;
+  Mem(const Mem &) = delete;
+  Mem &operator=(const Mem &) = delete;
+  ~Mem() { release(); }
+  cudaError_t reserve(size_t bytes) {
+    if (bytes <= cap) return cudaSuccess;
+    release();
+    const cudaError_t e = Device ? cudaMalloc((void **)&p, bytes) : cudaMallocHost((void **)&p, bytes);
+    if (e == cudaSuccess) cap = bytes;
+    return e;
+  }
+  void release() {
+    if (p) Device ? cudaFree(p) : cudaFreeHost(p);
+    p = nullptr;
+    cap = 0;
+  }
+  T *operator->() const { return p; }
+  operator T *() const { return p; }
+};
+
+// a CUDA stream or event owned by its holder; it converts to the plain handle
+template <class H, cudaError_t (*Destroy)(H)> struct Handle {
+  H h = nullptr;
+  Handle() = default;
+  Handle(const Handle &) = delete;
+  Handle &operator=(const Handle &) = delete;
+  ~Handle() { if (h) Destroy(h); }
+  operator H() const { return h; }
+};
+struct Stream : Handle<cudaStream_t, cudaStreamDestroy> {
+  cudaError_t create() { return cudaStreamCreateWithFlags(&h, cudaStreamNonBlocking); }
+  cudaError_t create(int prio) { return cudaStreamCreateWithPriority(&h, cudaStreamNonBlocking, prio); }
+};
+struct Event : Handle<cudaEvent_t, cudaEventDestroy> {
+  cudaError_t create(unsigned flags) { return cudaEventCreateWithFlags(&h, flags); }
+};
+
+const int kSideStreams = 16;   // >= kMaxSegs: no two segments of a phase share a side stream
+
+// device buffers of the window cutting (split_capi.inl), allocated by the first split
+struct SplitBufs {
+  DevBuf let[3], pk[3], off[3], order, hl, st_in, pool, wins, win_off, job_n, job_l, status, kidx, nrec, nl[3], base[4], w_off[3], w_let[3], rf, misc;
+};
+
 // pinned: what a context reads back from the device, one field per value (and copies of exactly its size)
 struct ReadBack {
   int64_t off_totals[4];     // run_device without host offsets: last ref and cor offsets, then first ref and cor offsets
@@ -69,27 +121,26 @@ struct ReadBack {
 }  // namespace
 
 struct elector_ctx {
-  int device = 0;
+  int device = -1;   // set by create_context once the device is known to exist
   int sm_count = 0;
-  size_t smem_optin = 0;
   int resident_ph1 = 0, resident_ph2 = 0, resident_ph1p = 0, resident_ph2l = 0, resident_coop = 0;  // POA kernel CTAs (one warp each) resident per SM
   int arena_ph1 = 0, arena_ph2 = 0, arena_ph1p = 0, arena_ph2l = 0, arena_ph2d = 0;   // bytes of the per-warp shared-memory arena of each kernel (fast part of the layouts)
   int coop_group = kCoopGroupDefault;  // windows per warp of the warp-cooperative kernel; 0 = the longest windows stay thread-per-window (ELECTOR_COOP_GROUP)
-  ReadBack *h_back = nullptr;              // pinned
-  cudaStream_t stream = nullptr;
-  cudaStream_t side[16] = {};   // one per segment that does not run on the main stream
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_mid = nullptr, uev0 = nullptr, uev1 = nullptr, ev_fork = nullptr, ev_rows = nullptr;
-  cudaStream_t lin_stream = nullptr;   // the sort of the linear segments of phase 2 (next to that of phase 1), then the sort of the general ones
-  cudaEvent_t ev_fork_v[6] = {}, ev_sorted = nullptr, ev_lin_done = nullptr, ev_lin_sorted = nullptr, ev_bulk1 = nullptr;
-  cudaEvent_t ev_view[3][2][2] = {};   // ELECTOR_TRACE=2: start / end of the launches of a view (phase 1, linear, general) x (cooperative, others)
+  Mem<ReadBack> h_back;
+  Stream stream;
+  Stream side[kSideStreams];   // one per segment that does not run on the main stream
+  Event ev0, ev1, ev_mid, uev0, uev1, ev_fork, ev_rows;
+  Stream lin_stream;   // the sort of the linear segments of phase 2 (next to that of phase 1), then the sort of the general ones
+  Event ev_fork_v[6], ev_sorted, ev_lin_done, ev_lin_sorted, ev_bulk1;
+  Event ev_view[3][2][2];   // ELECTOR_TRACE=2: start / end of the launches of a view (phase 1, linear, general) x (cooperative, others)
   float last_ms_phase1 = 0.f;  // sort 1 + phase-1 kernels of the last run (last_ms covers everything)
-  cudaEvent_t ev_join[16] = {};
-  elector::BinTable *h_bintab = nullptr;  // pinned: the two tables of the last call as the device left them (errors, scratch needs)
-  cudaStream_t copy_in = nullptr, copy_out = nullptr;   // H2D / D2H of the pipelined host entry point
-  cudaEvent_t ev_call = nullptr;                        // ELECTOR_TRACE: start of a pipelined call on the device
+  Event ev_join[kSideStreams];
+  Mem<elector::BinTable> h_bintab;   // the two tables of the last call as the device left them (errors, scratch needs)
+  Stream copy_in, copy_out;   // H2D / D2H of the pipelined host entry point
+  Event ev_call;              // ELECTOR_TRACE: start of a pipelined call on the device
   ScoreMatrix mat;
   ScoringSetup sc;
-  CallCtrl *d_ctrl = nullptr;
+  Mem<CallCtrl, true> d_ctrl;
   DevBuf d_tab, d_ref, d_cor, d_unc, d_roff, d_coff, d_uoff, d_items, d_scratch, d_scratch_lin, d_scratch2, d_hist, d_bintab, d_key, d_key2, d_n1, d_p1;
   DevBuf d_rows, d_rowoff, d_stride, d_nring, d_s1, d_s2, d_cells;
   int64_t merged_cap = 0;  // bytes per merged-row buffer of the last merge
@@ -97,27 +148,34 @@ struct elector_ctx {
   std::vector<elector_ctx *> workers;
   std::vector<elector_ctx *> peers;   // worker contexts of elector_reads_pipeline_run on the other devices
   DevBuf d_pk[3], d_exc_pos, d_exc_byte, d_rel, d_nib[3], d_esc_pos, d_esc_byte;   // compact wire format: packed letters, exceptions, 32-bit offsets in; 4-bit merged rows and their escapes out
-  void *h_stage = nullptr; size_t h_stage_cap = 0;   // pinned staging of a chunk's 32-bit offsets
+  Mem<int32_t> h_stage;   // staging of a chunk's 32-bit offsets
   DevBuf d_stretch; int64_t stretch_reads = 0;
   DevBuf d_wdst, d_sums, d_tally_scan, d_tally_out, d_readfirst, d_mtot, d_moff, d_mlen, d_mref, d_mcor, d_munc;
   bool trace = false;
   int band_w = 6;          // ELECTOR_BAND_W: base half-width of the diagonal band of the packed linear kernels (+ rows/16 in phase 1, + rows/8 in phase 2; 0 = full DP)
   int resident_ph2d = 0;   // 0: the general windows of phase 2 run the INT32 kernel with frontier sets
   unsigned side_used = 0;        // side streams with launches that `st` has not been made to wait for yet
-  elector::BinTable *h_plan = nullptr;   // pinned: the plans of phase 1 / phase 2 of the current call (read_plans)
+  Mem<elector::BinTable> h_plan;   // the plans of phase 1 / phase 2 of the current call (read_plans)
   // rows of a pipelined chunk in two regions: the windows of the linear segments of phase 2 (most windows, finished early)
   // write theirs behind their own cursor, so that they can leave for the host while the general windows still compute
-  bool split_rows = false;          // set by process_chunk around run_device
-  cudaEvent_t ev_lin = nullptr;     // the linear region is complete; its cursor and start are in h_back->lin
-  cudaEvent_t ev_merged = nullptr;  // the merge of a chunk is done and its rows are packed for the wire (before the tally); h_back->merged_cols and n_esc hold their size
+  bool split_rows = false;   // set by process_chunk around run_device
+  Event ev_lin;              // the linear region is complete; its cursor and start are in h_back->lin
+  Event ev_merged;           // the merge of a chunk is done and its rows are packed for the wire (before the tally); h_back->merged_cols and n_esc hold their size
   cudaEvent_t wait_in[2] = {nullptr, nullptr};   // run_device: phase 1 / phase 2 wait for these (letters still on their way), when set
-  cudaEvent_t ev_in[2] = {nullptr, nullptr};
-  void *split_state = nullptr;   // device buffers of the window cutting (split_capi.inl)
-  cudaEvent_t ev_split0 = nullptr, ev_split1 = nullptr, ev_mt0 = nullptr, ev_mt1 = nullptr;   // window cutting; merge + tally of elector_reads_run
+  Event ev_in[2];
+  SplitBufs split;
+  Event ev_split0, ev_split1, ev_mt0, ev_mt1;   // window cutting; merge + tally of elector_reads_run
   float last_ms_split = 0.f, last_ms_tally = 0.f;
   std::string err;
   float last_ms = 0.f;
   int last_launches = 0;
+
+  // the members free themselves; the worker and peer contexts free theirs, each on its own device
+  ~elector_ctx() {
+    for (elector_ctx *w : workers) delete w;
+    for (elector_ctx *w : peers) delete w;
+    if (device >= 0) cudaSetDevice(device);
+  }
 
   int fail(int code, const char *fmt, ...) {
     char buf[512];
@@ -140,7 +198,6 @@ struct elector_ctx {
 
 namespace {
 
-const int kSideStreams = 16;   // >= kMaxSegs: no two segments of a phase share a side stream
 const int kScratchRetries = 3; // runs of an alignment again after its scratch pools were grown (check_tables)
 
 #ifndef EL_MIN_WARPS_PH1P
@@ -367,7 +424,7 @@ int launch_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, const SegS
       cudaStream_t ls = bulk ? st : ctx->side[side];
       if (!bulk) CU(cudaStreamWaitEvent(ls, fork, 0));
       PoaArgs a = base;
-      a.tab = v.dtab; a.seg = s; a.items_base = v.items; a.scratch_base = v.pool->as<uint32_t>(); a.ctrl = reinterpret_cast<int32_t *>(ctx->d_ctrl);
+      a.tab = v.dtab; a.seg = s; a.items_base = v.items; a.scratch_base = v.pool->as<uint32_t>(); a.ctrl = reinterpret_cast<int32_t *>(ctx->d_ctrl.p);
       const bool linear_seg = v.phase == 2 && s >= kFirstLinSeg2;
       const cudaError_t e = ctx->sc.generic_sub ? launch_phase<true>(v.phase, kind, ls, a, grid, ctx->d_tab.as<SymbolTables>(), ss.coop_group, linear_seg, ctx)
                                                 : launch_phase<false>(v.phase, kind, ls, a, grid, ctx->d_tab.as<SymbolTables>(), ss.coop_group, linear_seg, ctx);
@@ -396,18 +453,29 @@ int join_view(elector_ctx *ctx, cudaStream_t st, int first, int count, int view)
   return ELECTOR_OK;
 }
 
+// An alignment's n windows: letters and offsets of ref, cor and unc on the device; h_roff / h_coff, host copies of the ref / cor
+// offsets, may be NULL
+struct AlignIn {
+  int64_t n;
+  const char *ref; const int64_t *roff; const char *cor; const int64_t *coff; const char *unc; const int64_t *uoff;
+  const int64_t *h_roff, *h_coff;
+};
+// its outputs on the device: rows_cap bytes of rows and the per-window arrays
+struct AlignOut {
+  char *rows; int64_t rows_cap;
+  int64_t *rowoff; int32_t *stride, *nring, *s1, *s2; int64_t *cells;
+};
+
 // Core: all pointers are device pointers; the host waits for the device twice, for the plans (read_plans).  Launch structure
 // of one call:
 //   main stream  : set-up -> size sort (recognises the windows whose cor is ref) -> sort + plan of phase 1 -> [read-back of
 //                  the plans of phase 1 and of the linear segments] -> phase-1 bulk -> linear bulk -> general bulk
 //   linear stream: sort + plan of the linear segments of phase 2 (next to that of phase 1); once phase 1 is done, sort + plan
 //                  of the general segments -> [read-back of their plans]
-// A segment that is not bulk runs on a side stream of its own.  h_roff / h_coff (host copies of the offsets) spare a read-back of four
+// A segment that is not bulk runs on a side stream of its own.  in.h_roff / in.h_coff (host copies of the offsets) spare a read-back of four
 // totals; errors (bad window, scratch pool too small) are left in the tables, which travel to h_bintab at the end (the rows cursor to h_back).
-int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_roff, const char *d_cor,
-               const int64_t *d_coff, const char *d_unc, const int64_t *d_uoff, const int64_t *h_roff, const int64_t *h_coff,
-               char *d_rows, int64_t rows_cap, int64_t *d_rowoff, int32_t *d_stride, int32_t *d_nring, int32_t *d_s1, int32_t *d_s2,
-               int64_t *d_cells, int64_t cursor_init = 0) {
+int run_device(elector_ctx *ctx, const AlignIn &in, const AlignOut &out, int64_t cursor_init = 0) {
+  const int64_t n = in.n;
   if (n == 0) return ELECTOR_OK;
   if (n > 0x7fffffff - 64) return ctx->fail(ELECTOR_EINVAL, "too many windows in one call");
   cudaStream_t st = ctx->stream;
@@ -422,12 +490,12 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   int32_t *items1 = ctx->d_items.as<int32_t>(), *itemsL = items1 + n, *items2 = itemsL + n;
   // letters of ref and cor of the call (size of the P1 node lists) and their first offsets
   int64_t tot[4];
-  if (h_roff && h_coff) { tot[0] = h_roff[n]; tot[1] = h_coff[n]; tot[2] = h_roff[0]; tot[3] = h_coff[0]; }
+  if (in.h_roff && in.h_coff) { tot[0] = in.h_roff[n]; tot[1] = in.h_coff[n]; tot[2] = in.h_roff[0]; tot[3] = in.h_coff[0]; }
   else {   // slow path: a read-back
-    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[0], d_roff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[1], d_coff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[2], d_roff, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[3], d_coff, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[0], in.roff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[1], in.coff + n, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[2], in.roff, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&ctx->h_back->off_totals[3], in.coff, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     for (int k = 0; k < 4; ++k) tot[k] = ctx->h_back->off_totals[k];
   }
@@ -459,8 +527,8 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   // the warp-cooperative kernel (which rebuilds lin(ref)) for the long ones.
   const bool ident_ok = ctx->sc.small_packed() && ctx->coop_group > 0;
   if (ident_ok && ctx->wait_in[0]) CU(cudaStreamWaitEvent(st, ctx->wait_in[0], 0));
-  IdentArgs ida{(const uint8_t *)d_ref, (const uint8_t *)d_cor, ctx->d_n1.as<int32_t>(), ctx->d_key2.as<int32_t>(), hist2, dtab2->seg_max, d_s1, &dtab2->lin_bytes};
-  bin1_count_kernel<<<bgrid, 256, 0, st>>>((int32_t)n, d_roff, d_coff, d_uoff, ctx->d_key.as<int32_t>(), hist1, dtab1, ident_ok, ida);
+  IdentArgs ida{(const uint8_t *)in.ref, (const uint8_t *)in.cor, ctx->d_n1.as<int32_t>(), ctx->d_key2.as<int32_t>(), hist2, dtab2->seg_max, out.s1, &dtab2->lin_bytes};
+  bin1_count_kernel<<<bgrid, 256, 0, st>>>((int32_t)n, in.roff, in.coff, in.uoff, ctx->d_key.as<int32_t>(), hist1, dtab1, ident_ok, ida);
   CU(cudaGetLastError());
   ++ctx->last_launches;
   const int lin_bin0 = kBigTiers + kSmallBins2;
@@ -473,22 +541,22 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   cudaStream_t sl = ctx->lin_stream;
   CU(cudaEventRecord(ctx->ev_sorted, st));
   CU(cudaStreamWaitEvent(sl, ctx->ev_sorted, 0));
-  int rc = sort_view(ctx, st, v1, (int32_t)n, ss1, rows_cap, false);
-  if (rc == ELECTOR_OK) rc = sort_view(ctx, sl, vL, (int32_t)n, ssL, rows_cap, ctx->split_rows);
+  int rc = sort_view(ctx, st, v1, (int32_t)n, ss1, out.rows_cap, false);
+  if (rc == ELECTOR_OK) rc = sort_view(ctx, sl, vL, (int32_t)n, ssL, out.rows_cap, ctx->split_rows);
   if (rc != ELECTOR_OK) return rc;
   CU(cudaEventRecord(ctx->ev_lin_sorted, sl));
 
   PoaArgs a;
   memset(&a, 0, sizeof a);
-  a.ref = (const uint8_t *)d_ref; a.cor = (const uint8_t *)d_cor; a.unc = (const uint8_t *)d_unc;
-  a.ref_off = d_roff; a.cor_off = d_coff; a.unc_off = d_uoff;
+  a.ref = (const uint8_t *)in.ref; a.cor = (const uint8_t *)in.cor; a.unc = (const uint8_t *)in.unc;
+  a.ref_off = in.roff; a.cor_off = in.coff; a.unc_off = in.uoff;
   a.match = ctx->sc.match; a.mismatch = ctx->sc.mismatch; a.open = ctx->sc.open; a.ext = ctx->sc.ext;
   { Scoring pk; pk.set(a.match, a.mismatch, a.open, a.ext); a.mis2 = pk.mis2; a.nopen2 = pk.nopen2; a.ext2 = pk.ext2; }
   a.ro0 = tot[2]; a.co0 = tot[3];
   a.p1_nodes = ctx->d_p1.as<uint16_t>(); a.n1 = ctx->d_n1.as<int32_t>(); a.key2 = ctx->d_key2.as<int32_t>();
   a.hist2 = hist2; a.seg2_max = dtab2->seg_max;
-  a.rows_out = (uint8_t *)d_rows; a.rows_cursor = &ctx->d_ctrl->head.rows_cursor; a.rows_cap = rows_cap;
-  a.row_off = d_rowoff; a.row_stride = d_stride; a.nring = d_nring; a.score1 = d_s1; a.score2 = d_s2; a.cells = d_cells;
+  a.rows_out = (uint8_t *)out.rows; a.rows_cursor = &ctx->d_ctrl->head.rows_cursor; a.rows_cap = out.rows_cap;
+  a.row_off = out.rowoff; a.row_stride = out.stride; a.nring = out.nring; a.score1 = out.s1; a.score2 = out.s2; a.cells = out.cells;
   a.error_flag = &ctx->d_ctrl->head.row_error;
   a.band_w = ctx->band_w;
   a.band_span = band_span_limit(ctx->sc.maxabs);
@@ -524,7 +592,7 @@ int run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_
   rc = join_view(ctx, sl, 0, 12, 0);
   if (rc != ELECTOR_OK) return rc;
   CU(cudaEventRecord(ctx->ev_mid, sl));
-  rc = sort_view(ctx, sl, v2, (int32_t)n, ss2, rows_cap, false);
+  rc = sort_view(ctx, sl, v2, (int32_t)n, ss2, out.rows_cap, false);
   if (rc == ELECTOR_OK) rc = read_plans(ctx, 2, 1, dtab2, sl);   // the host waits for sort 2 alone; the linear segments run meanwhile
   if (rc != ELECTOR_OK) return rc;
   if (ctx->wait_in[1]) CU(cudaStreamWaitEvent(sl, ctx->wait_in[1], 0));
@@ -597,30 +665,30 @@ void add_kernel_ms(elector_ctx *ctx) {
 
 // One alignment on ctx's stream, waited for: run_device, the rows cursor read back, check_tables; a run whose scratch pools
 // were too small runs again with the grown pools.  d_rows_used (device memory, may be NULL) receives the rows cursor.
-int align_device(elector_ctx *ctx, int64_t n, const char *d_ref, const int64_t *d_roff, const char *d_cor, const int64_t *d_coff,
-                 const char *d_unc, const int64_t *d_uoff, const int64_t *h_roff, const int64_t *h_coff, char *d_rows, int64_t rows_cap,
-                 int64_t *d_rowoff, int32_t *d_stride, int32_t *d_nring, int32_t *d_s1, int32_t *d_s2, int64_t *d_cells, int64_t *d_rows_used) {
+int align_device(elector_ctx *ctx, const AlignIn &in, const AlignOut &out, int64_t *d_rows_used) {
   for (int attempt = 0;; ++attempt) {
-    int rc = run_device(ctx, n, d_ref, d_roff, d_cor, d_coff, d_unc, d_uoff, h_roff, h_coff, d_rows, rows_cap, d_rowoff, d_stride, d_nring, d_s1, d_s2, d_cells);
+    int rc = run_device(ctx, in, out);
     if (rc != ELECTOR_OK) return rc;
     if (d_rows_used) CU(cudaMemcpyAsync(d_rows_used, &ctx->d_ctrl->head.rows_cursor, sizeof(int64_t), cudaMemcpyDeviceToDevice, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));   // the one wait of the alignment
-    if (n == 0) return ELECTOR_OK;            // run_device queued nothing: no tables, no times
+    if (in.n == 0) return ELECTOR_OK;         // run_device queued nothing: no tables, no times
     rc = check_tables(ctx);
     if (rc == 1 && attempt < kScratchRetries) continue;
     if (rc != ELECTOR_OK) return rc == 1 ? ctx->fail(ELECTOR_ECUDA, "scratch pools keep overflowing") : rc;
     break;
   }
   add_kernel_ms(ctx);
-  if (ctx->h_back->head.row_error) return ctx->fail(ELECTOR_ECAPACITY, "row buffer capacity %lld too small", (long long)rows_cap);
+  if (ctx->h_back->head.row_error) return ctx->fail(ELECTOR_ECAPACITY, "row buffer capacity %lld too small", (long long)out.rows_cap);
   return ELECTOR_OK;
 }
 
-// device buffers of an alignment's outputs for nw windows into rows_bytes of rows, and of the tally of its n_reads reads
-int reserve_outputs(elector_ctx *ctx, int64_t nw, int64_t rows_bytes, int64_t n_reads) {
+// device buffers of an alignment's outputs for nw windows into rows_bytes of rows (out), and of the tally of its n_reads reads
+int reserve_outputs(elector_ctx *ctx, int64_t nw, int64_t rows_bytes, int64_t n_reads, AlignOut &out) {
   CU(ctx->d_rows.reserve(rows_bytes)); CU(ctx->d_rowoff.reserve(nw * 8)); CU(ctx->d_stride.reserve(nw * 4));
   CU(ctx->d_nring.reserve(nw * 4)); CU(ctx->d_s1.reserve(nw * 4)); CU(ctx->d_s2.reserve(nw * 4)); CU(ctx->d_cells.reserve(nw * 8));
   if (n_reads > 0) CU(ctx->d_tally_out.reserve(n_reads * ELECTOR_TALLY_K * 8));
+  out = {ctx->d_rows.as<char>(), rows_bytes, ctx->d_rowoff.as<int64_t>(), ctx->d_stride.as<int32_t>(), ctx->d_nring.as<int32_t>(),
+         ctx->d_s1.as<int32_t>(), ctx->d_s2.as<int32_t>(), ctx->d_cells.as<int64_t>()};
   return ELECTOR_OK;
 }
 
@@ -645,14 +713,14 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64
   const int64_t w0 = j.w0, w1 = j.w1, nw = w1 - w0, r0 = j.r0, r1 = j.r1, nr = r1 - r0;
   const int64_t first[3] = {pa.ro[w0], pa.co[w0], pa.uo[w0]};
   const int64_t len[3] = {pa.ro[w1] - first[0], pa.co[w1] - first[1], pa.uo[w1] - first[2]};
-  const int64_t br0 = first[0], bc0 = first[1], bu0 = first[2], br = len[0], bc = len[1], bu = len[2];
   DevBuf *d_let[3] = {&ctx->d_ref, &ctx->d_cor, &ctx->d_unc};
   DevBuf *d_off[3] = {&ctx->d_roff, &ctx->d_coff, &ctx->d_uoff};
   const int64_t *h_off[3] = {pa.ro, pa.co, pa.uo};
   const char *h_let[3] = {io.ref, io.cor, io.unc};
   const elector_packed *h_pk[3] = {io.pref, io.pcor, io.punc};
   for (int k = 0; k < 3; ++k) { CU(d_let[k]->reserve(len[k] + 8)); CU(d_off[k]->reserve((nw + 1) * 8)); }
-  int rc = reserve_outputs(ctx, nw, j.rows_len, nr);
+  AlignOut out;
+  int rc = reserve_outputs(ctx, nw, j.rows_len, nr, out);
   if (rc != ELECTOR_OK) return rc;
   // compact wire format: the 32-bit offsets of the chunk (relative to its first letter) are made here, on the worker's
   // thread, while the chunks before it are on their way; the exceptions of the chunk are found by binary search
@@ -661,13 +729,8 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64
   bool use_len = false;
   if (pa.packed) {
     const size_t need = (size_t)3 * (nw + 1) * sizeof(int32_t);
-    if (need > ctx->h_stage_cap) {
-      if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
-      ctx->h_stage = nullptr; ctx->h_stage_cap = 0;
-      CU(cudaMallocHost(&ctx->h_stage, need + need / 4));
-      ctx->h_stage_cap = need + need / 4;
-    }
-    stage = static_cast<int32_t *>(ctx->h_stage);
+    if (need > ctx->h_stage.cap) CU(ctx->h_stage.reserve(need + need / 4));
+    stage = ctx->h_stage;
     const int32_t *h_len[3] = {io.ref_len, io.cor_len, io.unc_len};
     const bool len16 = io.ref_len16 && io.cor_len16 && io.unc_len16;
     use_len = ((h_len[0] && h_len[1] && h_len[2]) || len16) && nw <= 1024 * 1024;   // the caller's 32-bit (or 16-bit) lengths cross the link as they are
@@ -692,178 +755,186 @@ int process_chunk(elector_ctx *ctx, const PipeArgs &pa, const ChunkJob &j, int64
     if (failed.load() != ELECTOR_OK) return ctx->fail(ELECTOR_ECUDA, "another chunk of the call failed");
     std::this_thread::yield();
   }
-  struct PassTurn {   // whatever happens below, the next chunk gets its turn
-    const PipeArgs &pa; int next; bool passed;
-    void pass() { if (!passed) { passed = true; pa.h2d_turn->store(next, std::memory_order_release); } }
-    ~PassTurn() { pass(); }
-  } pass_turn{pa, j.index + 1, false};
-  if (*pa.h2d_prev) CU(cudaStreamWaitEvent(st, *pa.h2d_prev, 0));
-  if (ctx->trace) CU(cudaEventRecord(ctx->uev0, st));
-  // the offsets first, on the compute stream: the size sort needs nothing else.  The letters follow on the copy stream --
-  // ref and cor (phase 1 waits for them), then unc (phase 2 waits for it) -- while the sort and phase 1 run.
-  if (pa.packed && use_len) {   // 32-bit lengths in, added up on the device
-    const int32_t *h_len[3] = {io.ref_len, io.cor_len, io.unc_len};
-    const uint16_t *h_len16[3] = {io.ref_len16, io.cor_len16, io.unc_len16};
-    const bool len16 = h_len16[0] && h_len16[1] && h_len16[2];
-    const int nblocks = (int)((nw + 1023) / 1024);
-    long long *totals = reinterpret_cast<long long *>(ctx->d_rel.as<int32_t>() + (size_t)3 * (nw + 1) + ((nw + 1) & 1));
-    uint16_t *d16 = reinterpret_cast<uint16_t *>(totals + 3 * 1032);
-    for (int k = 0; k < 3; ++k) {
-      int32_t *dl = ctx->d_rel.as<int32_t>() + (size_t)k * (nw + 1);
-      if (len16) {
-        uint16_t *dk = d16 + (size_t)k * (nw + 4);
-        CU(cudaMemcpyAsync(dk, h_len16[k] + w0, (size_t)nw * 2, cudaMemcpyHostToDevice, st));
-        widen_len16_kernel<<<(unsigned)((nw + 255) / 256), 256, 0, st>>>(nw, dk, dl);
-      } else
-        CU(cudaMemcpyAsync(dl, h_len[k] + w0, (size_t)nw * 4, cudaMemcpyHostToDevice, st));
-      len_scan_blocks_kernel<<<nblocks, 1024, 0, st>>>(nw, dl, totals + (size_t)k * 1032);
-      len_scan_totals_kernel<<<1, 1024, 0, st>>>(nblocks, totals + (size_t)k * 1032);
-      len_to_offsets_kernel<<<(unsigned)((nw + 256) / 256), 256, 0, st>>>(nw, dl, totals + (size_t)k * 1032, nblocks, first[k], d_off[k]->as<int64_t>());
-    }
-    CU(cudaGetLastError());
-    ctx->last_launches += 9;
-  } else if (pa.packed) {
-    CU(cudaMemcpyAsync(ctx->d_rel.p, stage, (size_t)3 * (nw + 1) * 4, cudaMemcpyHostToDevice, st));
-    for (int k = 0; k < 3; ++k)
-      widen_offsets_kernel<<<(unsigned)((nw + 256) / 256), 256, 0, st>>>(nw + 1, ctx->d_rel.as<int32_t>() + (size_t)k * (nw + 1), first[k], d_off[k]->as<int64_t>());
-    CU(cudaGetLastError());
-    ctx->last_launches += 3;
-  } else
-    for (int k = 0; k < 3; ++k) CU(cudaMemcpyAsync(d_off[k]->p, h_off[k] + w0, (nw + 1) * 8, cudaMemcpyHostToDevice, st));
-  CU(cudaEventRecord(ctx->ev_fork, st));
-  CU(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_fork, 0));   // the copy engine serves the offsets first
-  int64_t exc_done = 0;
-  for (int k = 0; k < 3; ++k) {
-    if (pa.packed) {   // packed bytes that hold the chunk's letters (+ one of padding), expanded on the device; then the exceptions
-      const int64_t b0 = first[k] >> 2, b1 = (first[k] + len[k] + 3) >> 2;
-      const int64_t have = (h_pk[k]->n_letters + 3) >> 2;
-      CU(cudaMemcpyAsync(ctx->d_pk[k].p, h_pk[k]->bits + b0, (size_t)std::min(b1 + 1, have) - b0, cudaMemcpyHostToDevice, ctx->copy_in));
-      if (len[k] > 0) unpack2_kernel<<<(unsigned)std::min<int64_t>((len[k] / 4 + 256) / 256, (int64_t)ctx->sm_count * 16), 256, 0, ctx->copy_in>>>(
-          ctx->d_pk[k].as<uint8_t>(), (int)(first[k] & 3), len[k], d_let[k]->as<uint8_t>());
-      const int64_t ne = exc1[k] - exc0[k];
-      if (ne > 0) {
-        CU(cudaMemcpyAsync(ctx->d_exc_pos.as<int64_t>() + exc_done, h_pk[k]->exc_pos + exc0[k], ne * 8, cudaMemcpyHostToDevice, ctx->copy_in));
-        CU(cudaMemcpyAsync(ctx->d_exc_byte.as<uint8_t>() + exc_done, h_pk[k]->exc_byte + exc0[k], ne, cudaMemcpyHostToDevice, ctx->copy_in));
-        patch_letters_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, ctx->copy_in>>>(ne, ctx->d_exc_pos.as<int64_t>() + exc_done, ctx->d_exc_byte.as<uint8_t>() + exc_done,
-                                                                                   first[k], d_let[k]->as<uint8_t>());
-        exc_done += ne;
+  // the rest of the chunk, queued behind its input turn: whatever fails there leaves through the one drain below
+  auto queued = [&]() -> int {
+    struct PassTurn {   // whatever happens below, the next chunk gets its turn
+      const PipeArgs &pa; int next; bool passed;
+      void pass() { if (!passed) { passed = true; pa.h2d_turn->store(next, std::memory_order_release); } }
+      ~PassTurn() { pass(); }
+    } pass_turn{pa, j.index + 1, false};
+    if (*pa.h2d_prev) CU(cudaStreamWaitEvent(st, *pa.h2d_prev, 0));
+    if (ctx->trace) CU(cudaEventRecord(ctx->uev0, st));
+    // the offsets first, on the compute stream: the size sort needs nothing else.  The letters follow on the copy stream --
+    // ref and cor (phase 1 waits for them), then unc (phase 2 waits for it) -- while the sort and phase 1 run.
+    if (pa.packed && use_len) {   // 32-bit lengths in, added up on the device
+      const int32_t *h_len[3] = {io.ref_len, io.cor_len, io.unc_len};
+      const uint16_t *h_len16[3] = {io.ref_len16, io.cor_len16, io.unc_len16};
+      const bool len16 = h_len16[0] && h_len16[1] && h_len16[2];
+      const int nblocks = (int)((nw + 1023) / 1024);
+      long long *totals = reinterpret_cast<long long *>(ctx->d_rel.as<int32_t>() + (size_t)3 * (nw + 1) + ((nw + 1) & 1));
+      uint16_t *d16 = reinterpret_cast<uint16_t *>(totals + 3 * 1032);
+      for (int k = 0; k < 3; ++k) {
+        int32_t *dl = ctx->d_rel.as<int32_t>() + (size_t)k * (nw + 1);
+        if (len16) {
+          uint16_t *dk = d16 + (size_t)k * (nw + 4);
+          CU(cudaMemcpyAsync(dk, h_len16[k] + w0, (size_t)nw * 2, cudaMemcpyHostToDevice, st));
+          widen_len16_kernel<<<(unsigned)((nw + 255) / 256), 256, 0, st>>>(nw, dk, dl);
+        } else
+          CU(cudaMemcpyAsync(dl, h_len[k] + w0, (size_t)nw * 4, cudaMemcpyHostToDevice, st));
+        len_scan_blocks_kernel<<<nblocks, 1024, 0, st>>>(nw, dl, totals + (size_t)k * 1032);
+        len_scan_totals_kernel<<<1, 1024, 0, st>>>(nblocks, totals + (size_t)k * 1032);
+        len_to_offsets_kernel<<<(unsigned)((nw + 256) / 256), 256, 0, st>>>(nw, dl, totals + (size_t)k * 1032, nblocks, first[k], d_off[k]->as<int64_t>());
       }
       CU(cudaGetLastError());
-      ctx->last_launches += ne > 0 ? 2 : 1;
+      ctx->last_launches += 9;
+    } else if (pa.packed) {
+      CU(cudaMemcpyAsync(ctx->d_rel.p, stage, (size_t)3 * (nw + 1) * 4, cudaMemcpyHostToDevice, st));
+      for (int k = 0; k < 3; ++k)
+        widen_offsets_kernel<<<(unsigned)((nw + 256) / 256), 256, 0, st>>>(nw + 1, ctx->d_rel.as<int32_t>() + (size_t)k * (nw + 1), first[k], d_off[k]->as<int64_t>());
+      CU(cudaGetLastError());
+      ctx->last_launches += 3;
     } else
-      CU(cudaMemcpyAsync(d_let[k]->p, h_let[k] + first[k], len[k], cudaMemcpyHostToDevice, ctx->copy_in));
-    if (k >= 1) CU(cudaEventRecord(ctx->ev_in[k - 1], ctx->copy_in));
-  }
-  ctx->wait_in[0] = ctx->ev_in[0]; ctx->wait_in[1] = ctx->ev_in[1];
-  *pa.h2d_prev = ctx->ev_in[1];
-  pass_turn.pass();
-  // the offsets stay those of the whole call: the letter pointers are moved back by the chunk's first offset, the row
-  // pointer by the chunk's base in the caller's row buffer (row_off[] then indexes the caller's buffer directly)
-  char *d_rows_v = ctx->d_rows.as<char>() - j.rows_base;
-  cudaStream_t so = ctx->copy_out;
-  const bool want_rows = io.rows_out != nullptr;
-  const bool want_merged = io.m_ref != nullptr;
-  for (int attempt = 0;; ++attempt) {
-    ctx->split_rows = j.split && want_rows;
-    rc = run_device(ctx, nw, ctx->d_ref.as<char>() - br0, ctx->d_roff.as<int64_t>(), ctx->d_cor.as<char>() - bc0, ctx->d_coff.as<int64_t>(),
-                    ctx->d_unc.as<char>() - bu0, ctx->d_uoff.as<int64_t>(), pa.ro + w0, pa.co + w0, d_rows_v, j.rows_base + j.rows_len,
-                    ctx->d_rowoff.as<int64_t>(), ctx->d_stride.as<int32_t>(), ctx->d_nring.as<int32_t>(), ctx->d_s1.as<int32_t>(),
-                    ctx->d_s2.as<int32_t>(), ctx->d_cells.as<int64_t>(), j.rows_base);
-    const bool split = ctx->split_rows;
-    ctx->split_rows = false;
-    if (rc != ELECTOR_OK) { ctx->wait_in[0] = ctx->wait_in[1] = nullptr; cudaStreamSynchronize(ctx->copy_in); cudaStreamSynchronize(st); return rc; }
-    CU(cudaEventRecord(ctx->ev_rows, st));
-    if (nr > 0) {
-      std::vector<int64_t> rf(io.read_first + r0, io.read_first + r1 + 1);
-      for (int64_t &v : rf) v -= w0;
-      const WirePack pack{io.m_nibbles, j.m_base, io.m_esc_cap};
-      rc = queue_merge_tally(ctx, nr, rf.data(), nw, reinterpret_cast<const uint8_t *>(d_rows_v), 3 * (br + bc + bu), ctx->d_rowoff.as<int64_t>(), ctx->d_stride.as<int32_t>(),
-                             ctx->d_nring.as<int32_t>(), ctx->d_tally_out.as<int64_t>(), true, want_merged ? &pack : nullptr, nullptr, ctx->ev1);   // ev1: the chunk's device time covers merge + tally too
-      if (rc != ELECTOR_OK) { ctx->wait_in[0] = ctx->wait_in[1] = nullptr; cudaStreamSynchronize(st); return rc; }
-      if (io.counters_out) CU(cudaMemcpyAsync(io.counters_out + r0 * ELECTOR_TALLY_K, ctx->d_tally_out.p, nr * ELECTOR_TALLY_K * 8, cudaMemcpyDeviceToHost, st));
-      if (io.m_off) CU(cudaMemcpyAsync(io.m_off + r0, ctx->d_moff.p, nr * 8, cudaMemcpyDeviceToHost, st));
-      if (io.m_len) CU(cudaMemcpyAsync(io.m_len + r0, ctx->d_mlen.p, nr * 4, cudaMemcpyDeviceToHost, st));
-    }
-    // the alignment results leave on the copy stream while merge and tally run: the host waits for the POA kernels only
-    // to learn how many row bytes the chunk used.  The linear region first: its segments run next to phase 1 and finish early.
-    const int64_t end_b = j.rows_base + j.rows_len;
-    int64_t base_b = end_b, used_b = end_b;
-    if (split) {
-      CU(cudaEventSynchronize(ctx->ev_lin));
-      used_b = (int64_t)ctx->h_back->lin.cursor; base_b = (int64_t)ctx->h_back->lin.start;
-      if (base_b >= j.rows_base && used_b > base_b && used_b <= end_b)
-        CU(cudaMemcpyAsync(io.rows_out + base_b, d_rows_v + base_b, used_b - base_b, cudaMemcpyDeviceToHost, so));
-    }
-    CU(cudaEventSynchronize(ctx->ev_rows));
-    ctx->wait_in[0] = ctx->wait_in[1] = nullptr;   // the letters have arrived: a second attempt does not wait for them again
-    rc = check_tables(ctx);
-    if (rc == 1 && attempt < kScratchRetries) {   // a scratch pool was too small (first call, or longer windows than before): grown, run the chunk again
-      CU(cudaStreamSynchronize(st));
-      CU(cudaStreamSynchronize(so));
-      if (ctx->trace) fprintf(stderr, "[elector trace] chunk w%lld: scratch pools grown to %zu / %zu / %zu MiB, running it again\n", (long long)w0,
-                              ctx->d_scratch.cap >> 20, ctx->d_scratch_lin.cap >> 20, ctx->d_scratch2.cap >> 20);
-      continue;
-    }
-    if (rc != ELECTOR_OK) { cudaStreamSynchronize(st); cudaStreamSynchronize(so); return rc == 1 ? ctx->fail(ELECTOR_ECUDA, "scratch pools keep overflowing") : rc; }
-    const int64_t used = (int64_t)ctx->h_back->head.rows_cursor;
-    if (ctx->h_back->head.row_error || used > base_b || used_b > end_b) {
-      cudaStreamSynchronize(st);
-      cudaStreamSynchronize(so);
-      return ctx->fail(ELECTOR_ECAPACITY, "rows of a chunk exceed their bound (%lld + %lld > %lld)", (long long)(used - j.rows_base), (long long)(used_b - base_b),
-                       (long long)j.rows_len);
-    }
-    if (want_rows) {
-      CU(cudaMemcpyAsync(io.rows_out + j.rows_base, ctx->d_rows.p, used - j.rows_base, cudaMemcpyDeviceToHost, so));
-      CU(cudaMemcpyAsync(io.row_off + w0, ctx->d_rowoff.p, nw * 8, cudaMemcpyDeviceToHost, so));
-      CU(cudaMemcpyAsync(io.row_stride + w0, ctx->d_stride.p, nw * 4, cudaMemcpyDeviceToHost, so));
-    }
-    if (io.nring) CU(cudaMemcpyAsync(io.nring + w0, ctx->d_nring.p, nw * 4, cudaMemcpyDeviceToHost, so));
-    if (io.score1) CU(cudaMemcpyAsync(io.score1 + w0, ctx->d_s1.p, nw * 4, cudaMemcpyDeviceToHost, so));
-    if (io.score2) CU(cudaMemcpyAsync(io.score2 + w0, ctx->d_s2.p, nw * 4, cudaMemcpyDeviceToHost, so));
-    if (io.cells) CU(cudaMemcpyAsync(io.cells + w0, ctx->d_cells.p, nw * 8, cudaMemcpyDeviceToHost, so));
-    if (nr > 0 && want_merged) {   // the merged rows: their size is known once the merge has run
-      CU(cudaEventSynchronize(ctx->ev_merged));
-      const int64_t cols = ctx->h_back->merged_cols;
-      if (j.m_base + cols > io.m_cap) { cudaStreamSynchronize(st); cudaStreamSynchronize(so); return ctx->fail(ELECTOR_ECAPACITY, "merged rows need more than m_cap = %lld columns", (long long)io.m_cap); }
-      char *dst[3] = {io.m_ref, io.m_cor, io.m_unc};
-      DevBuf *srcb[3] = {&ctx->d_mref, &ctx->d_mcor, &ctx->d_munc};
-      if (io.m_nibbles == 2) CU(cudaMemcpyAsync(dst[0] + j.m_base, ctx->d_nib[0].p, (size_t)cols, cudaMemcpyDeviceToHost, so));
-      else for (int k = 0; k < 3; ++k) {
-        if (io.m_nibbles) CU(cudaMemcpyAsync(dst[k] + j.m_base / 2, ctx->d_nib[k].p, (size_t)(cols + 1) / 2, cudaMemcpyDeviceToHost, so));
-        else CU(cudaMemcpyAsync(dst[k] + j.m_base, srcb[k]->p, (size_t)cols, cudaMemcpyDeviceToHost, so));
-      }
-      if (io.m_nibbles) {
-        const int64_t ne = (int64_t)ctx->h_back->n_esc;
+      for (int k = 0; k < 3; ++k) CU(cudaMemcpyAsync(d_off[k]->p, h_off[k] + w0, (nw + 1) * 8, cudaMemcpyHostToDevice, st));
+    CU(cudaEventRecord(ctx->ev_fork, st));
+    CU(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_fork, 0));   // the copy engine serves the offsets first
+    int64_t exc_done = 0;
+    for (int k = 0; k < 3; ++k) {
+      if (pa.packed) {   // packed bytes that hold the chunk's letters (+ one of padding), expanded on the device; then the exceptions
+        const int64_t b0 = first[k] >> 2, b1 = (first[k] + len[k] + 3) >> 2;
+        const int64_t have = (h_pk[k]->n_letters + 3) >> 2;
+        CU(cudaMemcpyAsync(ctx->d_pk[k].p, h_pk[k]->bits + b0, (size_t)std::min(b1 + 1, have) - b0, cudaMemcpyHostToDevice, ctx->copy_in));
+        if (len[k] > 0) unpack2_kernel<<<(unsigned)std::min<int64_t>((len[k] / 4 + 256) / 256, (int64_t)ctx->sm_count * 16), 256, 0, ctx->copy_in>>>(
+            ctx->d_pk[k].as<uint8_t>(), (int)(first[k] & 3), len[k], d_let[k]->as<uint8_t>());
+        const int64_t ne = exc1[k] - exc0[k];
         if (ne > 0) {
-          const long long at = pa.n_esc->fetch_add(ne);
-          if (at + ne > io.m_esc_cap || ne > io.m_esc_cap) { cudaStreamSynchronize(st); cudaStreamSynchronize(so); return ctx->fail(ELECTOR_ECAPACITY, "more than m_esc_cap = %lld characters outside the 4-bit code", (long long)io.m_esc_cap); }
-          CU(cudaMemcpyAsync(io.m_esc_pos + at, ctx->d_esc_pos.p, (size_t)ne * 8, cudaMemcpyDeviceToHost, so));
-          CU(cudaMemcpyAsync(io.m_esc_byte + at, ctx->d_esc_byte.p, (size_t)ne, cudaMemcpyDeviceToHost, so));
+          CU(cudaMemcpyAsync(ctx->d_exc_pos.as<int64_t>() + exc_done, h_pk[k]->exc_pos + exc0[k], ne * 8, cudaMemcpyHostToDevice, ctx->copy_in));
+          CU(cudaMemcpyAsync(ctx->d_exc_byte.as<uint8_t>() + exc_done, h_pk[k]->exc_byte + exc0[k], ne, cudaMemcpyHostToDevice, ctx->copy_in));
+          patch_letters_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, ctx->copy_in>>>(ne, ctx->d_exc_pos.as<int64_t>() + exc_done, ctx->d_exc_byte.as<uint8_t>() + exc_done,
+                                                                                     first[k], d_let[k]->as<uint8_t>());
+          exc_done += ne;
+        }
+        CU(cudaGetLastError());
+        ctx->last_launches += ne > 0 ? 2 : 1;
+      } else
+        CU(cudaMemcpyAsync(d_let[k]->p, h_let[k] + first[k], len[k], cudaMemcpyHostToDevice, ctx->copy_in));
+      if (k >= 1) CU(cudaEventRecord(ctx->ev_in[k - 1], ctx->copy_in));
+    }
+    ctx->wait_in[0] = ctx->ev_in[0]; ctx->wait_in[1] = ctx->ev_in[1];
+    *pa.h2d_prev = ctx->ev_in[1];
+    pass_turn.pass();
+    // the offsets stay those of the whole call: the letter pointers are moved back by the chunk's first offset, the row
+    // pointer by the chunk's base in the caller's row buffer (row_off[] then indexes the caller's buffer directly)
+    const AlignIn in{nw, ctx->d_ref.as<char>() - first[0], ctx->d_roff.as<int64_t>(), ctx->d_cor.as<char>() - first[1], ctx->d_coff.as<int64_t>(),
+                     ctx->d_unc.as<char>() - first[2], ctx->d_uoff.as<int64_t>(), pa.ro + w0, pa.co + w0};
+    out.rows -= j.rows_base;
+    out.rows_cap += j.rows_base;
+    cudaStream_t so = ctx->copy_out;
+    const bool want_rows = io.rows_out != nullptr;
+    const bool want_merged = io.m_ref != nullptr;
+    for (int attempt = 0;; ++attempt) {
+      ctx->split_rows = j.split && want_rows;
+      rc = run_device(ctx, in, out, j.rows_base);
+      const bool split = ctx->split_rows;
+      ctx->split_rows = false;
+      if (rc != ELECTOR_OK) return rc;
+      CU(cudaEventRecord(ctx->ev_rows, st));
+      if (nr > 0) {
+        std::vector<int64_t> rf(io.read_first + r0, io.read_first + r1 + 1);
+        for (int64_t &v : rf) v -= w0;
+        const WirePack pack{io.m_nibbles, j.m_base, io.m_esc_cap};
+        const WindowRows rows{reinterpret_cast<const uint8_t *>(out.rows), 3 * (len[0] + len[1] + len[2]), out.rowoff, out.stride, out.nring};
+        rc = queue_merge_tally(ctx, nr, rf.data(), nw, rows, ctx->d_tally_out.as<int64_t>(), true, want_merged ? &pack : nullptr, nullptr, ctx->ev1);   // ev1: the chunk's device time covers merge + tally too
+        if (rc != ELECTOR_OK) return rc;
+        if (io.counters_out) CU(cudaMemcpyAsync(io.counters_out + r0 * ELECTOR_TALLY_K, ctx->d_tally_out.p, nr * ELECTOR_TALLY_K * 8, cudaMemcpyDeviceToHost, st));
+        if (io.m_off) CU(cudaMemcpyAsync(io.m_off + r0, ctx->d_moff.p, nr * 8, cudaMemcpyDeviceToHost, st));
+        if (io.m_len) CU(cudaMemcpyAsync(io.m_len + r0, ctx->d_mlen.p, nr * 4, cudaMemcpyDeviceToHost, st));
+      }
+      // the alignment results leave on the copy stream while merge and tally run: the host waits for the POA kernels only
+      // to learn how many row bytes the chunk used.  The linear region first: its segments run next to phase 1 and finish early.
+      const int64_t end_b = j.rows_base + j.rows_len;
+      int64_t base_b = end_b, used_b = end_b;
+      if (split) {
+        CU(cudaEventSynchronize(ctx->ev_lin));
+        used_b = (int64_t)ctx->h_back->lin.cursor; base_b = (int64_t)ctx->h_back->lin.start;
+        if (base_b >= j.rows_base && used_b > base_b && used_b <= end_b)
+          CU(cudaMemcpyAsync(io.rows_out + base_b, out.rows + base_b, used_b - base_b, cudaMemcpyDeviceToHost, so));
+      }
+      CU(cudaEventSynchronize(ctx->ev_rows));
+      ctx->wait_in[0] = ctx->wait_in[1] = nullptr;   // the letters have arrived: a second attempt does not wait for them again
+      rc = check_tables(ctx);
+      if (rc == 1 && attempt < kScratchRetries) {   // a scratch pool was too small (first call, or longer windows than before): grown, run the chunk again
+        CU(cudaStreamSynchronize(st));
+        CU(cudaStreamSynchronize(so));
+        if (ctx->trace) fprintf(stderr, "[elector trace] chunk w%lld: scratch pools grown to %zu / %zu / %zu MiB, running it again\n", (long long)w0,
+                                ctx->d_scratch.cap >> 20, ctx->d_scratch_lin.cap >> 20, ctx->d_scratch2.cap >> 20);
+        continue;
+      }
+      if (rc != ELECTOR_OK) return rc == 1 ? ctx->fail(ELECTOR_ECUDA, "scratch pools keep overflowing") : rc;
+      const int64_t used = (int64_t)ctx->h_back->head.rows_cursor;
+      if (ctx->h_back->head.row_error || used > base_b || used_b > end_b)
+        return ctx->fail(ELECTOR_ECAPACITY, "rows of a chunk exceed their bound (%lld + %lld > %lld)", (long long)(used - j.rows_base), (long long)(used_b - base_b),
+                         (long long)j.rows_len);
+      if (want_rows) {
+        CU(cudaMemcpyAsync(io.rows_out + j.rows_base, ctx->d_rows.p, used - j.rows_base, cudaMemcpyDeviceToHost, so));
+        CU(cudaMemcpyAsync(io.row_off + w0, ctx->d_rowoff.p, nw * 8, cudaMemcpyDeviceToHost, so));
+        CU(cudaMemcpyAsync(io.row_stride + w0, ctx->d_stride.p, nw * 4, cudaMemcpyDeviceToHost, so));
+      }
+      if (io.nring) CU(cudaMemcpyAsync(io.nring + w0, ctx->d_nring.p, nw * 4, cudaMemcpyDeviceToHost, so));
+      if (io.score1) CU(cudaMemcpyAsync(io.score1 + w0, ctx->d_s1.p, nw * 4, cudaMemcpyDeviceToHost, so));
+      if (io.score2) CU(cudaMemcpyAsync(io.score2 + w0, ctx->d_s2.p, nw * 4, cudaMemcpyDeviceToHost, so));
+      if (io.cells) CU(cudaMemcpyAsync(io.cells + w0, ctx->d_cells.p, nw * 8, cudaMemcpyDeviceToHost, so));
+      if (nr > 0 && want_merged) {   // the merged rows: their size is known once the merge has run
+        CU(cudaEventSynchronize(ctx->ev_merged));
+        const int64_t cols = ctx->h_back->merged_cols;
+        if (j.m_base + cols > io.m_cap) return ctx->fail(ELECTOR_ECAPACITY, "merged rows need more than m_cap = %lld columns", (long long)io.m_cap);
+        char *dst[3] = {io.m_ref, io.m_cor, io.m_unc};
+        DevBuf *srcb[3] = {&ctx->d_mref, &ctx->d_mcor, &ctx->d_munc};
+        if (io.m_nibbles == 2) CU(cudaMemcpyAsync(dst[0] + j.m_base, ctx->d_nib[0].p, (size_t)cols, cudaMemcpyDeviceToHost, so));
+        else for (int k = 0; k < 3; ++k) {
+          if (io.m_nibbles) CU(cudaMemcpyAsync(dst[k] + j.m_base / 2, ctx->d_nib[k].p, (size_t)(cols + 1) / 2, cudaMemcpyDeviceToHost, so));
+          else CU(cudaMemcpyAsync(dst[k] + j.m_base, srcb[k]->p, (size_t)cols, cudaMemcpyDeviceToHost, so));
+        }
+        if (io.m_nibbles) {
+          const int64_t ne = (int64_t)ctx->h_back->n_esc;
+          if (ne > 0) {
+            const long long at = pa.n_esc->fetch_add(ne);
+            if (at + ne > io.m_esc_cap || ne > io.m_esc_cap) return ctx->fail(ELECTOR_ECAPACITY, "more than m_esc_cap = %lld characters outside the 4-bit code", (long long)io.m_esc_cap);
+            CU(cudaMemcpyAsync(io.m_esc_pos + at, ctx->d_esc_pos.p, (size_t)ne * 8, cudaMemcpyDeviceToHost, so));
+            CU(cudaMemcpyAsync(io.m_esc_byte + at, ctx->d_esc_byte.p, (size_t)ne, cudaMemcpyDeviceToHost, so));
+          }
         }
       }
+      if (ctx->trace) CU(cudaEventRecord(ctx->uev1, so));
+      CU(cudaStreamSynchronize(st));
+      CU(cudaStreamSynchronize(so));
+      if (nr > 0 && io.m_off) for (int64_t r = r0; r < r1; ++r) io.m_off[r] += j.m_base;   // chunk-relative -> the caller's buffers
+      break;
     }
-    if (ctx->trace) CU(cudaEventRecord(ctx->uev1, so));
-    CU(cudaStreamSynchronize(st));
-    CU(cudaStreamSynchronize(so));
-    if (nr > 0 && io.m_off) for (int64_t r = r0; r < r1; ++r) io.m_off[r] += j.m_base;   // chunk-relative -> the caller's buffers
-    break;
+    if (ctx->trace) {   // device timeline of the chunk, ms after the start of the call
+      float t[6] = {0, 0, 0, 0, 0, 0};
+      cudaEventElapsedTime(&t[0], pa.ev_call, ctx->uev0); cudaEventElapsedTime(&t[1], pa.ev_call, ctx->ev0);
+      cudaEventElapsedTime(&t[2], pa.ev_call, ctx->ev_mid); cudaEventElapsedTime(&t[3], pa.ev_call, ctx->ev_rows);
+      cudaEventElapsedTime(&t[4], pa.ev_call, ctx->ev1); cudaEventElapsedTime(&t[5], pa.ev_call, ctx->uev1);
+      fprintf(stderr, "[elector trace] chunk w%lld: h2d %.2f | sort1 %.2f | phase 1 done %.2f | phase 2 done %.2f | merge+tally done %.2f | results on host %.2f\n",
+              (long long)w0, t[0], t[1], t[2], t[3], t[4], t[5]);
+      (void)cudaGetLastError();
+    }
+    add_kernel_ms(ctx);
+    if (nr > 0) {
+      rc = tally_status(ctx);
+      if (rc != ELECTOR_OK) return rc;
+      for (int f = 0; f < ELECTOR_TALLY_K; ++f) sums[f] += ctx->h_back->sums[f];
+    }
+    return ELECTOR_OK;
+  };
+  rc = queued();
+  if (rc != ELECTOR_OK) {   // nothing of the chunk may still run when the call returns: it uses the caller's buffers and this worker's
+    ctx->wait_in[0] = ctx->wait_in[1] = nullptr;
+    cudaStreamSynchronize(ctx->copy_in);
+    cudaStreamSynchronize(st);
+    cudaStreamSynchronize(ctx->copy_out);
   }
-  if (ctx->trace) {   // device timeline of the chunk, ms after the start of the call
-    float t[6] = {0, 0, 0, 0, 0, 0};
-    cudaEventElapsedTime(&t[0], pa.ev_call, ctx->uev0); cudaEventElapsedTime(&t[1], pa.ev_call, ctx->ev0);
-    cudaEventElapsedTime(&t[2], pa.ev_call, ctx->ev_mid); cudaEventElapsedTime(&t[3], pa.ev_call, ctx->ev_rows);
-    cudaEventElapsedTime(&t[4], pa.ev_call, ctx->ev1); cudaEventElapsedTime(&t[5], pa.ev_call, ctx->uev1);
-    fprintf(stderr, "[elector trace] chunk w%lld: h2d %.2f | sort1 %.2f | phase 1 done %.2f | phase 2 done %.2f | merge+tally done %.2f | results on host %.2f\n",
-            (long long)w0, t[0], t[1], t[2], t[3], t[4], t[5]);
-    (void)cudaGetLastError();
-  }
-  add_kernel_ms(ctx);
-  if (nr > 0) {
-    rc = tally_status(ctx);
-    if (rc != ELECTOR_OK) return rc;
-    for (int f = 0; f < ELECTOR_TALLY_K; ++f) sums[f] += ctx->h_back->sums[f];
-  }
-  return ELECTOR_OK;
+  return rc;
 }
 
 int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int worker = 0);
@@ -897,7 +968,7 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
   elector_ctx *ctx = new elector_ctx();
   auto bail = [&](int code) {
     g_init_error = ctx->err;
-    elector_poa_free(ctx);
+    delete ctx;
     return code;
   };
   ctx->mat = mat;
@@ -916,52 +987,29 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
   cudaDeviceProp prop;
   cudaGetDeviceProperties(&prop, device);
   ctx->sm_count = prop.multiProcessorCount;
-  ctx->smem_optin = prop.sharedMemPerBlockOptin;
   int prio_lo = 0, prio_hi = 0;
   cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);   // numerically lower = higher priority
   const int prio = std::min(prio_lo, prio_hi + worker);
-  if ((e = cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio)) != cudaSuccess ||
-      (e = cudaEventCreate(&ctx->ev0)) != cudaSuccess || (e = cudaEventCreate(&ctx->ev1)) != cudaSuccess ||
-      (e = cudaEventCreate(&ctx->ev_mid)) != cudaSuccess ||
-      (e = cudaEventCreate(&ctx->ev_split0)) != cudaSuccess || (e = cudaEventCreate(&ctx->ev_split1)) != cudaSuccess ||
-      (e = cudaEventCreate(&ctx->ev_mt0)) != cudaSuccess || (e = cudaEventCreate(&ctx->ev_mt1)) != cudaSuccess ||
-      (e = cudaEventCreate(&ctx->ev_rows)) != cudaSuccess ||
-      (e = cudaEventCreateWithFlags(&ctx->ev_lin, cudaEventDisableTiming)) != cudaSuccess ||
-      (e = cudaEventCreateWithFlags(&ctx->ev_merged, cudaEventDisableTiming)) != cudaSuccess ||
-      (e = cudaEventCreateWithFlags(&ctx->ev_in[0], cudaEventDisableTiming)) != cudaSuccess ||
-      (e = cudaEventCreateWithFlags(&ctx->ev_in[1], cudaEventDisableTiming)) != cudaSuccess ||
-      (e = cudaEventCreate(&ctx->uev0)) != cudaSuccess || (e = cudaEventCreate(&ctx->uev1)) != cudaSuccess ||
-      (e = cudaEventCreate(&ctx->ev_call)) != cudaSuccess ||
-      (e = cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming)) != cudaSuccess ||
-      (e = cudaStreamCreateWithPriority(&ctx->lin_stream, cudaStreamNonBlocking, prio)) != cudaSuccess ||
-      (e = cudaEventCreateWithFlags(&ctx->ev_sorted, cudaEventDisableTiming)) != cudaSuccess ||
-      (e = cudaEventCreate(&ctx->ev_lin_done)) != cudaSuccess ||
-      (e = cudaEventCreateWithFlags(&ctx->ev_lin_sorted, cudaEventDisableTiming)) != cudaSuccess ||
-      (e = cudaEventCreateWithFlags(&ctx->ev_bulk1, cudaEventDisableTiming)) != cudaSuccess ||
-      (e = cudaStreamCreateWithFlags(&ctx->copy_in, cudaStreamNonBlocking)) != cudaSuccess ||
-      (e = cudaStreamCreateWithFlags(&ctx->copy_out, cudaStreamNonBlocking)) != cudaSuccess ||
-      (e = cudaMallocHost((void **)&ctx->h_bintab, 2 * sizeof(BinTable))) != cudaSuccess ||
-      (e = cudaMallocHost((void **)&ctx->h_plan, 2 * sizeof(BinTable))) != cudaSuccess ||
-      (e = cudaMallocHost((void **)&ctx->h_back, sizeof(ReadBack))) != cudaSuccess ||
-      (e = ctx->d_tab.reserve(sizeof(SymbolTables))) != cudaSuccess ||
-      (e = cudaMalloc((void **)&ctx->d_ctrl, sizeof(CallCtrl))) != cudaSuccess ||
-      (e = cudaMemset(ctx->d_ctrl, 0, sizeof(CallCtrl))) != cudaSuccess ||
-      (e = cudaMemcpy(ctx->d_tab.p, &ctx->sc.tab, sizeof(SymbolTables), cudaMemcpyHostToDevice)) != cudaSuccess) {
+  // the order in which the streams are created decides which of them share a hardware queue.  Only events whose times are read
+  // keep timing: a stream waits on an event without it at a lower cost.
+  auto ok = [&e](cudaError_t r) { e = r; return r == cudaSuccess; };
+  bool made = ok(ctx->stream.create(prio)) && ok(ctx->lin_stream.create(prio)) && ok(ctx->copy_in.create()) && ok(ctx->copy_out.create());
+  for (Stream &s : ctx->side) made = made && ok(s.create(prio));
+  for (Event *ev : {&ctx->ev0, &ctx->ev1, &ctx->ev_mid, &ctx->ev_rows, &ctx->ev_split0, &ctx->ev_split1, &ctx->ev_mt0, &ctx->ev_mt1, &ctx->uev0, &ctx->uev1,
+                    &ctx->ev_call, &ctx->ev_lin_done})
+    made = made && ok(ev->create(cudaEventDefault));
+  for (auto &view : ctx->ev_view) for (auto &side : view) for (Event &ev : side) made = made && ok(ev.create(cudaEventDefault));
+  for (Event *ev : {&ctx->ev_lin, &ctx->ev_merged, &ctx->ev_in[0], &ctx->ev_in[1], &ctx->ev_fork, &ctx->ev_sorted, &ctx->ev_lin_sorted, &ctx->ev_bulk1})
+    made = made && ok(ev->create(cudaEventDisableTiming));
+  for (Event &ev : ctx->ev_fork_v) made = made && ok(ev.create(cudaEventDisableTiming));
+  for (Event &ev : ctx->ev_join) made = made && ok(ev.create(cudaEventDisableTiming));
+  made = made && ok(ctx->h_bintab.reserve(2 * sizeof(BinTable))) && ok(ctx->h_plan.reserve(2 * sizeof(BinTable))) && ok(ctx->h_back.reserve(sizeof(ReadBack))) &&
+         ok(ctx->d_tab.reserve(sizeof(SymbolTables))) && ok(ctx->d_ctrl.reserve(sizeof(CallCtrl))) && ok(cudaMemset(ctx->d_ctrl, 0, sizeof(CallCtrl))) &&
+         ok(cudaMemcpy(ctx->d_tab.p, &ctx->sc.tab, sizeof(SymbolTables), cudaMemcpyHostToDevice));
+  if (!made) {
     ctx->fail(ELECTOR_ECUDA, "context setup: %s", cudaGetErrorString(e));
     return bail(ELECTOR_ECUDA);
   }
-  for (int k = 0; k < 12; ++k) cudaEventCreate(&ctx->ev_view[k / 4][(k / 2) & 1][k & 1]);
-  for (int k = 0; k < 6; ++k)
-    if ((e = cudaEventCreateWithFlags(&ctx->ev_fork_v[k], cudaEventDisableTiming)) != cudaSuccess) {
-      ctx->fail(ELECTOR_ECUDA, "context setup: %s", cudaGetErrorString(e));
-      return bail(ELECTOR_ECUDA);
-    }
-  for (int k = 0; k < kSideStreams; ++k)
-    if ((e = cudaStreamCreateWithPriority(&ctx->side[k], cudaStreamNonBlocking, prio)) != cudaSuccess ||
-        (e = cudaEventCreateWithFlags(&ctx->ev_join[k], cudaEventDisableTiming)) != cudaSuccess) {
-      ctx->fail(ELECTOR_ECUDA, "context setup: %s", cudaGetErrorString(e));
-      return bail(ELECTOR_ECUDA);
-    }
   if (ctx->sc.generic_sub) resident_warps_per_sm<true>(ctx, prop.sharedMemPerMultiprocessor);
   else resident_warps_per_sm<false>(ctx, prop.sharedMemPerMultiprocessor);
   if (const char *e = getenv("ELECTOR_COOP_GROUP")) ctx->coop_group = std::max(0, std::min(32, atoi(e)));
@@ -1061,54 +1109,7 @@ int run_pool(elector_ctx *ctx, const std::vector<elector_ctx *> &slots, size_t n
 
 extern "C" {
 
-void elector_split_release(elector_ctx *ctx);
-void elector_poa_free(elector_ctx *ctx) {
-  if (!ctx) return;
-  elector_split_release(ctx);
-  for (elector_ctx *w : ctx->workers) elector_poa_free(w);
-  ctx->workers.clear();
-  for (elector_ctx *w : ctx->peers) { cudaSetDevice(w->device); elector_poa_free(w); }   // their buffers and streams belong to their device
-  if (!ctx->peers.empty()) cudaSetDevice(ctx->device);
-  ctx->peers.clear();
-  if (ctx->d_ctrl) cudaFree(ctx->d_ctrl);
-  DevBuf *bufs[] = {&ctx->d_tab, &ctx->d_ref, &ctx->d_cor, &ctx->d_unc, &ctx->d_roff, &ctx->d_coff, &ctx->d_uoff,
-                    &ctx->d_items, &ctx->d_scratch, &ctx->d_scratch_lin, &ctx->d_scratch2, &ctx->d_hist, &ctx->d_bintab, &ctx->d_key, &ctx->d_key2, &ctx->d_n1, &ctx->d_p1, &ctx->d_rows, &ctx->d_rowoff, &ctx->d_stride,
-                    &ctx->d_nring, &ctx->d_s1, &ctx->d_s2, &ctx->d_cells, &ctx->d_wdst, &ctx->d_sums, &ctx->d_stretch, &ctx->d_tally_scan, &ctx->d_tally_out,
-                    &ctx->d_readfirst, &ctx->d_mtot, &ctx->d_moff, &ctx->d_mlen, &ctx->d_mref, &ctx->d_mcor, &ctx->d_munc};
-  for (DevBuf *b : bufs) b->release();
-  if (ctx->ev0) cudaEventDestroy(ctx->ev0);
-  if (ctx->ev1) cudaEventDestroy(ctx->ev1);
-  if (ctx->ev_mid) cudaEventDestroy(ctx->ev_mid);
-  for (cudaEvent_t ev : {ctx->ev_split0, ctx->ev_split1, ctx->ev_mt0, ctx->ev_mt1}) if (ev) cudaEventDestroy(ev);
-  if (ctx->ev_rows) cudaEventDestroy(ctx->ev_rows);
-  for (int k = 0; k < 2; ++k) if (ctx->ev_in[k]) cudaEventDestroy(ctx->ev_in[k]);
-  if (ctx->ev_lin) cudaEventDestroy(ctx->ev_lin);
-  if (ctx->ev_merged) cudaEventDestroy(ctx->ev_merged);
-  if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
-  for (DevBuf *b : {&ctx->d_pk[0], &ctx->d_pk[1], &ctx->d_pk[2], &ctx->d_nib[0], &ctx->d_nib[1], &ctx->d_nib[2], &ctx->d_exc_pos, &ctx->d_exc_byte, &ctx->d_rel, &ctx->d_esc_pos, &ctx->d_esc_byte}) b->release();
-  if (ctx->uev0) cudaEventDestroy(ctx->uev0);
-  if (ctx->uev1) cudaEventDestroy(ctx->uev1);
-  if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
-  if (ctx->ev_sorted) cudaEventDestroy(ctx->ev_sorted);
-  if (ctx->ev_lin_done) cudaEventDestroy(ctx->ev_lin_done);
-  for (int k = 0; k < 6; ++k) if (ctx->ev_fork_v[k]) cudaEventDestroy(ctx->ev_fork_v[k]);
-  if (ctx->ev_lin_sorted) cudaEventDestroy(ctx->ev_lin_sorted);
-  if (ctx->ev_bulk1) cudaEventDestroy(ctx->ev_bulk1);
-  for (int k = 0; k < 12; ++k) if (ctx->ev_view[k / 4][(k / 2) & 1][k & 1]) cudaEventDestroy(ctx->ev_view[k / 4][(k / 2) & 1][k & 1]);
-  if (ctx->lin_stream) cudaStreamDestroy(ctx->lin_stream);
-  for (int k = 0; k < kSideStreams; ++k) {
-    if (ctx->ev_join[k]) cudaEventDestroy(ctx->ev_join[k]);
-    if (ctx->side[k]) cudaStreamDestroy(ctx->side[k]);
-  }
-  if (ctx->h_bintab) cudaFreeHost(ctx->h_bintab);
-  if (ctx->h_plan) cudaFreeHost(ctx->h_plan);
-  if (ctx->ev_call) cudaEventDestroy(ctx->ev_call);
-  if (ctx->copy_in) cudaStreamDestroy(ctx->copy_in);
-  if (ctx->copy_out) cudaStreamDestroy(ctx->copy_out);
-  if (ctx->h_back) cudaFreeHost(ctx->h_back);
-  if (ctx->stream) cudaStreamDestroy(ctx->stream);
-  delete ctx;
-}
+void elector_poa_free(elector_ctx *ctx) { delete ctx; }
 
 const char *elector_last_error(const elector_ctx *ctx) { return ctx ? ctx->err.c_str() : g_init_error.c_str(); }
 
@@ -1131,8 +1132,9 @@ int elector_poa_run_device(elector_ctx *ctx, int64_t n, const char *d_ref, const
   ctx->trace = getenv("ELECTOR_TRACE") != nullptr;
   ctx->last_ms = ctx->last_ms_phase1 = 0.f;
   ctx->last_launches = 0;
-  return align_device(ctx, n, d_ref, d_roff, d_cor, d_coff, d_unc, d_uoff, h_roff, h_coff, d_rows, rows_cap, d_rowoff, d_stride, d_nring, d_s1, d_s2,
-                      d_cells, d_rows_used);
+  const AlignIn in{n, d_ref, d_roff, d_cor, d_coff, d_unc, d_uoff, h_roff, h_coff};
+  const AlignOut out{d_rows, rows_cap, d_rowoff, d_stride, d_nring, d_s1, d_s2, d_cells};
+  return align_device(ctx, in, out, d_rows_used);
 }
 
 int elector_poa_run(elector_ctx *ctx, int64_t n, const char *ref, const int64_t *ro, const char *cor, const int64_t *co,
