@@ -123,9 +123,8 @@ struct ReadBack {
 struct elector_ctx {
   int device = -1;   // set by create_context once the device is known to exist
   int sm_count = 0;
-  int resident_ph1 = 0, resident_ph2 = 0, resident_ph1p = 0, resident_ph2l = 0, resident_coop = 0;  // POA kernel CTAs (one warp each) resident per SM
+  int resident_ph1 = 0, resident_ph2 = 0, resident_ph1p = 0, resident_ph2l = 0, resident_ph2d = 0, resident_coop = 0;  // POA kernel CTAs (one warp each) resident per SM
   int arena_ph1 = 0, arena_ph2 = 0, arena_ph1p = 0, arena_ph2l = 0, arena_ph2d = 0;   // bytes of the per-warp shared-memory arena of each kernel (fast part of the layouts)
-  int coop_group = kCoopGroupDefault;  // windows per warp of the warp-cooperative kernel; 0 = the longest windows stay thread-per-window (ELECTOR_COOP_GROUP)
   Mem<ReadBack> h_back;
   Stream stream;
   Stream side[kSideStreams];   // one per segment that does not run on the main stream
@@ -153,7 +152,6 @@ struct elector_ctx {
   DevBuf d_wdst, d_sums, d_tally_scan, d_tally_out, d_readfirst, d_mtot, d_moff, d_mlen, d_mref, d_mcor, d_munc;
   bool trace = false;
   int band_w = 6;          // ELECTOR_BAND_W: base half-width of the diagonal band of the packed linear kernels (+ rows/16 in phase 1, + rows/8 in phase 2; 0 = full DP)
-  int resident_ph2d = 0;   // 0: the general windows of phase 2 run the INT32 kernel with frontier sets
   unsigned side_used = 0;        // side streams with launches that `st` has not been made to wait for yet
   Mem<elector::BinTable> h_plan;   // the plans of phase 1 / phase 2 of the current call (read_plans)
   // rows of a pipelined chunk in two regions: the windows of the linear segments of phase 2 (most windows, finished early)
@@ -216,11 +214,11 @@ const int kScratchRetries = 3; // runs of an alignment again after its scratch p
 enum SegKind { kInt32 = 0, kPacked = 1, kLinear = 2, kCoop = 3, kDual = 4 };
 
 template <bool GS>
-cudaError_t launch_phase(int phase, int kind, cudaStream_t st, PoaArgs &a, int grid, const SymbolTables *tab, int coop_group, bool linear_seg,
+cudaError_t launch_phase(int phase, int kind, cudaStream_t st, PoaArgs &a, int grid, const SymbolTables *tab, bool linear_seg,
                          const elector_ctx *ctx) {
   auto arena = [&](int bytes) { a.arena_words = (uint32_t)(bytes / 128); return (size_t)bytes; };
-  if (kind == kCoop && phase == 1) { a.arena_words = 0; poa_dp1_coop_kernel<GS><<<grid, 32, 0, st>>>(a, tab, coop_group); }
-  else if (kind == kCoop) { a.arena_words = 0; poa_dp2_coop_kernel<GS><<<grid, 32, 0, st>>>(a, tab, coop_group, linear_seg); }
+  if (kind == kCoop && phase == 1) { a.arena_words = 0; poa_dp1_coop_kernel<GS><<<grid, 32, 0, st>>>(a, tab); }
+  else if (kind == kCoop) { a.arena_words = 0; poa_dp2_coop_kernel<GS><<<grid, 32, 0, st>>>(a, tab, linear_seg); }
   else if (phase == 1) {
     if (kind == kPacked) poa_dp1_kernel<Phase1P, EL_MIN_WARPS_PH1P><<<grid, 32, arena(ctx->arena_ph1p), st>>>(a, tab);
     else poa_dp1_kernel<Phase1<GS>, EL_MIN_WARPS_PH1><<<grid, 32, arena(ctx->arena_ph1), st>>>(a, tab);
@@ -251,17 +249,26 @@ void size_arena(K kernel, size_t smem_per_sm, int &resident, int &arena_bytes) {
   if (arena_bytes > 48 * 1024 - (int)fa.sharedSizeBytes) arena_bytes = (48 * 1024 - (int)fa.sharedSizeBytes) & ~127;
 }
 
+// Residency and arena of every DP kernel.  Returns the name of a kernel of which no CTA fits on an SM, or nullptr: every
+// segment kind has one kernel, and no slower one to fall back to.
 template <bool GS>
-void resident_warps_per_sm(elector_ctx *ctx, size_t smem_per_sm) {
+const char *resident_warps_per_sm(elector_ctx *ctx, size_t smem_per_sm) {
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->resident_coop, poa_dp2_coop_kernel<GS>, 32, 0);
   int coop1 = 0;
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&coop1, poa_dp1_coop_kernel<GS>, 32, 0);
-  ctx->resident_coop = std::min(ctx->resident_coop, coop1);
   size_arena(poa_dp2_kernel<Phase2L, EL_MIN_WARPS_PH2L>, smem_per_sm, ctx->resident_ph2l, ctx->arena_ph2l);
   size_arena(poa_dp1_kernel<Phase1<GS>, EL_MIN_WARPS_PH1>, smem_per_sm, ctx->resident_ph1, ctx->arena_ph1);
   size_arena(poa_dp2_kernel<Phase2<GS>, EL_MIN_WARPS_PH2>, smem_per_sm, ctx->resident_ph2, ctx->arena_ph2);
   size_arena(poa_dp1_kernel<Phase1P, EL_MIN_WARPS_PH1P>, smem_per_sm, ctx->resident_ph1p, ctx->arena_ph1p);
   size_arena(poa_dp2_kernel<Phase2D, EL_MIN_WARPS_PH2D>, smem_per_sm, ctx->resident_ph2d, ctx->arena_ph2d);
+  const struct { const char *name; int resident; } fit[] = {
+      {"poa_dp1_coop_kernel", coop1}, {"poa_dp2_coop_kernel", ctx->resident_coop}, {"poa_dp2_kernel<Phase2L>", ctx->resident_ph2l},
+      {"poa_dp1_kernel<Phase1>", ctx->resident_ph1}, {"poa_dp2_kernel<Phase2>", ctx->resident_ph2}, {"poa_dp1_kernel<Phase1P>", ctx->resident_ph1p},
+      {"poa_dp2_kernel<Phase2D>", ctx->resident_ph2d}};
+  ctx->resident_coop = std::min(ctx->resident_coop, coop1);
+  for (const auto &k : fit)
+    if (k.resident < 1) return k.name;
+  return nullptr;
 }
 
 // ---- device-side planning of a sort view's segments --------------------------------------------------------------
@@ -275,7 +282,6 @@ struct SegStatic {
   int32_t grid[kMaxSegs];    // CTAs of the segment's launch
   int32_t seg0, seg1;        // the view's segments
   int32_t phase;             // 1 or 2
-  int32_t coop_group;
   int32_t counter0;          // control word of segment 0's work counter
   unsigned long long pool_words;     // scratch pool of the view
   unsigned long long budget_words;   // no single segment takes more than this
@@ -306,7 +312,7 @@ __global__ void plan_segments_kernel(BinTable *tab, SegStatic ss, CallCtrl *ctrl
     pl.start = tab->seg[s].start; pl.count = tab->seg[s].count; pl.counter = ss.counter0 + s;
     if (pl.count > 0) {
       pl.warp_words = layout_words(ss.phase, ss.kind[s], tab->seg_max[s * 4], tab->seg_max[s * 4 + 1]);
-      const int per = ss.kind[s] == kCoop ? ss.coop_group : 32;
+      const int per = ss.kind[s] == kCoop ? kCoopGroup : 32;
       long long ctas = ((long long)pl.count + per - 1) / per;
       if (ctas > ss.grid[s]) ctas = ss.grid[s];
       const unsigned long long per_warp = (unsigned long long)pl.warp_words * 32;
@@ -349,16 +355,13 @@ struct SortView {
   DevBuf *pool;
 };
 
-// kernel of a segment (static: known before the sort runs, see SegStatic)
+// kernel of a segment (static: known before the sort runs, see SegStatic).  Windows of more than 128 rows run a warp per
+// window: the big tiers and the first small segment (129 .. 256 rows) of phase 1, of the general and of the linear segments
+// of phase 2; the other segments a thread per window, on packed cells when the matrix allows it (small_packed).
 int seg_kind(const elector_ctx *ctx, int phase, int s) {
   const bool small16 = ctx->sc.small_packed();
-  // windows of more than 128 rows run a warp per window: the big tiers and the first small segment (129 .. 256 rows) of phase 1,
-  // of the general and of the linear segments of phase 2
-  if (phase == 1) return (s <= kBigTiers && ctx->coop_group > 0) ? kCoop : (s >= kBigTiers && small16) ? kPacked : kInt32;
-  const bool longest = s <= kBigTiers || s == kFirstLinSeg2;
-  if (longest && ctx->coop_group > 0) return kCoop;
-  if (s < kBigTiers || !small16) return kInt32;
-  return s >= kFirstLinSeg2 ? kLinear : ctx->resident_ph2d > 0 ? kDual : kInt32;
+  if (phase == 1) return s <= kBigTiers ? kCoop : small16 ? kPacked : kInt32;
+  return s <= kBigTiers || s == kFirstLinSeg2 ? kCoop : !small16 ? kInt32 : s >= kFirstLinSeg2 ? kLinear : kDual;
 }
 int seg_resident(const elector_ctx *ctx, int phase, int kind) {
   switch (kind) {
@@ -379,14 +382,14 @@ int sort_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, int32_t n, S
   bin_scatter_kernel<<<(int)(((int64_t)n + kScatterTile - 1) / kScatterTile), kScatterThreads, 0, st>>>(n, v.key, v.hist, v.chunks, v.items,
                                                                                                         v.bin0, v.bin1, end_bit);
   memset(&ss, 0, sizeof ss);
-  ss.seg0 = v.seg0; ss.seg1 = v.seg1; ss.phase = v.phase; ss.coop_group = std::max(1, ctx->coop_group);
+  ss.seg0 = v.seg0; ss.seg1 = v.seg1; ss.phase = v.phase;
   ss.counter0 = (int32_t)((v.phase == 1 ? offsetof(CallCtrl, work1) : offsetof(CallCtrl, work2)) / sizeof(int32_t));
   ss.pool_words = v.pool->cap / 4;
   ss.budget_words = ((unsigned long long)24 << 30) / 4;
   for (int s = v.seg0; s < v.seg1; ++s) {
     const int kind = seg_kind(ctx, v.phase, s);
     ss.kind[s] = (int8_t)kind;
-    ss.grid[s] = std::max(1, seg_resident(ctx, v.phase, kind)) * ctx->sm_count;
+    ss.grid[s] = seg_resident(ctx, v.phase, kind) * ctx->sm_count;   // >= 1 per SM (create_context)
   }
   plan_segments_kernel<<<1, 32, 0, st>>>(v.dtab, ss, ctx->d_ctrl, rows_cap, split_rows ? 1 : 0);
   CU(cudaGetLastError());
@@ -426,8 +429,8 @@ int launch_view(elector_ctx *ctx, cudaStream_t st, const SortView &v, const SegS
       PoaArgs a = base;
       a.tab = v.dtab; a.seg = s; a.items_base = v.items; a.scratch_base = v.pool->as<uint32_t>(); a.ctrl = reinterpret_cast<int32_t *>(ctx->d_ctrl.p);
       const bool linear_seg = v.phase == 2 && s >= kFirstLinSeg2;
-      const cudaError_t e = ctx->sc.generic_sub ? launch_phase<true>(v.phase, kind, ls, a, grid, ctx->d_tab.as<SymbolTables>(), ss.coop_group, linear_seg, ctx)
-                                                : launch_phase<false>(v.phase, kind, ls, a, grid, ctx->d_tab.as<SymbolTables>(), ss.coop_group, linear_seg, ctx);
+      const cudaError_t e = ctx->sc.generic_sub ? launch_phase<true>(v.phase, kind, ls, a, grid, ctx->d_tab.as<SymbolTables>(), linear_seg, ctx)
+                                                : launch_phase<false>(v.phase, kind, ls, a, grid, ctx->d_tab.as<SymbolTables>(), linear_seg, ctx);
       if (e != cudaSuccess) return ctx->fail(ELECTOR_ECUDA, "kernel launch: %s", cudaGetErrorString(e));
       ++ctx->last_launches;
       cudaEvent_t done = ctx->ev_join[side];
@@ -525,7 +528,7 @@ int run_device(elector_ctx *ctx, const AlignIn &in, const AlignOut &out, int64_t
   // windows whose corrected letters are the reference letters need no phase 1 (bin_kernel.cuh): the sort then reads the
   // letters, so it waits for them too.  Only when their phase 2 needs no node list: Phase2L for the small linear segments,
   // the warp-cooperative kernel (which rebuilds lin(ref)) for the long ones.
-  const bool ident_ok = ctx->sc.small_packed() && ctx->coop_group > 0;
+  const bool ident_ok = ctx->sc.small_packed();
   if (ident_ok && ctx->wait_in[0]) CU(cudaStreamWaitEvent(st, ctx->wait_in[0], 0));
   IdentArgs ida{(const uint8_t *)in.ref, (const uint8_t *)in.cor, ctx->d_n1.as<int32_t>(), ctx->d_key2.as<int32_t>(), hist2, dtab2->seg_max, out.s1, &dtab2->lin_bytes};
   bin1_count_kernel<<<bgrid, 256, 0, st>>>((int32_t)n, in.roff, in.coff, in.uoff, ctx->d_key.as<int32_t>(), hist1, dtab1, ident_ok, ida);
@@ -1010,15 +1013,13 @@ int create_context(int device, const ScoreMatrix &mat, elector_ctx **out, int wo
     ctx->fail(ELECTOR_ECUDA, "context setup: %s", cudaGetErrorString(e));
     return bail(ELECTOR_ECUDA);
   }
-  if (ctx->sc.generic_sub) resident_warps_per_sm<true>(ctx, prop.sharedMemPerMultiprocessor);
-  else resident_warps_per_sm<false>(ctx, prop.sharedMemPerMultiprocessor);
-  if (const char *e = getenv("ELECTOR_COOP_GROUP")) ctx->coop_group = std::max(0, std::min(32, atoi(e)));
-  if (ctx->resident_coop < 1) ctx->coop_group = 0;
+  const char *unfit = ctx->sc.generic_sub ? resident_warps_per_sm<true>(ctx, prop.sharedMemPerMultiprocessor)
+                                          : resident_warps_per_sm<false>(ctx, prop.sharedMemPerMultiprocessor);
   if (ctx->trace)
     fprintf(stderr, "[elector trace] resident warps / arena bytes per warp: Phase1P %d / %d, Phase2L %d / %d, Phase2D %d / %d, Phase1 %d / %d, Phase2 %d / %d, coop %d\n",
             ctx->resident_ph1p, ctx->arena_ph1p, ctx->resident_ph2l, ctx->arena_ph2l, ctx->resident_ph2d, ctx->arena_ph2d, ctx->resident_ph1, ctx->arena_ph1,
             ctx->resident_ph2, ctx->arena_ph2, ctx->resident_coop);
-  if (ctx->resident_ph1 < 1 || ctx->resident_ph2 < 1) { ctx->fail(ELECTOR_ECUDA, "POA kernel does not fit on this device"); return bail(ELECTOR_ECUDA); }
+  if (unfit) { ctx->fail(ELECTOR_ECUDA, "POA kernel %s does not fit on this device", unfit); return bail(ELECTOR_ECUDA); }
   *out = ctx;
   return ELECTOR_OK;
 }

@@ -6,7 +6,7 @@
 // has finished (profiles/r1c_launches_packed.csv: the 32-warp launch of the longest windows takes 3.9 ms,
 // the bulk of the same 650 k-window chunk 0.8 ms).  The longest windows therefore run here:
 //
-//   * a warp owns a small GROUP of windows (2 by default, in lanes 0..group-1 of the lane-interleaved
+//   * a warp owns a small GROUP of windows (kCoopGroup, in lanes 0..kCoopGroup-1 of the lane-interleaved
 //     scratch); the serial per-window steps (letter packing, node
 //     preparation, traceback, fuse + MSA emit) stay thread-per-window and are the code of Phase2;
 //   * the DP of each window of the group is computed by ALL 32 LANES: lane l owns rows 8l .. 8l+7 of a
@@ -30,7 +30,7 @@ namespace elector {
 
 constexpr int kCoopRows = 8;                    // rows per lane
 constexpr int kCoopPassRows = 32 * kCoopRows;   // rows per pass of the warp
-constexpr int kCoopGroupDefault = 2;            // windows per warp (measured: 1, 2 and 4 within 2 % of each other on config 1, 8 and more slower)
+constexpr int kCoopGroup = 2;                   // windows per warp (measured: 1, 2 and 4 within 2 % of each other on config 1, 8 and more slower)
 
 // what lane l hands to lane l+1 after it has finished a node
 struct CoopLink {
@@ -201,11 +201,11 @@ __device__ __forceinline__ void coop_dp(const Phase2<GENERIC_SUB> &win, uint32_t
 #define EL_MIN_WARPS_COOP 24
 #endif
 
-// Phase 2 of the longest windows: groups of `group` windows per warp (owners = lanes 0..group-1).
+// Phase 2 of the longest windows: groups of kCoopGroup windows per warp (owners = lanes 0..kCoopGroup-1).
 template <bool GENERIC_SUB>
 // linear_seg: the launch holds windows whose P1 is lin(ref) with every node carrying both letters (the linear segments of
 // sort 2); their node list is rebuilt from the reference letters (windows whose cor is ref never ran phase 1, bin_kernel.cuh).
-__global__ void __launch_bounds__(32, EL_MIN_WARPS_COOP) poa_dp2_coop_kernel(PoaArgs a, const SymbolTables *g_tab, int group, bool linear_seg) {
+__global__ void __launch_bounds__(32, EL_MIN_WARPS_COOP) poa_dp2_coop_kernel(PoaArgs a, const SymbolTables *g_tab, bool linear_seg) {
   __shared__ uint32_t s_tab[(GENERIC_SUB ? sizeof(SymbolTables) : offsetof(SymbolTables, sub)) / 4];
   __shared__ Layout2 s_layout;
   __shared__ uint32_t s_bset[2 * kSlotWords];
@@ -222,10 +222,10 @@ __global__ void __launch_bounds__(32, EL_MIN_WARPS_COOP) poa_dp2_coop_kernel(Poa
   c.Lp = &s_layout;
   for (;;) {
     int base = 0;
-    if (lane == 0) base = atomicAdd(s_run.work_counter, group);
+    if (lane == 0) base = atomicAdd(s_run.work_counter, kCoopGroup);
     base = __shfl_sync(EL_WARP_FULL, base, 0);
     if (base >= s_run.n_items) break;
-    const int cnt = min(group, s_run.n_items - base);
+    const int cnt = min(kCoopGroup, s_run.n_items - base);
     const bool owner = lane < cnt;
     int nring = 0, w = -1, n1 = 0, lu = 0;
     int64_t ro = 0, co = 0, uo = 0;
@@ -284,7 +284,7 @@ __global__ void __launch_bounds__(32, EL_MIN_WARPS_COOP) poa_dp2_coop_kernel(Poa
 
 // Phase 1 of the longest windows: same grouping; results and phase-2 bookkeeping as poa_dp1_kernel.
 template <bool GENERIC_SUB>
-__global__ void __launch_bounds__(32, EL_MIN_WARPS_COOP) poa_dp1_coop_kernel(PoaArgs a, const SymbolTables *g_tab, int group) {
+__global__ void __launch_bounds__(32, EL_MIN_WARPS_COOP) poa_dp1_coop_kernel(PoaArgs a, const SymbolTables *g_tab) {
   __shared__ uint32_t s_tab[(GENERIC_SUB ? sizeof(SymbolTables) : offsetof(SymbolTables, sub)) / 4];
   __shared__ LayoutC1 s_layout;
   __shared__ uint32_t s_bset[2 * kSlotWords];
@@ -301,10 +301,10 @@ __global__ void __launch_bounds__(32, EL_MIN_WARPS_COOP) poa_dp1_coop_kernel(Poa
   c.Lp = &s_layout.l2;
   for (;;) {
     int base = 0;
-    if (lane == 0) base = atomicAdd(s_run.work_counter, group);
+    if (lane == 0) base = atomicAdd(s_run.work_counter, kCoopGroup);
     base = __shfl_sync(EL_WARP_FULL, base, 0);
     if (base >= s_run.n_items) break;
-    const int cnt = min(group, s_run.n_items - base);
+    const int cnt = min(kCoopGroup, s_run.n_items - base);
     const bool owner = lane < cnt;
     int w = -1, lr = 0, lc = 0;
     int64_t ro = 0, co = 0;

@@ -92,11 +92,10 @@ def test_large_tier_vs_oracle(ctx):
         assert res.window_rows(w) == oracle.window_rows(o, w), w
 
 
-@pytest.mark.parametrize("group", ["0", "1", "8", "32"])
-def test_long_windows_warp_cooperative_vs_oracle(group, monkeypatch):
-    """windows of 120..600 letters (the segments the warp-cooperative kernel of poa_coop.cuh runs, one and several
-    256-row passes, odd and even lane counts, partial groups) against the oracle, for several group sizes;
-    group 0 = the same windows through the thread-per-window kernels"""
+def test_long_windows_warp_cooperative_vs_oracle():
+    """windows of 120..600 letters (the segments the warp-cooperative kernels of poa_coop.cuh run, one and several
+    256-row passes, odd and even lane counts, a partial group at the end of every segment with an odd count) against
+    the oracle"""
     import elector_b200
     from elector_b200 import windows_to_csr
     from oracle import oracle, synth
@@ -114,7 +113,6 @@ def test_long_windows_warp_cooperative_vs_oracle(group, monkeypatch):
         unc = synth.mutate(rng, ref, [0.1, 0.2][rng.below(2)], ab) or "A"
         wins.append((ref, cor, unc))
     r, ro = windows_to_csr([w[0] for w in wins]); c, co = windows_to_csr([w[1] for w in wins]); u, uo = windows_to_csr([w[2] for w in wins])
-    monkeypatch.setenv("ELECTOR_COOP_GROUP", group)
     with elector_b200.PoaContext(0) as c2:
         res = c2.run_csr(r, ro, c, co, u, uo)
     o = oracle.batch(r, ro, c, co, u, uo, nthreads=os.cpu_count() or 1)

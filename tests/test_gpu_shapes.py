@@ -52,7 +52,6 @@ def assert_window(res, i, o, j, what):
 
 SETTINGS = {
     "default": {},
-    "coop0": {"ELECTOR_COOP_GROUP": "0"},      # long windows thread-per-window on INT32, the cor-is-ref shortcut off
     "band0": {"ELECTOR_BAND_W": "0"},
     "band1": {"ELECTOR_BAND_W": "1"},
 }
